@@ -16,6 +16,9 @@ public API: the step's session indices (pinned host memory, what a sampler yield
 built there from the device-resident columnar corpus (corpus.DeviceCorpus), the result is read back; every step.
 `--impl reference`: the UNMODIFIED reference modules from oracle/_ref (oracle/make_ref.py) on the host cores, on a bounded
 sample of the same workload; the oracle port only if that copy is absent.
+`--dump-outputs DIR`: after the timed steps, what the last of them returned (model outputs, losses and parameter gradients
+of a train step; outputs and NDCG sums of an eval or baselines step) as DIR/<name>.npy.  The inputs and initial weights
+are drawn from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -83,7 +86,13 @@ def parse():
     ap.add_argument("--e2e_dense_api", action="store_true", help="also time the host-packed dense-API input path of round 1")
     ap.add_argument("--eval_steps", type=int, default=10)
     ap.add_argument("--profile_mode", action="store_true", help="under ncu: only warm-up + timed steps, nothing else")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (see dump_outputs), to compare builds")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
     c = CONFIGS[a.config]
     for k in ("variant", "batch", "list_len", "model_num", "intent_num"):
         if getattr(a, k) is None:
@@ -107,6 +116,45 @@ def make_cfg(a) -> tuple:
 
 def batch_bytes(batch) -> int:
     return sum(t.numel() * t.element_size() for t in batch.values() if torch.is_tensor(t))
+
+
+DUMP_BYTES = 60 << 20        # array data; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(arrays, out_dir: str) -> None:
+    """Writes every tensor of `arrays` as <out_dir>/<name>.npy: float64 stays float64, other floating types become
+    float32, integers float64.  Their data totals DUMP_BYTES at most: the smaller arrays are written whole, and an array
+    beyond its share of what is left keeps a seeded sample of its rows along the first axis (of its elements if one row
+    is already too large), drawn first among the rows that are not all zero, so that a sparse gradient such as that of
+    an embedding table keeps the rows the step touched.  The indices of the kept rows go to <name>.rows.npy (float64,
+    ascending); they are part of what two builds compare."""
+    os.makedirs(out_dir, exist_ok=True)
+
+    def dtype_of(t):
+        return torch.float32 if t.is_floating_point() and t.dtype != torch.float64 else torch.float64
+
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel() * dtype_of(kv[1]).itemsize)
+    left = DUMP_BYTES
+    for j, (name, t) in enumerate(items):
+        t = t.detach().to(dtype_of(t))
+        share = left // (len(items) - j)
+        if t.dim() > 0 and t.numel() * t.element_size() > share:
+            if t[0].numel() * t.element_size() + 8 > share:
+                t = t.reshape(-1)
+            n, row_bytes = t.shape[0], t[0].numel() * t.element_size()
+            k = min(n, share // (row_bytes + 8))                  # + 8: the row's entry in <name>.rows.npy
+            live = (t.reshape(n, -1) != 0).any(1).nonzero().flatten().cpu().numpy()
+            rng = np.random.default_rng(0)
+            if len(live) >= k:
+                rows = rng.choice(live, k, replace=False)
+            else:
+                rows = np.concatenate([live, rng.choice(np.setdiff1d(np.arange(n), live), k - len(live), replace=False)])
+            rows = np.sort(rows)
+            t = t.index_select(0, torch.from_numpy(rows).to(t.device))
+            np.save(os.path.join(out_dir, name + ".rows.npy"), rows.astype(np.float64))
+            left -= rows.size * 8
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+        left -= t.numel() * t.element_size()
 
 
 def metric_name(mode: str) -> str:
@@ -317,7 +365,8 @@ def run_b200(a):
     single = [baselines.SingleSort(choose_list=n) for n in ("pCTR", "pCVR", "pFVR")]      # script/baselines.sh:1-20
     borda, fusion = baselines.Borda(), baselines.RandomFusion()
 
-    def train_step(batch):
+    # keep: a dict that receives what a caller of the step gets back (model outputs, losses, gradients, NDCG sums)
+    def train_step(batch, keep=None):
         for p in model.parameters():
             p.grad = None
         out = model(batch)
@@ -325,22 +374,34 @@ def run_b200(a):
         loss.backward()
         if reducer is not None:
             reducer.allreduce()
+        if keep is not None:
+            keep.update(out, loss=loss, ensemble_loss=ens_l, intent_loss=int_l)
+            keep.update({"grad." + n: p.grad for n, p in model.named_parameters() if p.grad is not None})
         return loss
 
     def ndcg(ens, b):
         return evaluate.ndcg_sums(ens, b["ranking"], b["session_len"], b["c_paynum_i"], b["c_favnum_i"], b["c_clicknum_i"],
                                   max(L, max(TOPK)), TOPK)[0]
 
-    def eval_step(b):
+    def eval_step(b, keep=None):
         with torch.no_grad():
             out = model(b)
-        return ndcg(out["ens_score"], b)
+        s = ndcg(out["ens_score"], b)
+        if keep is not None:
+            keep.update(out, ndcg_sums=s)
+        return s
 
-    def baselines_step(b):
+    def baselines_step(b, keep=None):
         s = None
-        for m in single + [borda, fusion]:
-            r = ndcg(m(b)["ens_score"], b)
+        for name, m in zip(("single_sort_pCTR", "single_sort_pCVR", "single_sort_pFVR", "borda", "random_fusion"),
+                           single + [borda, fusion]):
+            out = m(b)
+            r = ndcg(out["ens_score"], b)
             s = r if s is None else s + r
+            if keep is not None:
+                keep.update({f"{name}.{k}": v for k, v in out.items()})
+        if keep is not None:
+            keep["ndcg_sums"] = s
         return s
 
     step_fn = {"train": train_step, "eval": eval_step, "baselines": baselines_step}[a.mode]
@@ -374,8 +435,13 @@ def run_b200(a):
     for i in range(a.warmup if a.profile_mode else max(a.warmup, 3)):
         step_fn(resident[i % len(resident)])
     sampler = ClockSampler(local) if rank == 0 else None
-    ms_total = timed(lambda i: step_fn(resident[i % len(resident)]), a.steps)
+    last = {} if a.dump_outputs else None
+    ms_total = timed(lambda i: step_fn(resident[i % len(resident)], last if i == a.steps - 1 else None), a.steps)
     clocks = sampler.stop() if sampler else None
+    if last is not None:
+        if rank == 0:
+            dump_outputs(last, a.dump_outputs)
+        last.clear()
     ms_step = ms_total / a.steps
     value = world * B / (ms_step * 1e-3)
     if a.profile_mode:

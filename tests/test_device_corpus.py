@@ -120,10 +120,21 @@ def test_device_built_batch_equals_collate_batch(wired, columnar, device, phase,
     assert out["batch_size"] == ref["batch_size"] and out["phase"] == ref["phase"]
 
 
-@needs_ref
-def test_default_shuffle_is_a_permutation_of_every_list(columnar, device):
-    from intel_sigir2023_b200.corpus import DeviceCorpus
-    dc = DeviceCorpus.from_columnar(columnar, "train", device)
+def _ragged(cols, seed=0):
+    """the synthetic corpus with every list cut to a random length in 1..L"""
+    L = int(cols["session_len"][0])
+    n = np.random.default_rng(seed).integers(1, L + 1, len(cols["session_len"]))
+    keep = (np.arange(L)[None, :] < n[:, None]).reshape(-1)
+    out = dict(cols, session_len=n.astype(np.int64), item_off=np.concatenate([[0], np.cumsum(n)]).astype(np.int64))
+    for k in ("item_id", "item_class", "ranking", "scores"):
+        out[k] = np.ascontiguousarray(cols[k][keep])
+    return out
+
+
+def test_default_shuffle_is_a_permutation_of_every_list(device):
+    from intel_sigir2023_b200.corpus import DeviceCorpus, synthetic_columns
+    cols, shared, nz = synthetic_columns(256, 40, 5000, 17, 30, 31, 3, 60, max_his=8, seed=1)
+    dc = DeviceCorpus(_ragged(cols), shared, 3, 60, 8, nz, device)
     rows = np.arange(100, 164)
     a = dc.batch(rows, shuffle=False)
     b = dc.batch(rows)
