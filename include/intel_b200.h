@@ -342,7 +342,8 @@ int intel_debug_use_fused_bert(int on);
 int intel_debug_gru_prep(int64_t B, int64_t T, const int64_t* lens, int32_t* order, int32_t* rows_t, int32_t* rows_t1,
                          int32_t* count, intel_stream_t stream);
 /* tuning / test hook: sessions that share one CTA (and one staged copy of the weights) in the fused stack
- * kernels, 1..4. */
+ * kernels, 1..4 (default 4).  The mma.sync forward kernel takes n as given; the backward kernel runs three sessions
+ * for n >= 3 where their tiles fit in shared memory (L <= 56) and two otherwise. */
 int intel_debug_stack_sessions_per_cta(int n);
 
 /* ---- building blocks exposed for unit tests --------------------------------------------- */

@@ -85,7 +85,8 @@ __device__ __forceinline__ void mma_ts(uint32_t d, uint32_t a, uint64_t b, uint3
 }
 
 // tensor memory <-> registers: the calling warp's 32 lanes, 32 consecutive columns, one row per thread.
-// ld32 does NOT wait: call wait_ld() before the registers are read.
+// ld32 does NOT wait: call wait_ld() before the registers are read.  ld8 / st8 (the parked weight-gradient and dQ | dK | dV
+// tiles of trunk_bwd_kernel) are covered by the GPU parity tests of that kernel rather than by the probe.
 __device__ __forceinline__ void ld32(uint32_t taddr, uint32_t (&r)[32]) {
     asm volatile(
         "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
@@ -117,6 +118,16 @@ __device__ __forceinline__ void st16(uint32_t taddr, const uint32_t (&r)[16]) {
         "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]),
         "r"(r[13]), "r"(r[14]), "r"(r[15])
         : "memory");
+}
+__device__ __forceinline__ void ld8(uint32_t taddr, uint32_t (&r)[8]) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+                 : "r"(taddr));
+}
+__device__ __forceinline__ void st8(uint32_t taddr, const uint32_t (&r)[8]) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]),
+                 "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
+                 : "memory");
 }
 __device__ __forceinline__ void wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 

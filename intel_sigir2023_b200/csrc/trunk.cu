@@ -10,6 +10,7 @@
 // Weight gradients stay in registers across all sessions of a CTA and are flushed once per CTA.
 #include "kernels.h"
 #include "mma.cuh"
+#include "tc05.cuh"
 
 namespace intel {
 
@@ -408,21 +409,25 @@ __global__ void __launch_bounds__(32 * MT * NS) trunk_fwd_kernel(TrunkArgs a) {
 }
 
 // ================================================================================================
-// Register-resident backward pass.  Four warps per session, two sessions per CTA (each with its own named
+// Register-resident backward pass.  Four warps per session, NS = 2 or 3 sessions per CTA (each with its own named
 // barrier).  Token-local work (LayerNorm, FFN and projection input gradients, the attention rows of a query
 // block) is done by the warp that owns the 16 tokens, on accumulator-layout registers as in the forward kernel.
 // Products that contract over the tokens of a session go through shared-memory tiles:
-//   region A: dF | dU tiles                 -> dW2 = dF^T relu(U), dW1 = dU^T A     (B operands read from HBM/L1)
 //   region B: K | V | Q | dA tiles          -> S, dP, dQ (row-local), dK = dS^T Q, dV = P^T dA (key-local)
-//   region C: P | dS of one head, later dQ | dK | dV tiles -> dWq/dWk/dWv = d{Q,K,V}^T X
-// Weight-gradient tiles are owned by fixed warps (2 tiles per matrix and warp) and live in registers across all
-// sessions of the CTA; each session's contribution is summed from zero and folded in with a rounded add.
-static const int BWD_NS = 2, BWD_WPS = 4;
+//   region C: first dF | dU tiles           -> dW2 = dF^T relu(U), dW1 = dU^T A     (B operands read from HBM/L1)
+//             then P | dS of one head, last dQ | dK | dV tiles -> dWq/dWk/dWv = d{Q,K,V}^T X
+// Weight-gradient tiles are owned by fixed warps (2 tiles per matrix and warp) and live across all sessions of the
+// CTA; each session's contribution is summed from zero and folded in with a rounded add.  They and the dQ | dK | dV
+// rows of the head loop are parked in tensor memory (Park below): at 168 registers three sessions (12 warps) fit an
+// SM, which hides more of the dependent-MMA latency this kernel waits on than 8 warps did.
+static const int BWD_WPS = 4;
+static const int kMaxSmemBytes = 227 * 1024;
 
 struct BwdPlan {
     int nkt, rows, ds, tile, ps, region_c, sess, off_cs, off_sess, total;     // in 4-byte words
+    bool fits() const { return (size_t)total * 4 <= (size_t)kMaxSmemBytes; }
 };
-__host__ __device__ inline BwdPlan bwd_plan(int L) {
+__host__ __device__ inline BwdPlan bwd_plan(int L, int ns) {
     BwdPlan p;
     p.nkt = (L + 7) >> 3;
     p.rows = 8 * p.nkt;
@@ -430,42 +435,69 @@ __host__ __device__ inline BwdPlan bwd_plan(int L) {
     p.tile = p.rows * WS;
     p.ps = p.rows * p.ds;
     p.region_c = 2 * p.ps > 3 * p.tile ? 2 * p.ps : 3 * p.tile;
-    p.sess = 6 * p.tile + p.region_c;
+    p.sess = 4 * p.tile + p.region_c;
     p.off_cs = 5 * TD * WS;                                  // after the five transposed weight planes
-    p.off_sess = p.off_cs + BWD_NS * BWD_WPS * 4 * TD;
-    p.total = p.off_sess + BWD_NS * p.sess;
+    p.off_sess = p.off_cs + ns * BWD_WPS * 4 * TD;
+    p.total = p.off_sess + ns * p.sess;
     return p;
 }
+
+// Per-thread values that live across much of the kernel but are touched rarely, parked in the thread's own lane of
+// tensor memory (the warp's 32-lane quarter): eight columns move per access, as two accumulator tiles.  tcgen05.ld /
+// st are warp-collective, so every access is warp-uniform.  The emulator has no tensor memory and keeps them in
+// registers, so that it runs the same kernel body.
+struct Park {
+    static constexpr int PW = 0, DQ = 40, DK = 56, DV = 72, COLS = 88;   // 5 weight-gradient tile pairs, dQ | dK | dV rows
+#ifdef INTEL_EMU
+    float r[COLS];
+    void get(float (*v)[4], int col) const {
+        for (int i = 0; i < 8; ++i) v[i >> 2][i & 3] = r[col + i];
+    }
+    void put(const float (*v)[4], int col) {
+        for (int i = 0; i < 8; ++i) r[col + i] = v[i >> 2][i & 3];
+    }
+#else
+    uint32_t base;                                                        // lane quarter + this warp's first column
+    __device__ __forceinline__ void get(float (*v)[4], int col) const {
+        uint32_t u[8];
+        tc05::wait_st();
+        tc05::ld8(base + col, u);
+        tc05::wait_ld();
+#pragma unroll
+        for (int i = 0; i < 8; ++i) v[i >> 2][i & 3] = __uint_as_float(u[i]);
+    }
+    __device__ __forceinline__ void put(const float (*v)[4], int col) {
+        uint32_t u[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) u[i] = __float_as_uint(v[i >> 2][i & 3]);
+        tc05::st8(base + col, u);
+    }
+#endif
+};
 
 // acc (16 x 8 NT) += A * B with B(k, n) = B[n * stride + k] read as fp32 and split here; tiles >= nlive are skipped
 template <int NT, int KS>
 __device__ __forceinline__ void mma_raw(float (&acc)[NT][4], const uint32_t (&ah)[KS][4], const uint32_t (&al)[KS][4],
                                         const float* __restrict__ B, int stride, int nlive, int lane) {
     const int off = (lane >> 2) * stride + 2 * (lane & 3);
-    float low[NT][4];
 #pragma unroll
-    for (int j = 0; j < NT; ++j)
+    for (int j = 0; j < NT; ++j) {                  // tile by tile: one small-term accumulator live instead of NT
+        if (j < nlive) {
+            float low[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
-        for (int c = 0; c < 4; ++c) low[j][c] = 0.f;
-#pragma unroll
-    for (int s = 0; s < KS; ++s) {
-#pragma unroll
-        for (int j = 0; j < NT; ++j) {
-            if (j < nlive) {
+            for (int s = 0; s < KS; ++s) {
                 const float2 v = *reinterpret_cast<const float2*>(B + off + j * 8 * stride + s * 8);
                 uint32_t bh[2], bl[2];
                 split_tf32(v.x, bh[0], bl[0]);
                 split_tf32(v.y, bh[1], bl[1]);
-                mma_tf32(low[j], al[s], bh);
-                mma_tf32(low[j], ah[s], bl);
+                mma_tf32(low, al[s], bh);
+                mma_tf32(low, ah[s], bl);
                 mma_tf32(acc[j], ah[s], bh);
             }
+#pragma unroll
+            for (int c = 0; c < 4; ++c) acc[j][c] += low[c];
         }
     }
-#pragma unroll
-    for (int j = 0; j < NT; ++j)
-#pragma unroll
-        for (int c = 0; c < 4; ++c) acc[j][c] += low[j][c];
 }
 
 // rows r0 / r1 of an accumulator-layout [16 x 32] block -> fp32 tile [rows][WS]
@@ -500,12 +532,19 @@ __device__ __forceinline__ void colsum_rows(float* slot, const float (&v)[4][4],
         }
 }
 
-// pw[a] (this warp's two 16x8 tiles of a 32x32 weight gradient) += T[a]^T B over the session's tokens, for NA
-// gradient tiles that share the B operand.  T[a]: shared tile [rows][WS] (m = T column), B: global rows of the
-// session [L][ldb] (n = B column), optional relu.  All B fragments are fetched before the first MMA so that the
+// rows r0 / r1 of a fp32 tile [rows][WS], columns col .. col + 7 -> accumulator layout (rows >= rows read as zero)
+__device__ __forceinline__ void get_tile(float (&v)[4], const float* T, int r0, int r1, int rows, int col, int t) {
+    const float2 lo = r0 < rows ? *reinterpret_cast<const float2*>(T + r0 * WS + col + 2 * t) : make_float2(0.f, 0.f);
+    const float2 hi = r1 < rows ? *reinterpret_cast<const float2*>(T + r1 * WS + col + 2 * t) : make_float2(0.f, 0.f);
+    v[0] = lo.x; v[1] = lo.y; v[2] = hi.x; v[3] = hi.y;
+}
+
+// parked tile pair pw + 8 a (this warp's two 16x8 tiles of a 32x32 weight gradient) += T[a]^T B over the session's
+// tokens, for NA gradient tiles that share the B operand.  T[a]: shared tile [rows][WS] (m = T column), B: global rows
+// of the session [L][ldb] (n = B column), optional relu.  All B fragments are fetched before the first MMA so that the
 // global-memory latency is paid once, not once per k-step.
 template <int NA, int NKT, bool RELU>
-__device__ __forceinline__ void wgrad_tiles(float (*pw)[2][4], const float* const (&T)[NA], const float* __restrict__ Bg, int ldb,
+__device__ __forceinline__ void wgrad_tiles(Park& park, int pw, const float* const (&T)[NA], const float* __restrict__ Bg, int ldb,
                                             int L, int nkt, int w, int lane) {
     const int g = lane >> 2, t = lane & 3;
     const int m0 = (w & 1) * 16 + g, n0 = (w >> 1) * 16 + g;
@@ -539,19 +578,23 @@ __device__ __forceinline__ void wgrad_tiles(float (*pw)[2][4], const float* cons
                 for (int n = 0; n < 2; ++n) mma_3xtf32(part[n], af, bv[s][n]);
             }
         }
+        float acc[2][4];
+        park.get(acc, pw + 8 * a);
 #pragma unroll
         for (int n = 0; n < 2; ++n)
 #pragma unroll
-            for (int c = 0; c < 4; ++c) pw[a][n][c] += part[n][c];
+            for (int c = 0; c < 4; ++c) acc[n][c] += part[n][c];
+        park.put(acc, pw + 8 * a);
     }
 }
 
-template <int MT, int DK>
-__global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(TrunkArgs a) {
+template <int MT, int DK, int NS>
+__global__ void __launch_bounds__(32 * NS * BWD_WPS, 1) trunk_bwd_kernel(TrunkArgs a) {
     constexpr int HEADS = TD / DK, KS = DK / 8, NKT = 2 * MT;
+    static_assert(KS % 2 == 0, "dQ | dK | dV rows are parked in pairs of accumulator tiles");
     DYN_SMEM(float, sm);
     const int L = a.L;
-    const BwdPlan pl = bwd_plan(L);
+    const BwdPlan pl = bwd_plan(L, NS);
     const int nkt = pl.nkt, rows = pl.rows, DS = pl.ds;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int slot = warp / BWD_WPS, w = warp % BWD_WPS;
@@ -560,14 +603,14 @@ __global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(Tru
     const float* WT = sm;                                   // transposed weights: WT[m][k_in * WS + n_out]
     float* cs = sm + pl.off_cs + warp * 4 * TD;             // this warp's column sums: db1 | db2 | dlnw | dlnb
     float* sess = sm + pl.off_sess + slot * pl.sess;
-    float* T_dF = sess;
-    float* T_dU = T_dF + pl.tile;
-    float* T_K = T_dU + pl.tile;
+    float* T_K = sess;
     float* T_V = T_K + pl.tile;
     float* T_Q = T_V + pl.tile;
     float* T_dA = T_Q + pl.tile;
     float* Ps = T_dA + pl.tile;                             // region C
     float* Ds = Ps + pl.ps;
+    float* T_dF = Ps;
+    float* T_dU = T_dF + pl.tile;
     float* T_dQ = Ps;
     float* T_dK = T_dQ + pl.tile;
     float* T_dV = T_dK + pl.tile;
@@ -575,28 +618,39 @@ __global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(Tru
         const float* src[5] = {a.wq, a.wk, a.wv, a.w1, a.w2};
         for (int m = 0; m < 5; ++m)
             for (int e = threadIdx.x; e < TD * TD; e += blockDim.x) sm[m * TD * WS + (e % TD) * WS + (e / TD)] = src[m][e];
-        for (int e = threadIdx.x; e < BWD_NS * BWD_WPS * 4 * TD; e += blockDim.x) sm[pl.off_cs + e] = 0.f;
+        for (int e = threadIdx.x; e < NS * BWD_WPS * 4 * TD; e += blockDim.x) sm[pl.off_cs + e] = 0.f;
     }
+    // tensor memory: the warps w of all sessions share lane quarter w, 128 columns per session
+    constexpr uint32_t TMEM_COLS = NS * 128 <= 256 ? 256 : 512;
+    static_assert(Park::COLS <= 128 && NS * 128 <= 512, "parked columns exceed tensor memory");
+    Park park;
+#ifdef INTEL_EMU
     __syncthreads();
+#else
+    __shared__ uint32_t tmem_slot;
+    if (warp == 0) tc05::tmem_alloc(&tmem_slot, TMEM_COLS);
+    tc05::fence_before();
+    __syncthreads();
+    tc05::fence_after();
+    park.base = tmem_slot + ((uint32_t)(w * 32) << 16) + (uint32_t)(slot * 128);
+#endif
     const float* lnw = a.lnw;
-    float pw[5][2][4];                                      // weight-gradient tiles: w2 w1 wq wk wv
+    {
+        const float zero[2][4] = {};                        // weight-gradient tiles: w2 w1 wq wk wv
 #pragma unroll
-    for (int m = 0; m < 5; ++m)
-#pragma unroll
-        for (int n = 0; n < 2; ++n)
-#pragma unroll
-            for (int c = 0; c < 4; ++c) pw[m][n][c] = 0.f;
+        for (int m = 0; m < 5; ++m) park.put(zero, Park::PW + 8 * m);
+    }
     const bool rowwarp = w < MT;                            // owns tokens 16 w .. 16 w + 15
     const int r0 = w * 16 + g, r1 = r0 + 8;
     const bool live0 = rowwarp && r0 < L, live1 = rowwarp && r1 < L;
     const int bar = 1 + slot;
 
-    for (int64_t b = (int64_t)blockIdx.x * BWD_NS + slot; b < a.B; b += (int64_t)gridDim.x * BWD_NS) {
+    for (int64_t b = (int64_t)blockIdx.x * NS + slot; b < a.B; b += (int64_t)gridDim.x * NS) {
         const int64_t row0 = b * L;
         float gx[4][4];                                     // d loss / d (layer output) of the warp's tokens
         get_rows(gx, a.dX, TD, row0 + r0, row0 + r1, live0, live1, t);
         for (int l = a.layers - 1; l >= 0; --l) {
-            float q[4][4], da[4][4];
+            float df[4][4];
             if (rowwarp) {
                 // ---- LayerNorm backward: gx <- dZ ----
                 {
@@ -636,7 +690,6 @@ __global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(Tru
                     }
                 }
                 // ---- FFN backward (token-local part): dF = dZ * dropout mask, dU = (dF W2) * (U > 0), dA = dU W1 ----
-                float df[4][4];
                 const Dropout& dr = a.drop[l];
 #pragma unroll
                 for (int j = 0; j < 4; ++j)
@@ -646,6 +699,9 @@ __global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(Tru
                         df[j][c] = gx[j][c] * dropout_scale(dr, row0 + r0, col, TD);
                         df[j][2 + c] = gx[j][2 + c] * dropout_scale(dr, row0 + r1, col, TD);
                     }
+            }
+            bar_sync(bar, 32 * BWD_WPS);                                                   // s0: region C is read (dQ | dK | dV)
+            if (rowwarp) {
                 put_tile(T_dF, df, r0, r1, rows, t);
                 colsum_rows(cs + TD, df, lane);
                 float du[4][4];
@@ -669,6 +725,7 @@ __global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(Tru
                 colsum_rows(cs, du, lane);
                 {
                     uint32_t uh[4][4], ul[4][4];
+                    float da[4][4];
 #pragma unroll
                     for (int s = 0; s < 4; ++s) c_to_a(du[s], uh[s], ul[s]);
 #pragma unroll
@@ -676,8 +733,8 @@ __global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(Tru
 #pragma unroll
                         for (int c = 0; c < 4; ++c) da[j][c] = 0.f;
                     mma_raw<4, 4>(da, uh, ul, WT + 3 * TD * WS, WS, 4, lane);
+                    put_tile(T_dA, da, r0, r1, rows, t);
                 }
-                put_tile(T_dA, da, r0, r1, rows, t);
                 // ---- the session's K, V, Q rows saved by the forward pass ----
                 {
                     float kv[4][4];
@@ -685,18 +742,18 @@ __global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(Tru
                     put_tile(T_K, kv, r0, r1, rows, t);
                     get_rows(kv, a.QKV[l] + 2 * TD, 3 * TD, row0 + r0, row0 + r1, live0, live1, t);
                     put_tile(T_V, kv, r0, r1, rows, t);
-                    get_rows(q, a.QKV[l], 3 * TD, row0 + r0, row0 + r1, live0, live1, t);
-                    put_tile(T_Q, q, r0, r1, rows, t);
+                    get_rows(kv, a.QKV[l], 3 * TD, row0 + r0, row0 + r1, live0, live1, t);
+                    put_tile(T_Q, kv, r0, r1, rows, t);
                 }
             }
-            bar_sync(bar, 32 * BWD_WPS);                                                   // s1: regions A and B are complete
+            bar_sync(bar, 32 * BWD_WPS);                                                   // s1: dF | dU and region B are complete
             {
                 const float* const t2[1] = {T_dF};
                 const float* const t1[1] = {T_dU};
-                wgrad_tiles<1, NKT, true>(pw + 0, t2, a.U[l] + row0 * TD, TD, L, nkt, w, lane);      // dW2 += dF^T relu(U)
-                wgrad_tiles<1, NKT, false>(pw + 1, t1, a.A[l] + row0 * TD, TD, L, nkt, w, lane);     // dW1 += dU^T A
+                wgrad_tiles<1, NKT, true>(park, Park::PW + 0, t2, a.U[l] + row0 * TD, TD, L, nkt, w, lane);    // dW2 += dF^T relu(U)
+                wgrad_tiles<1, NKT, false>(park, Park::PW + 8, t1, a.A[l] + row0 * TD, TD, L, nkt, w, lane);   // dW1 += dU^T A
             }
-            float dq[4][4], dk[4][4], dv[4][4];
+            bar_sync(bar, 32 * BWD_WPS);                                                   // s2: dF | dU are read, region C takes P | dS
 #pragma unroll
             for (int hd = 0; hd < HEADS; ++hd) {
                 const int ho = hd * DK;
@@ -710,10 +767,18 @@ __global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(Tru
                     {
                         uint32_t qh[KS][4], ql[KS][4];
 #pragma unroll
-                        for (int s = 0; s < KS; ++s) c_to_a(q[hd * KS + s], qh[s], ql[s]);
+                        for (int s = 0; s < KS; ++s) {
+                            float f[4];
+                            get_tile(f, T_Q, r0, r1, rows, ho + 8 * s, t);
+                            c_to_a(f, qh[s], ql[s]);
+                        }
                         mma_raw<NKT, KS>(p, qh, ql, T_K + ho, WS, nkt, lane);
 #pragma unroll
-                        for (int s = 0; s < KS; ++s) c_to_a(da[hd * KS + s], qh[s], ql[s]);
+                        for (int s = 0; s < KS; ++s) {
+                            float f[4];
+                            get_tile(f, T_dA, r0, r1, rows, ho + 8 * s, t);
+                            c_to_a(f, qh[s], ql[s]);
+                        }
                         mma_raw<NKT, KS>(dp, qh, ql, T_V + ho, WS, nkt, lane);
                     }
                     float m0 = -INFINITY, m1 = -INFINITY;
@@ -796,9 +861,12 @@ __global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(Tru
                         }
                     }
 #pragma unroll
-                    for (int n = 0; n < KS; ++n)
+                    for (int n = 0; n < KS; n += 2) {
+                        float d[2][4];
 #pragma unroll
-                        for (int c = 0; c < 4; ++c) dq[hd * KS + n][c] = qe[n][c] + qo[n][c];
+                        for (int c = 0; c < 4; ++c) { d[0][c] = qe[n][c] + qo[n][c]; d[1][c] = qe[n + 1][c] + qo[n + 1][c]; }
+                        park.put(d, Park::DQ + 4 * (hd * KS + n));
+                    }
                 }
                 bar_sync(bar, 32 * BWD_WPS);                                               // P / dS of every query row are visible
                 if (rowwarp) {
@@ -826,32 +894,35 @@ __global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(Tru
                         }
                     }
 #pragma unroll
-                    for (int n = 0; n < KS; ++n)
-#pragma unroll
-                        for (int c = 0; c < 4; ++c) { dk[hd * KS + n][c] = ke[n][c]; dv[hd * KS + n][c] = ve[n][c]; }
+                    for (int n = 0; n < KS; n += 2) {
+                        const float dk[2][4] = {{ke[n][0], ke[n][1], ke[n][2], ke[n][3]}, {ke[n + 1][0], ke[n + 1][1], ke[n + 1][2], ke[n + 1][3]}};
+                        const float dv[2][4] = {{ve[n][0], ve[n][1], ve[n][2], ve[n][3]}, {ve[n + 1][0], ve[n + 1][1], ve[n + 1][2], ve[n + 1][3]}};
+                        park.put(dk, Park::DK + 4 * (hd * KS + n));
+                        park.put(dv, Park::DV + 4 * (hd * KS + n));
+                    }
                 }
                 bar_sync(bar, 32 * BWD_WPS);                                               // region C may be overwritten
             }
             if (rowwarp) {
                 // ---- projections backward: dX = dQ Wq + dK Wk + dV Wv + dZ; dQ | dK | dV tiles for the weight gradients ----
-                put_tile(T_dQ, dq, r0, r1, rows, t);
-                put_tile(T_dK, dk, r0, r1, rows, t);
-                put_tile(T_dV, dv, r0, r1, rows, t);
-                uint32_t fh[4][4], fl[4][4];
+                float* const td[3] = {T_dQ, T_dK, T_dV};
+                const int col[3] = {Park::DQ, Park::DK, Park::DV};
 #pragma unroll
-                for (int s = 0; s < 4; ++s) c_to_a(dq[s], fh[s], fl[s]);
-                mma_raw<4, 4>(gx, fh, fl, WT + 0 * TD * WS, WS, 4, lane);
+                for (int m = 0; m < 3; ++m) {
+                    float d[4][4];
+                    park.get(d, col[m]);
+                    park.get(d + 2, col[m] + 8);
+                    put_tile(td[m], d, r0, r1, rows, t);
+                    uint32_t fh[4][4], fl[4][4];
 #pragma unroll
-                for (int s = 0; s < 4; ++s) c_to_a(dk[s], fh[s], fl[s]);
-                mma_raw<4, 4>(gx, fh, fl, WT + 1 * TD * WS, WS, 4, lane);
-#pragma unroll
-                for (int s = 0; s < 4; ++s) c_to_a(dv[s], fh[s], fl[s]);
-                mma_raw<4, 4>(gx, fh, fl, WT + 2 * TD * WS, WS, 4, lane);
+                    for (int s = 0; s < 4; ++s) c_to_a(d[s], fh[s], fl[s]);
+                    mma_raw<4, 4>(gx, fh, fl, WT + m * TD * WS, WS, 4, lane);
+                }
             }
             bar_sync(bar, 32 * BWD_WPS);                                                   // dQ | dK | dV tiles are complete
             {
                 const float* const tq[3] = {T_dQ, T_dK, T_dV};
-                wgrad_tiles<3, NKT, false>(pw + 2, tq, a.X[l] + row0 * TD, TD, L, nkt, w, lane);    // dW{q,k,v} += d{Q,K,V}^T X
+                wgrad_tiles<3, NKT, false>(park, Park::PW + 16, tq, a.X[l] + row0 * TD, TD, L, nkt, w, lane);   // dW{q,k,v} += d{Q,K,V}^T X
             }
         }
         if (rowwarp) {
@@ -862,24 +933,36 @@ __global__ void __launch_bounds__(32 * BWD_NS * BWD_WPS, 1) trunk_bwd_kernel(Tru
             }
         }
     }
-    // ---- flush: weight-gradient tiles straight from registers, vector gradients through the warp-private sums ----
+    // ---- flush: weight-gradient tiles straight from tensor memory, vector gradients through the warp-private sums ----
     {
         float* dst[5] = {a.gw2, a.gw1, a.gwq, a.gwk, a.gwv};
         const int m0 = (w & 1) * 16 + g, n0 = (w >> 1) * 16 + 2 * t;
 #pragma unroll
-        for (int m = 0; m < 5; ++m)
+        for (int m = 0; m < 5; ++m) {
+            float pw[2][4];
+            park.get(pw, Park::PW + 8 * m);
 #pragma unroll
             for (int n = 0; n < 2; ++n) {
-                atomicAdd(dst[m] + m0 * TD + n0 + 8 * n, pw[m][n][0]);
-                atomicAdd(dst[m] + m0 * TD + n0 + 8 * n + 1, pw[m][n][1]);
-                atomicAdd(dst[m] + (m0 + 8) * TD + n0 + 8 * n, pw[m][n][2]);
-                atomicAdd(dst[m] + (m0 + 8) * TD + n0 + 8 * n + 1, pw[m][n][3]);
+                atomicAdd(dst[m] + m0 * TD + n0 + 8 * n, pw[n][0]);
+                atomicAdd(dst[m] + m0 * TD + n0 + 8 * n + 1, pw[n][1]);
+                atomicAdd(dst[m] + (m0 + 8) * TD + n0 + 8 * n, pw[n][2]);
+                atomicAdd(dst[m] + (m0 + 8) * TD + n0 + 8 * n + 1, pw[n][3]);
             }
+        }
     }
+#ifndef INTEL_EMU
+    tc05::fence_before();
+#endif
     __syncthreads();
+#ifndef INTEL_EMU
+    if (warp == 0) {
+        tc05::fence_after();
+        tc05::tmem_free(tmem_slot, TMEM_COLS);
+    }
+#endif
     if (threadIdx.x < 4 * TD) {
         float v = 0.f;
-        for (int ww = 0; ww < BWD_NS * BWD_WPS; ++ww) v += sm[pl.off_cs + ww * 4 * TD + threadIdx.x];
+        for (int ww = 0; ww < NS * BWD_WPS; ++ww) v += sm[pl.off_cs + ww * 4 * TD + threadIdx.x];
         float* dst = threadIdx.x < TD ? a.gb1 : (threadIdx.x < 2 * TD ? a.gb2 : (threadIdx.x < 3 * TD ? a.glnw : a.glnb));
         atomicAdd(dst + (threadIdx.x & (TD - 1)), v);
     }
@@ -889,11 +972,11 @@ bool trunk_supported(int64_t L, int d, int heads, int layers) {
     return d == TD && L >= 1 && L <= 64 && layers >= 1 && layers <= 8 && (heads == 1 || heads == 2);
 }
 
-static int g_fwd_sessions_per_cta = 4;
+static int g_sessions_per_cta = 4;
 static int g_reserved_sms = 0, g_reserve_now = 0;
 void trunk_reserve_sms(int n) { g_reserved_sms = n < 0 ? 0 : (n > 64 ? 64 : n); }
 void trunk_reserve_apply(bool on) { g_reserve_now = on ? 1 : 0; }
-void trunk_debug_sessions_per_cta(int n) { g_fwd_sessions_per_cta = n < 1 ? 1 : (n > 4 ? 4 : n); }
+void trunk_debug_sessions_per_cta(int n) { g_sessions_per_cta = n < 1 ? 1 : (n > 4 ? 4 : n); }
 
 // algorithmic HBM bytes per token: the stack input (and dX in / out), and per layer the saved q|k|v (96), attention
 // output, FFN hidden, pre-LN sum, layer output (32 each) and LN statistics (2) that the forward pass writes when it
@@ -920,7 +1003,7 @@ static int trunk_fwd_launch(const TrunkArgs& a, cudaStream_t s) {
 
 template <int MT, int DK>
 static int trunk_fwd_sessions(const TrunkArgs& a, cudaStream_t s) {
-    switch (g_fwd_sessions_per_cta) {
+    switch (g_sessions_per_cta) {
         case 1: return trunk_fwd_launch<MT, DK, 1>(a, s);
         case 2: return trunk_fwd_launch<MT, DK, 2>(a, s);
         case 3: return trunk_fwd_launch<MT, DK, 3>(a, s);
@@ -928,18 +1011,25 @@ static int trunk_fwd_sessions(const TrunkArgs& a, cudaStream_t s) {
     }
 }
 
-template <int TP, int DK>
-static int trunk_launch(const TrunkArgs& a, bool bwd, cudaStream_t s) {
-    if (!bwd) return trunk_fwd_sessions<TP / 16, DK>(a, s);
-    const size_t smem = (size_t)bwd_plan(a.L).total * 4;
-    unsigned grid = stream_grid((a.B + BWD_NS - 1) / BWD_NS, 1);
+template <int TP, int DK, int NS>
+static int trunk_bwd_launch(const TrunkArgs& a, cudaStream_t s) {
+    const size_t smem = (size_t)bwd_plan(a.L, NS).total * 4;
+    unsigned grid = stream_grid((a.B + NS - 1) / NS, 1);
     if (g_reserve_now && grid > (unsigned)(kNumSMs - g_reserved_sms)) grid = (unsigned)(kNumSMs - g_reserved_sms);   // one CTA owns an SM
-    auto k = trunk_bwd_kernel<TP / 16, DK>;
+    auto k = trunk_bwd_kernel<TP / 16, DK, NS>;
     ensure_smem(k, smem);
-    LAUNCH(k, dim3(grid), dim3(32 * BWD_NS * BWD_WPS), smem, s, a);
+    LAUNCH(k, dim3(grid), dim3(32 * NS * BWD_WPS), smem, s, a);
     double bytes, flops;
     trunk_account(a, true, bytes, flops);
     return check_launch("trunk_bwd", bytes, flops);
+}
+
+template <int TP, int DK>
+static int trunk_launch(const TrunkArgs& a, bool bwd, cudaStream_t s) {
+    if (!bwd) return trunk_fwd_sessions<TP / 16, DK>(a, s);
+    // three sessions (12 warps) where their tiles fit in shared memory (L <= 56), two otherwise or when asked for
+    if (g_sessions_per_cta >= 3 && bwd_plan(a.L, 3).fits()) return trunk_bwd_launch<TP, DK, 3>(a, s);
+    return trunk_bwd_launch<TP, DK, 2>(a, s);
 }
 
 bool trunk_fwd_supported(int64_t L, int heads, int layers) {
