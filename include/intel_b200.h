@@ -163,6 +163,32 @@ int intel_ensemble_bwd_phase(const intel_dims_t* d, const intel_tensors_t* param
                              const float* intents, const float* d_weights, const float* d_ens,
                              intel_tensors_t* grads, float* d_intents_out,
                              void* workspace, size_t workspace_bytes, intel_stream_t stream, int phases);
+/* ---- sparse table gradients (IntEL sparse_grad = 1) ----------------------------------------------------
+ * Row set of one table for one step: the ascending unique ids in [0, table_rows) of ids_a [n_a] and ids_b [n_b] (either may
+ * be empty; other ids are skipped, as the dense scatter skips them).  row_slot: caller-owned device int32 [table_rows],
+ * zero-filled once before the first call; every call leaves all entries >= 0 and sets row_slot[id] = the position of id
+ * in the set for each id of the set.  rows_out: device int64 [>= min(table_rows, n_a + n_b)]; count_out: device int64 [1]
+ * receives U, the size of the set.  Deterministic.  Data-parallel callers pass the ids of all ranks. */
+size_t intel_rowset_workspace_bytes(int64_t table_rows);
+int intel_rowset_build(int64_t table_rows, const int64_t* ids_a, int64_t n_a, const int64_t* ids_b, int64_t n_b,
+                       int32_t* row_slot, int64_t* rows_out, int64_t* count_out, void* workspace, size_t workspace_bytes,
+                       intel_stream_t stream);
+/* The row_slot maps of the four embedding tables (any may be NULL: that table's gradient stays dense).  With a map, the
+ * table's gradient buffer in `grads` is the compact [U, d] block of its row set: row j holds the gradient of row
+ * rows_out[j].  Every id the batch feeds to that table must be in the set. */
+typedef struct {
+    const int32_t *iid, *item, *uid, *ctx;
+} intel_row_maps_t;
+/* intel_ensemble_bwd_phase / intel_intent_bwd writing the table gradients through the maps (maps NULL: the plain calls) */
+int intel_ensemble_bwd_phase_rows(const intel_dims_t* d, const intel_tensors_t* params, const intel_batch_t* batch,
+                                  const float* intents, const float* d_weights, const float* d_ens,
+                                  intel_tensors_t* grads, float* d_intents_out,
+                                  void* workspace, size_t workspace_bytes, intel_stream_t stream, int phases,
+                                  const intel_row_maps_t* maps);
+int intel_intent_bwd_rows(const intel_dims_t* d, const intel_tensors_t* params, const intel_batch_t* batch,
+                          const float* intents, const float* d_intents, const float* d_intents_extra,
+                          intel_tensors_t* grads, void* workspace, size_t workspace_bytes, intel_stream_t stream,
+                          const intel_row_maps_t* maps);
 /* Number of SMs (0..64) the persistent backward kernel of the self-attention stack leaves free when the SCORE phase is
  * called on its own, so that a collective launched on another stream finds room to run beside it.  Default 0. */
 int intel_reserve_sms(int n);
@@ -309,6 +335,14 @@ int intel_lambdarank_lambdas(int64_t B, int64_t L, const int64_t* ranking, const
 int intel_adam_step(int count, float* const* params, const float* const* grads, float* const* exp_avg,
                     float* const* exp_avg_sq, const int64_t* numel, const float* weight_decay, double lr, double beta1,
                     double beta2, double eps, int64_t step, intel_stream_t stream);
+
+/* Row-wise form for sparse gradients: tensor i updates rows[i][0..nrows[i]) (distinct) of params / exp_avg / exp_avg_sq
+ * ([*, dim[i]] row-major) with the compact gradient grads[i] [nrows[i], dim[i]], element by element as intel_adam_step
+ * would with that gradient; all other rows are left untouched.  rows / grads are device pointers in HOST arrays. */
+int intel_adam_rows_step(int count, float* const* params, float* const* exp_avg, float* const* exp_avg_sq,
+                         const int64_t* const* rows, const float* const* grads, const int64_t* nrows, const int32_t* dim,
+                         const float* weight_decay, double lr, double beta1, double beta2, double eps, int64_t step,
+                         intel_stream_t stream);
 
 /* ---- host-side input packing (no GPU work) ---------------------------------------------------
  * dense float64 [rows, I] host tensor (the reference's his_intents / his_item_int rows, collate_batch) -> the compact

@@ -16,8 +16,15 @@ from typing import Dict, Optional
 import torch
 import torch.nn as nn
 
-from . import _lib
+from . import _lib, optim
 from .config import IntelConfig
+
+# embedding tables that --sparse_grad 1 covers: parameter, the batch fields whose ids index it (the backward scatters from
+# exactly these), the row map's field in intel_row_maps_t
+SPARSE_TABLES = (("iid_embeddings.weight", ("i_id_s", "his_item_id"), "iid"),
+                 ("item_embeddings.weight", ("i_class_c",), "item"),
+                 ("uid_embeddings.weight", ("u_id_c",), "uid"),
+                 ("context_embeddings.weight", ("context_mh", "his_context_mh"), "ctx"))
 
 
 def _encoder_container(cfg: IntelConfig, d: int) -> nn.Module:
@@ -75,6 +82,60 @@ def _give_ws(model, t: torch.Tensor) -> None:
         pool.append(t)
 
 
+class _RowSets:
+    """The row sets of one training step (IntEL with sparse_grad = 1): per covered table the ascending unique ids the batch
+    feeds it, built on the device at the start of the forward pass.  The set sizes travel to pinned host memory behind an
+    event that backward waits on (it has long completed by then), so the step gains no host synchronisation."""
+
+    def __init__(self, model: "IntEL", batch: Dict[str, object], dev: torch.device, stream) -> None:
+        self.model, self.dev, self.stream = model, dev, stream
+        self.tables = []            # (parameter name, [id arrays], row count, rows buffer)
+        for name, keys, _ in SPARSE_TABLES:
+            if name not in model._param_names:
+                continue
+            ids = [batch[k].reshape(-1) for k in keys]
+            if model._gather_ids is not None:       # data parallel: the union over the ranks (dp.GradReducer)
+                ids = [model._gather_ids(torch.cat(ids))]
+            n_rows = model.get_parameter(name).shape[0]
+            rows = torch.empty(max(1, min(n_rows, sum(t.numel() for t in ids))), dtype=torch.int64, device=dev)
+            self.tables.append((name, ids, n_rows, rows))
+        self.count = torch.empty(len(self.tables), dtype=torch.int64, device=dev)
+        self.build()
+        self.host = torch.empty(len(self.tables), dtype=torch.int64, pin_memory=dev.type == "cuda")
+        self.host.copy_(self.count, non_blocking=True)
+        self.event = torch.cuda.Event() if dev.type == "cuda" else None
+        if self.event is not None:
+            self.event.record(torch.cuda.current_stream(dev))
+
+    def build(self) -> None:
+        """(Re)writes the rows buffers and the model's row -> slot maps; the result depends on the ids alone."""
+        lib, model = _lib.load(), self.model
+        for j, (name, ids, n_rows, rows) in enumerate(self.tables):
+            slot = model._row_slot.get(name)
+            if slot is None or slot.device != self.dev or slot.numel() != n_rows:
+                slot = model._row_slot[name] = torch.zeros(n_rows, dtype=torch.int32, device=self.dev)
+            ws = torch.empty(lib.intel_rowset_workspace_bytes(n_rows), dtype=torch.uint8, device=self.dev)
+            a, b = (ids + [None])[:2]
+            _lib.check(lib.intel_rowset_build(n_rows, _lib.ptr(a, torch.int64), a.numel(), _lib.ptr(b, torch.int64),
+                                              0 if b is None else b.numel(), _lib.ptr(slot), _lib.ptr(rows),
+                                              _lib.ptr(self.count[j:j + 1]), _lib.ptr(ws), ws.numel(), self.stream))
+        model._row_sets_current = self
+
+    def sizes(self) -> Dict[str, int]:
+        if self.event is not None:
+            self.event.synchronize()
+        if self.model._row_sets_current is not self:     # another training forward pass rewrote the shared maps since
+            self.build()
+        return {t[0]: int(u) for t, u in zip(self.tables, self.host.tolist())}
+
+    def maps(self) -> "_lib.RowMaps":
+        m = _lib.RowMaps()
+        for name, _, field in SPARSE_TABLES:
+            if any(t[0] == name for t in self.tables):
+                setattr(m, field, _lib.ptr(self.model._row_slot[name]))
+        return m
+
+
 class _IntelFn(torch.autograd.Function):
     """(parameters...) -> (weights, ens_score, intents); backward = ensemble_bwd then intent_bwd."""
 
@@ -99,6 +160,7 @@ class _IntelFn(torch.autograd.Function):
         ws_ens = _take_ws(model, lib.intel_ensemble_workspace_bytes(dims), dev)
         if model.validate_inputs:
             model._queue_input_check(lib, dims, bt, dev, stream)
+        row_sets = _RowSets(model, batch, dev, stream) if keep and cfg.sparse_grad else None
         intents = torch.empty(B, cfg.intent_num, dtype=torch.float32, device=dev)
         weights = torch.empty(B, L, cfg.model_num, dtype=torch.float32, device=dev)
         ens = torch.empty(B, L, dtype=torch.float32, device=dev)
@@ -111,6 +173,7 @@ class _IntelFn(torch.autograd.Function):
             ctx.model, ctx.batch, ctx.dims = model, batch, dims
             ctx.ws_int, ctx.ws_ens = ws_int, ws_ens
             ctx.params = params
+            ctx.row_sets = row_sets
             # `intents` is an output: holding it as a plain attribute would close a ctx -> tensor -> grad_fn -> ctx
             # cycle that only the cyclic GC frees, and every leaked step costs the allocator a fresh cudaMalloc.
             ctx.save_for_backward(intents)
@@ -135,6 +198,11 @@ class _IntelFn(torch.autograd.Function):
         # per-parameter gradients are 256-byte aligned views into it.  The score stream's parameters sit at the end: they
         # are the last gradients the pass below completes, so everything before `late` can be exchanged while they are
         # still being computed (dp.GradReducer installs model._early_reduce for that).
+        # sparse_grad: a covered table's gradient is the compact [U, d] block of its row set (the table writes all happen
+        # before the SCORE phase, so the blocks sit before `late` with the other early gradients)
+        row_sets = ctx.row_sets
+        U = row_sets.sizes() if row_sets is not None else {}
+        numel = [U[n] * p[0].numel() if n in U else p.numel() for n, p in zip(names, params)]
         late_names = model._late_grad_names
         pack = [n for n in model._packed_grad_names if n in names]
         rest = [n for n in names if n not in late_names and n not in pack]
@@ -147,22 +215,24 @@ class _IntelFn(torch.autograd.Function):
             # the three weights multiplied by the predicted intents sit back to back (no alignment gap): the library then
             # forms their gradients with one product (api_model.cu, intel_ensemble_bwd_phase)
             packed_next = names[i] in pack and names[i] != pack[-1]
-            total += params[i].numel() if packed_next else (params[i].numel() + 63) // 64 * 64
+            total += numel[i] if packed_next else (numel[i] + 63) // 64 * 64
         late = total if late is None else late
         flat = torch.zeros(total, dtype=torch.float32, device=dev)
-        grads = [flat[o:o + p.numel()].view(p.shape) for o, p in zip(offs, params)]
+        grads = [flat[o:o + n].view((U[k],) + p.shape[1:] if k in U else p.shape) for o, n, k, p in zip(offs, numel, names, params)]
         model._flat_grad = flat         # dp.GradReducer all-reduces this one buffer when the .grad tensors still alias it
         model._flat_late = late
         G = _lib.make_tensors(cfg, dict(zip(names, grads)))
         bt = _lib.make_batch(batch, cfg)
         stream = _lib.stream_ptr(dev)
+        maps = row_sets.maps() if row_sets is not None else None
         have_ens = d_weights is not None or d_ens is not None
         d_int_ens: Optional[torch.Tensor] = None
         dw = de = None
 
         def ens_bwd(phases: int) -> None:
-            _lib.check(lib.intel_ensemble_bwd_phase(dims, P, bt, _lib.ptr(intents), _lib.ptr(dw), _lib.ptr(de), G,
-                                                    _lib.ptr(d_int_ens), _lib.ptr(ctx.ws_ens), ctx.ws_ens.numel(), stream, phases))
+            _lib.check(lib.intel_ensemble_bwd_phase_rows(dims, P, bt, _lib.ptr(intents), _lib.ptr(dw), _lib.ptr(de), G,
+                                                         _lib.ptr(d_int_ens), _lib.ptr(ctx.ws_ens), ctx.ws_ens.numel(), stream,
+                                                         phases, maps))
 
         # order of the pass (SURVEY 8e): head + cross attentions (the gradient w.r.t. the predicted intents is final) ->
         # intent predictor -> item stack + embedding rows -> [every gradient but the score stream's is final] -> score stack
@@ -175,8 +245,8 @@ class _IntelFn(torch.autograd.Function):
         first = d_intents.contiguous() if d_intents is not None else d_int_ens
         extra = d_int_ens if d_intents is not None else None
         if first is not None:
-            _lib.check(lib.intel_intent_bwd(dims, P, bt, _lib.ptr(intents), _lib.ptr(first), _lib.ptr(extra), G,
-                                            _lib.ptr(ctx.ws_int), ctx.ws_int.numel(), stream))
+            _lib.check(lib.intel_intent_bwd_rows(dims, P, bt, _lib.ptr(intents), _lib.ptr(first), _lib.ptr(extra), G,
+                                                 _lib.ptr(ctx.ws_int), ctx.ws_int.numel(), stream, maps))
         if have_ens and not single:
             ens_bwd(_lib.ENS_BWD_ITEM)
         early = getattr(model, "_early_reduce", None)
@@ -186,7 +256,16 @@ class _IntelFn(torch.autograd.Function):
             ens_bwd(_lib.ENS_BWD_SCORE)
         _give_ws(model, ctx.ws_int)
         _give_ws(model, ctx.ws_ens)
-        ctx.ws_int = ctx.ws_ens = None
+        ctx.ws_int = ctx.ws_ens = ctx.row_sets = None
+        if row_sets is not None:
+            # COO gradients whose values are the compact blocks; optim.Adam recognises these indices as coalesced (autograd
+            # drops the flag on its way into .grad); the indices are valid by construction, so no invariant check
+            with torch.sparse.check_sparse_tensor_invariants(enable=False):
+                for name, _, _, rows in row_sets.tables:
+                    i = names.index(name)
+                    optim.note_coalesced_rows((id(model), name), rows)
+                    grads[i] = torch.sparse_coo_tensor(rows[:U[name]].view(1, -1), grads[i], size=params[i].shape,
+                                                       is_coalesced=True)
         return (None, None, None) + tuple(grads)
 
 
@@ -214,6 +293,8 @@ class IntEL(nn.Module):
         parser.add_argument('--model_path', type=str, default='', help='Model save path.')
         parser.add_argument('--buffer', type=int, default=1, help='Whether to buffer feed dicts for dev/test')
         parser.add_argument('--model_num', type=int, default=2, help='Number of base models.')
+        parser.add_argument('--sparse_grad', type=int, default=0,
+                            help='Row-sparse gradients for the embedding tables (needs optim.Adam: BaseRunner_b200).')
         return parser
 
     def __init__(self, args, corpus=None, cfg: Optional[IntelConfig] = None):
@@ -266,6 +347,11 @@ class IntEL(nn.Module):
         self._late_grad_names = {n for n in self._param_names
                                  if n.startswith(("s_attn_head.", "s_W1.", "s_W2.", "s_layer_norm.", "score_embeddings."))}
         self._early_reduce = None       # set by dp.GradReducer: callable(flat_grad, late_offset)
+        # sparse_grad: persistent row -> slot map per table (intel_rowset_build), the row sets of the last training forward
+        # pass, and dp.GradReducer's hook that gathers the ids of all ranks (every rank then builds the same row sets)
+        self._row_slot: Dict[str, torch.Tensor] = {}
+        self._row_sets_current = None
+        self._gather_ids = None
         # gradients kept back to back in the flat buffer, in the row order of the library's stacked weight (Wcat)
         self._packed_grad_names = (["intent_item_attention.query_layer.weight", "intent_score_attention.query_layer.weight",
                                     "intent_embeddings.weight"] if c.cross_attention else [])

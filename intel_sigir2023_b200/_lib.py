@@ -53,6 +53,10 @@ class Tensors(C.Structure):
                [("enc", Encoder), ("item_enc", Encoder), ("pred_w", _p), ("pred_b", _p)]
 
 
+class RowMaps(C.Structure):
+    _fields_ = [(n, _p) for n in ("iid", "item", "uid", "ctx")]
+
+
 class Batch(C.Structure):
     _fields_ = [(n, _p) for n in ("u_id", "i_id", "i_class", "session_len", "scores", "context_mh", "his_context",
                                   "his_intents", "history_len", "his_item_id", "his_item_int", "history_item_len",
@@ -68,7 +72,7 @@ _allow_host_tensors = False     # flipped only by tests/emu (kernel-logic emulat
 
 def _declare(lib: C.CDLL) -> None:
     i64, i32, dbl, sz = C.c_int64, C.c_int, C.c_double, C.c_size_t
-    PD, PT, PB = C.POINTER(Dims), C.POINTER(Tensors), C.POINTER(Batch)
+    PD, PT, PB, PM = C.POINTER(Dims), C.POINTER(Tensors), C.POINTER(Batch), C.POINTER(RowMaps)
     sig = {
         "intel_last_error": (C.c_char_p, []),
         "intel_abi_version": (i32, []),
@@ -79,6 +83,10 @@ def _declare(lib: C.CDLL) -> None:
         "intel_ensemble_fwd": (i32, [PD, PT, PB, _p, _p, _p, _p, sz, _p]),
         "intel_ensemble_bwd": (i32, [PD, PT, PB, _p, _p, _p, PT, _p, _p, sz, _p]),
         "intel_ensemble_bwd_phase": (i32, [PD, PT, PB, _p, _p, _p, PT, _p, _p, sz, _p, i32]),
+        "intel_ensemble_bwd_phase_rows": (i32, [PD, PT, PB, _p, _p, _p, PT, _p, _p, sz, _p, i32, PM]),
+        "intel_intent_bwd_rows": (i32, [PD, PT, PB, _p, _p, _p, PT, _p, sz, _p, PM]),
+        "intel_rowset_workspace_bytes": (sz, [i64]),
+        "intel_rowset_build": (i32, [i64, _p, i64, _p, i64, _p, _p, _p, _p, sz, _p]),
         "intel_reserve_sms": (i32, [i32]),
         "intel_loss_pl_fwd_bwd": (i32, [i64, i64, i64, _p, _p, _p, _p, _p, i32, dbl, _p, _p, _p, _p]),
         "intel_loss_bpr_fwd_bwd": (i32, [i64, i64, i64, _p, _p, _p, _p, _p, _p, C.c_uint64, i32, dbl, _p, _p, _p, _p]),
@@ -121,6 +129,7 @@ def _declare(lib: C.CDLL) -> None:
         "intel_pool_head_bwd": (i32, [i64, i64, i32, _p, _p, _p, _p, _p, _p, _p]),
         "intel_lambdarank_lambdas": (i32, [i64, i64, _p, _p, _p, _p, _p]),
         "intel_adam_step": (i32, [i32, _p, _p, _p, _p, _p, _p, dbl, dbl, dbl, dbl, i64, _p]),
+        "intel_adam_rows_step": (i32, [i32, _p, _p, _p, _p, _p, _p, _p, _p, dbl, dbl, dbl, dbl, i64, _p]),
         "intel_profile_enable": (i32, [i32]),
         "intel_profile_report": (i32, [C.c_char_p, sz]),
     }
@@ -140,7 +149,9 @@ EXPORTED = ["intel_ensemble_bwd_phase", "intel_reserve_sms", "intel_last_error",
             "intel_mha_bwd", "intel_debug_use_fused_stack", "intel_debug_stack_sessions_per_cta", "intel_debug_use_tcgen05_gemm", "intel_host_pack_rows", "intel_adam_step", "intel_awelv_fwd", "intel_awelv_bwd",
             "intel_lambdarank_lambdas", "intel_pool_head_fwd", "intel_pool_head_bwd",
             "intel_linear_fwd_ex", "intel_linear_dx_ex", "intel_linear_dw_ex", "intel_softmax_rows_fwd", "intel_softmax_rows_bwd",
-            "intel_batch_validate", "intel_debug_use_tcgen05_stack", "intel_batch_build", "intel_debug_use_tcgen05_gru", "intel_debug_use_rows_gemm", "intel_debug_gru_prep", "intel_debug_use_fused_bert"]
+            "intel_batch_validate", "intel_debug_use_tcgen05_stack", "intel_batch_build", "intel_debug_use_tcgen05_gru", "intel_debug_use_rows_gemm", "intel_debug_gru_prep", "intel_debug_use_fused_bert",
+            "intel_rowset_workspace_bytes", "intel_rowset_build", "intel_ensemble_bwd_phase_rows", "intel_intent_bwd_rows",
+            "intel_adam_rows_step"]
 
 
 def load(path: Optional[str] = None) -> C.CDLL:

@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 ROOT = os.path.dirname(HERE)
 LIB = os.path.join(HERE, "libintel_b200.so")
-SOURCES = ["batch.cu", "api_misc.cu", "api_model.cu", "attn.cu", "bert_fused.cu", "embed.cu", "eval.cu", "fuse.cu", "gemm.cu", "gemm_rows_tc.cu", "gemm_wgrad_tc.cu", "gru.cu", "gru_tc.cu", "host_pack.cu", "loss.cu", "mha.cu", "optim.cu", "trunk.cu", "trunk_tc.cu"]
+SOURCES = ["batch.cu", "api_misc.cu", "api_model.cu", "attn.cu", "bert_fused.cu", "embed.cu", "eval.cu", "fuse.cu", "gemm.cu", "gemm_rows_tc.cu", "gemm_wgrad_tc.cu", "gru.cu", "gru_tc.cu", "host_pack.cu", "loss.cu", "mha.cu", "optim.cu", "rowset.cu", "trunk.cu", "trunk_tc.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",

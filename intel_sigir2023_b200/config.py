@@ -36,6 +36,8 @@ class IntelConfig:
     gru_hidden: int = 128     # GRU4RecEncoder(hidden_size=128)  (IntEL.py:105-106)
     bert_layers: int = 2      # BERT4RecEncoder(num_layers=2, num_heads=2) (IntEL.py:108-109)
     bert_heads: int = 2
+    # --sparse_grad 1: the four embedding tables get row-sparse (COO) gradients over the rows a step names
+    sparse_grad: int = 0
 
     # ---- derived widths ----
     @property
@@ -81,7 +83,7 @@ class IntelConfig:
             intent_emb_size=g("intent_emb_size", 16), cross_attn_qsize=g("cross_attn_qsize", 32),
             num_heads=g("num_heads", 1), num_layers=g("num_layers", 1),
             cross_attention=int(g("cross_attention", 1)), dropout=float(g("dropout", 0.0)),
-            history_max=int(g("history_max", 20)))
+            history_max=int(g("history_max", 20)), sparse_grad=int(g("sparse_grad", 0)))
 
     def to_dict(self) -> Dict[str, object]:
         return asdict(self)

@@ -583,10 +583,12 @@ int intel_ensemble_fwd(const intel_dims_t* d, const intel_tensors_t* P, const in
 // final afterwards, d(stack output) of each stream is left in the workspace), ITEM / SCORE = the self-attention stack of
 // one stream and the gradients of its inputs.  A data-parallel caller runs HEAD, intel_intent_bwd, ITEM - after which every
 // gradient except the score stream's is final and can be exchanged - and hides that exchange behind SCORE.
-int intel_ensemble_bwd_phase(const intel_dims_t* d, const intel_tensors_t* P, const intel_batch_t* bt, const float* intents,
-                             const float* d_weights, const float* d_ens, intel_tensors_t* G, float* d_intents_out,
-                             void* workspace, size_t workspace_bytes, intel_stream_t stream, int phases) {
+int intel_ensemble_bwd_phase_rows(const intel_dims_t* d, const intel_tensors_t* P, const intel_batch_t* bt, const float* intents,
+                                  const float* d_weights, const float* d_ens, intel_tensors_t* G, float* d_intents_out,
+                                  void* workspace, size_t workspace_bytes, intel_stream_t stream, int phases,
+                                  const intel_row_maps_t* maps) {
     INTEL_TRY(check_dims(d));
+    const intel_row_maps_t M = maps ? *maps : intel_row_maps_t{};
     INTEL_REQUIRE(phases > 0 && phases < 8, INTEL_ERR_ARG, "ensemble_bwd: phases must be a combination of INTEL_ENS_BWD_*");
     const bool do_head = phases & INTEL_ENS_BWD_HEAD, do_item = phases & INTEL_ENS_BWD_ITEM, do_score = phases & INTEL_ENS_BWD_SCORE;
     INTEL_REQUIRE(P && bt && intents && G && d_intents_out, INTEL_ERR_ARG, "ensemble_bwd: null argument");
@@ -619,7 +621,7 @@ int intel_ensemble_bwd_phase(const intel_dims_t* d, const intel_tensors_t* P, co
         const int dc = di + ds + dint;
         INTEL_TRY(relu_bwd(B, dint, w.dall + off_h, D, w.all + off_h, D, w.dcat + di + ds, dc, s));
         // h_u = relu(uid_embeddings[u])
-        INTEL_TRY(scatter_add_rows(B, du, w.dall + off_u, D, bt->u_id, G->uid_emb, P->uid_emb, s, d->user_rows));
+        INTEL_TRY(scatter_add_rows(B, du, w.dall + off_u, D, bt->u_id, G->uid_emb, P->uid_emb, s, d->user_rows, M.uid));
         // the two pooled cross attentions
         for (int st = 0; st < 2; ++st) {
             const int dd = st == 0 ? di : ds;
@@ -670,7 +672,7 @@ int intel_ensemble_bwd_phase(const intel_dims_t* d, const intel_tensors_t* P, co
         INTEL_TRY(linear_dw(B, dint, I, w.dvec, dint, intents, I, G->intent_w, I, G->intent_b, s));
         INTEL_TRY(linear_dx(B, dint, I, w.dvec, dint, P->intent_w, I, d_intents_out, I, s, 0));
         INTEL_TRY(bcast_rows_bwd(B, L, du, w.dall_item + off_u, D, w.dvec, du, 0, s));
-        INTEL_TRY(scatter_add_rows(B, du, w.dvec, du, bt->u_id, G->uid_emb, P->uid_emb, s, d->user_rows));
+        INTEL_TRY(scatter_add_rows(B, du, w.dvec, du, bt->u_id, G->uid_emb, P->uid_emb, s, d->user_rows, M.uid));
         for (int st = 0; st < 2; ++st) {
             const int dd = st == 0 ? di : ds;
             const int off = st == 0 ? 0 : di;
@@ -691,8 +693,9 @@ int intel_ensemble_bwd_phase(const intel_dims_t* d, const intel_tensors_t* P, co
     if (do_item) {
         INTEL_TRY(stack_bwd(B, L, di, d->heads, d->layers, P->item, G->item, w.item, w.dXa, w.t1, w.t2, w.dqkv, d->dropout_p,
                             d->dropout_seed, 0, s));
-        INTEL_TRY(scatter_add_rows(R, d->d_iid, w.dXa, di, bt->i_id, G->iid_emb, nullptr, s, d->item_rows));
-        if (d->d_im > 0) INTEL_TRY(scatter_add_rows(R, d->d_im, w.dXa + d->d_iid, di, bt->i_class, G->item_emb, nullptr, s, d->class_rows));
+        INTEL_TRY(scatter_add_rows(R, d->d_iid, w.dXa, di, bt->i_id, G->iid_emb, nullptr, s, d->item_rows, M.iid));
+        if (d->d_im > 0)
+            INTEL_TRY(scatter_add_rows(R, d->d_im, w.dXa + d->d_iid, di, bt->i_class, G->item_emb, nullptr, s, d->class_rows, M.item));
     }
     if (do_score) {
         // run on its own, this phase is the one a caller overlaps with its gradient exchange: leave the reserved SMs free
@@ -705,6 +708,13 @@ int intel_ensemble_bwd_phase(const intel_dims_t* d, const intel_tensors_t* P, co
         else INTEL_TRY(linear_dw(R, ds, K, w.dXs, ds, w.xs, K, G->score_w, K, G->score_b, s));
     }
     return INTEL_OK;
+}
+
+int intel_ensemble_bwd_phase(const intel_dims_t* d, const intel_tensors_t* P, const intel_batch_t* bt, const float* intents,
+                             const float* d_weights, const float* d_ens, intel_tensors_t* G, float* d_intents_out,
+                             void* workspace, size_t workspace_bytes, intel_stream_t stream, int phases) {
+    return intel_ensemble_bwd_phase_rows(d, P, bt, intents, d_weights, d_ens, G, d_intents_out, workspace, workspace_bytes, stream,
+                                         phases, nullptr);
 }
 
 int intel_ensemble_bwd(const intel_dims_t* d, const intel_tensors_t* P, const intel_batch_t* bt, const float* intents,
@@ -776,10 +786,11 @@ int intel_intent_fwd(const intel_dims_t* d, const intel_tensors_t* P, const inte
     return softmax_rows(B, I, w.logits, intents_out, s, pad4(I));
 }
 
-int intel_intent_bwd(const intel_dims_t* d, const intel_tensors_t* P, const intel_batch_t* bt, const float* intents,
-                     const float* d_intents, const float* d_intents_extra, intel_tensors_t* G, void* workspace,
-                     size_t workspace_bytes, intel_stream_t stream) {
+int intel_intent_bwd_rows(const intel_dims_t* d, const intel_tensors_t* P, const intel_batch_t* bt, const float* intents,
+                          const float* d_intents, const float* d_intents_extra, intel_tensors_t* G, void* workspace,
+                          size_t workspace_bytes, intel_stream_t stream, const intel_row_maps_t* maps) {
     INTEL_TRY(check_dims(d));
+    const intel_row_maps_t M = maps ? *maps : intel_row_maps_t{};
     INTEL_REQUIRE(P && bt && intents && d_intents && G, INTEL_ERR_ARG, "intent_bwd: null argument");
     Arena a(workspace, workspace_bytes);
     IntWs w;
@@ -794,8 +805,8 @@ int intel_intent_bwd(const intel_dims_t* d, const intel_tensors_t* P, const inte
     INTEL_TRY(softmax_rows_bwd(B, I, intents, d_intents, d_intents_extra, w.dlogits, s, pad4(I)));
     INTEL_TRY(linear_dw(B, I, Dp, w.dlogits, pad4(I), w.feat, Dp, G->pred_w, Dp, G->pred_b, s));
     INTEL_TRY(linear_dx(B, I, Dp, w.dlogits, pad4(I), P->pred_w, Dp, w.dfeat, Dp, s));
-    INTEL_TRY(scatter_add_rows(B, dctx, w.dfeat, Dp, bt->context_mh, G->ctx_emb, nullptr, s, d->ctx_rows));
-    INTEL_TRY(scatter_add_rows(B, du, w.dfeat + dctx, Dp, bt->u_id, G->uid_emb, nullptr, s, d->user_rows));
+    INTEL_TRY(scatter_add_rows(B, dctx, w.dfeat, Dp, bt->context_mh, G->ctx_emb, nullptr, s, d->ctx_rows, M.ctx));
+    INTEL_TRY(scatter_add_rows(B, du, w.dfeat + dctx, Dp, bt->u_id, G->uid_emb, nullptr, s, d->user_rows, M.uid));
     if (d->encoder == INTEL_ENCODER_BERT4REC) {
         INTEL_TRY(bert_bwd(d, P->enc, G->enc, w.e1, bt->history_len, w.dfeat + off_v1, Dp, w.t1, w.t2, w.dqkv, s));
         INTEL_TRY(bert_bwd(d, P->item_enc, G->item_enc, w.e2, bt->history_item_len, w.dfeat + off_v2, Dp, w.t1, w.t2, w.dqkv, s));
@@ -814,7 +825,7 @@ int intel_intent_bwd(const intel_dims_t* d, const intel_tensors_t* P, const inte
         INTEL_TRY(gru_bwd(d, P->item_enc, G->item_enc, w.e2, bt->history_item_len, w.dfeat + off_v2, Dp, s, have_dh));
     }
     INTEL_TRY(fill_zero(w.dWt, (size_t)I * dint * 4, s));
-    INTEL_TRY(scatter_add_rows(B * d->H1, dctx, w.e1.dseq, d1, bt->his_context, G->ctx_emb, nullptr, s, d->ctx_rows));
+    INTEL_TRY(scatter_add_rows(B * d->H1, dctx, w.e1.dseq, d1, bt->his_context, G->ctx_emb, nullptr, s, d->ctx_rows, M.ctx));
     if (bt->his_intents_idx) {
         INTEL_TRY(dense_rows_linear_bwd(B * d->H1, I, dint, nullptr, w.e1.dseq + dctx, d1, bt->his_intents_idx,
                                         bt->his_intents_val, nullptr, bt->nz1, w.dWt, s, G->intent_b));
@@ -822,7 +833,7 @@ int intel_intent_bwd(const intel_dims_t* d, const intel_tensors_t* P, const inte
         INTEL_TRY(dense_rows_linear_bwd(B * d->H1, I, dint, bt->his_intents, w.e1.dseq + dctx, d1, w.e1.nz_idx, w.e1.nz_val,
                                         w.e1.nz_cnt, NZ_CAP, w.dWt, s, G->intent_b));      // + the bias gradient (column sums)
     }
-    INTEL_TRY(scatter_add_rows(B * d->H2, diid, w.e2.dseq, d2, bt->his_item_id, G->iid_emb, nullptr, s, d->item_rows));
+    INTEL_TRY(scatter_add_rows(B * d->H2, diid, w.e2.dseq, d2, bt->his_item_id, G->iid_emb, nullptr, s, d->item_rows, M.iid));
     if (bt->his_item_int_idx) {
         INTEL_TRY(dense_rows_linear_bwd(B * d->H2, I, dint, nullptr, w.e2.dseq + diid, d2, bt->his_item_int_idx,
                                         bt->his_item_int_val, nullptr, bt->nz2, w.dWt, s, G->intent_b));
@@ -831,6 +842,12 @@ int intel_intent_bwd(const intel_dims_t* d, const intel_tensors_t* P, const inte
                                         w.e2.nz_cnt, NZ_CAP, w.dWt, s, G->intent_b));
     }
     return transpose(I, dint, w.dWt, G->intent_w, 1, s);
+}
+
+int intel_intent_bwd(const intel_dims_t* d, const intel_tensors_t* P, const intel_batch_t* bt, const float* intents,
+                     const float* d_intents, const float* d_intents_extra, intel_tensors_t* G, void* workspace,
+                     size_t workspace_bytes, intel_stream_t stream) {
+    return intel_intent_bwd_rows(d, P, bt, intents, d_intents, d_intents_extra, G, workspace, workspace_bytes, stream, nullptr);
 }
 
 }  // extern "C"

@@ -44,10 +44,13 @@ int gather_rows(int64_t rows, int d, const float* table, const int64_t* idx, flo
 
 // scatter-add: grad_table[idx[r], :] += d_out[r, :]   (embedding_dense_backward; the gradient stays
 // DENSE so torch.optim.Adam(weight_decay) is a drop-in).  fp32 atomics.
+// REMAP (sparse table gradients, sparse.cu): the destination row is slot[idx[r]], a row of the compact [U, d] gradient of
+// the step's row set; the ReLU gate still reads the parameter row of the original id.
+template <bool REMAP>
 __global__ void __launch_bounds__(256) scatter_add_kernel(int64_t rows, int d, const float* __restrict__ d_out,
                                                           int64_t ld, const int64_t* __restrict__ idx,
                                                           float* grad_table, const float* __restrict__ relu_table,
-                                                          int64_t table_rows) {
+                                                          int64_t table_rows, const int32_t* __restrict__ slot) {
     const int64_t total = rows * d;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
         const int64_t r = e / d;
@@ -56,16 +59,24 @@ __global__ void __launch_bounds__(256) scatter_add_kernel(int64_t rows, int d, c
         if (table_rows > 0 && (id < 0 || id >= table_rows)) continue;      // would land in another parameter's gradient
         float g = d_out[r * ld + c];
         if (relu_table && !(relu_table[id * d + c] > 0.f)) g = 0.f;
-        if (g != 0.f) atomicAdd(grad_table + id * d + c, g);
+        const int64_t dst = REMAP ? (int64_t)slot[id] : id;
+        if (g != 0.f) atomicAdd(grad_table + dst * d + c, g);
     }
 }
 
 int scatter_add_rows(int64_t rows, int d, const float* d_out, int64_t ld, const int64_t* idx, float* grad_table,
-                     const float* relu_table, cudaStream_t s, int64_t table_rows) {
+                     const float* relu_table, cudaStream_t s, int64_t table_rows, const int32_t* slot) {
     if (rows <= 0 || d <= 0) return INTEL_OK;
     INTEL_REQUIRE(d_out && idx && grad_table, INTEL_ERR_ARG, "scatter_add: null pointer");
+    INTEL_REQUIRE(!slot || table_rows > 0, INTEL_ERR_ARG, "scatter_add: a row-slot map needs the table's row count");
     unsigned grid = stream_grid(ceil_div(rows * d, 256), 8);
-    LAUNCH(scatter_add_kernel, dim3(grid), dim3(256), 0, s, rows, d, d_out, ld, idx, grad_table, relu_table, table_rows);
+    if (slot) {
+        auto k = scatter_add_kernel<true>;
+        LAUNCH(k, dim3(grid), dim3(256), 0, s, rows, d, d_out, ld, idx, grad_table, relu_table, table_rows, slot);
+    } else {
+        auto k = scatter_add_kernel<false>;
+        LAUNCH(k, dim3(grid), dim3(256), 0, s, rows, d, d_out, ld, idx, grad_table, relu_table, table_rows, slot);
+    }
     return check_launch("scatter_add", (double)rows * (12.0 * d + 8.0), (double)rows * d);
 }
 

@@ -51,9 +51,10 @@ int colsum(int64_t M, int64_t N, const float* X, int64_t ld, float* out, cudaStr
 // error itself is reported by batch_validate)
 int gather_rows(int64_t rows, int d, const float* table, const int64_t* idx, float* out, int64_t ld_out,
                 int relu, cudaStream_t s, int64_t table_rows = 0);
-// grad_table[idx[r]] += d_out[r] (* (table[idx[r]] > 0) when relu_table != null)
+// grad_table[idx[r]] += d_out[r] (* (table[idx[r]] > 0) when relu_table != null); slot != null: the destination row is
+// slot[idx[r]] (the compact gradient of a row set, sparse.cu)
 int scatter_add_rows(int64_t rows, int d, const float* d_out, int64_t ld, const int64_t* idx, float* grad_table,
-                     const float* relu_table, cudaStream_t s, int64_t table_rows = 0);
+                     const float* relu_table, cudaStream_t s, int64_t table_rows = 0, const int32_t* slot = nullptr);
 // ORs a bit into flags[0] for every class of out-of-range input (bit values: INTEL_BAD_* of intel_b200.h)
 struct ValidateArgs {
     int64_t B, L, H1, H2, I, item_rows, class_rows, user_rows, ctx_rows;

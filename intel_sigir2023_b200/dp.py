@@ -32,6 +32,11 @@ def configure_nccl_for_overlap(sms: int = OVERLAP_SMS) -> None:
     os.environ.setdefault("NCCL_CGA_CLUSTER_SIZE", "0")
 
 
+def _buffer_ptr(g: torch.Tensor) -> int:
+    """storage of a gradient (the values of a sparse one)"""
+    return (g._values() if g.is_sparse else g).untyped_storage().data_ptr()
+
+
 class GradReducer:
     """Average the dense ``.grad`` buffers over the ranks after backward.
 
@@ -41,7 +46,11 @@ class GradReducer:
     backward kernel, which leaves ``overlap_sms`` SMs free for it; ``allreduce()`` then exchanges the small tail and
     joins.  This needs ``p.grad is None`` before backward (``zero_grad(set_to_none=True)``, the torch default): gradient
     accumulation into existing ``.grad`` tensors is refused loudly.  Without the flat buffer (other models) the few
-    large tensors are reduced in place, one collective each, and the small ones travel in one flat bucket."""
+    large tensors are reduced in place, one collective each, and the small ones travel in one flat bucket.
+
+    With ``IntEL(sparse_grad=1)`` the reducer also makes every rank build the same row sets: the model's forward pass
+    all-gathers each table's ids (``_gather_ids``) and builds the union, so the compact table gradients in the flat
+    buffer line up row for row across the ranks and the same all-reduce averages them."""
 
     def __init__(self, model: torch.nn.Module, world: int, small_numel: int = 1 << 16, overlap: bool = True,
                  overlap_sms: Optional[int] = None):
@@ -55,6 +64,8 @@ class GradReducer:
         self._pending = None
         self.overlap = (bool(overlap) and world > 1 and hasattr(model, "_early_reduce")
                         and os.environ.get("INTEL_DP_OVERLAP", "1") != "0")      # the environment switch is for A/B timing
+        if world > 1 and hasattr(model, "_gather_ids"):
+            model._gather_ids = self._gather_ids
         if self.overlap:
             model._early_reduce = self._early
             if backend == "nccl":
@@ -67,6 +78,12 @@ class GradReducer:
         if late > 0:
             self._pending = (dist.all_reduce(flat[:late], op=self.avg_op, async_op=True), flat, late)
 
+    def _gather_ids(self, ids: torch.Tensor) -> torch.Tensor:
+        """ids of every rank, concatenated (the shards have equal shapes: synthetic.shard_batch)"""
+        parts = [torch.empty_like(ids) for _ in range(self.world)]
+        dist.all_gather(parts, ids.contiguous())
+        return torch.cat(parts)
+
     def allreduce(self) -> None:
         if self.world <= 1:
             return
@@ -75,7 +92,7 @@ class GradReducer:
         if pending is not None:
             work, flat, late = pending
             base = flat.untyped_storage().data_ptr()
-            if len(grads) != len(self.params) or any(g.untyped_storage().data_ptr() != base for g in grads):
+            if len(grads) != len(self.params) or any(_buffer_ptr(g) != base for g in grads):
                 work.wait()
                 raise RuntimeError("GradReducer(overlap=True): the .grad tensors do not alias the flat gradient buffer of this "
                                    "backward pass (gradient accumulation into existing .grad?); clear them with "
@@ -91,11 +108,14 @@ class GradReducer:
         flat = getattr(self.model, "_flat_grad", None)
         if flat is not None and grads and len(grads) == len(self.params):
             base = flat.untyped_storage().data_ptr()
-            if all(g.untyped_storage().data_ptr() == base for g in grads):
+            if all(_buffer_ptr(g) == base for g in grads):
                 dist.all_reduce(flat, op=self.avg_op)
                 if self.post_scale != 1.0:
                     flat.mul_(self.post_scale)
                 return
+        if any(g.is_sparse for g in grads):
+            raise RuntimeError("GradReducer: sparse table gradients are exchanged only inside the flat gradient buffer of the "
+                               "backward pass that produced them")
         big = [g for g in grads if g.numel() > self.small_numel]
         small = [g for g in grads if g.numel() <= self.small_numel]
         works = [dist.all_reduce(g, op=self.avg_op, async_op=True) for g in big]
