@@ -344,6 +344,29 @@ int intel_adam_rows_step(int count, float* const* params, float* const* exp_avg,
                          const float* weight_decay, double lr, double beta1, double beta2, double eps, int64_t step,
                          intel_stream_t stream);
 
+/* Exact row-wise form (IntEL sparse_grad = 2): the zero-gradient updates that dense Adam gives the rows a step does not
+ * name are deferred, and replayed in order through the same per-element arithmetic when the row is next updated or read,
+ * so the result is bitwise intel_adam_step's.  Per tensor the caller owns (the library allocates nothing):
+ *   n_updates[i]  the number of updates recorded since the bookkeeping was last reset, this step's included;
+ *   hist[i]       device float [>= n, 8]: entry k holds the scalars of update k + 1 (lr / (1 - beta1^step),
+ *                 sqrt(1 - beta2^step), beta2, eps, 1 - beta1, 1 - beta2, weight decay, 0);
+ *   done[i]       device int32 [table rows], zero-filled before the first update: how many of the n updates row r has
+ *                 received.  Invariant: row r of params / exp_avg / exp_avg_sq equals dense Adam after done[r] updates.
+ * The step replays updates done[r] + 1 .. n - 1 on each listed row with a +0.0 gradient, applies update n with the row's
+ * gradient, sets done[r] = n and stores update n's scalars to hist[n - 1].  A tensor with nrows[i] = 0 still records its
+ * update.  rows / grads / done / hist are device pointers in HOST arrays. */
+int intel_adam_deferred_rows_step(int count, float* const* params, float* const* exp_avg, float* const* exp_avg_sq,
+                                  const int64_t* const* rows, const float* const* grads, const int64_t* nrows, const int32_t* dim,
+                                  const float* weight_decay, int32_t* const* done, float* const* hist, const int32_t* n_updates,
+                                  double lr, double beta1, double beta2, double eps, int64_t step, intel_stream_t stream);
+/* Brings rows up to date (all n_updates[i] updates) without a new update.  rows[i] non-NULL: the first *row_count[i]
+ * (a device int64, at most nrows[i]) distinct rows of rows[i], each left with done[r] = n.  rows[i] NULL: every one of the
+ * nrows[i] rows of the table (a flush); done is then reset to 0 everywhere, and the caller restarts its count at 0. */
+int intel_adam_deferred_catch_up(int count, float* const* params, float* const* exp_avg, float* const* exp_avg_sq,
+                                 const int64_t* const* rows, const int64_t* const* row_count, const int64_t* nrows,
+                                 const int32_t* dim, int32_t* const* done, const float* const* hist, const int32_t* n_updates,
+                                 intel_stream_t stream);
+
 /* ---- host-side input packing (no GPU work) ---------------------------------------------------
  * dense float64 [rows, I] host tensor (the reference's his_intents / his_item_int rows, collate_batch) -> the compact
  * form of intel_batch_t: idx int32 [rows, nz], val float32 [rows, nz], zero padded, both in host memory (pinned for

@@ -19,7 +19,7 @@ import torch.nn as nn
 from . import _lib, optim
 from .config import IntelConfig
 
-# embedding tables that --sparse_grad 1 covers: parameter, the batch fields whose ids index it (the backward scatters from
+# embedding tables that --sparse_grad 1 and 2 cover: parameter, the batch fields whose ids index it (the backward scatters from
 # exactly these), the row map's field in intel_row_maps_t
 SPARSE_TABLES = (("iid_embeddings.weight", ("i_id_s", "his_item_id"), "iid"),
                  ("item_embeddings.weight", ("i_class_c",), "item"),
@@ -83,9 +83,10 @@ def _give_ws(model, t: torch.Tensor) -> None:
 
 
 class _RowSets:
-    """The row sets of one training step (IntEL with sparse_grad = 1): per covered table the ascending unique ids the batch
-    feeds it, built on the device at the start of the forward pass.  The set sizes travel to pinned host memory behind an
-    event that backward waits on (it has long completed by then), so the step gains no host synchronisation."""
+    """The row sets of one training step (IntEL with sparse_grad = 1 or 2): per covered table the ascending unique ids the
+    batch feeds it, built on the device at the start of the forward pass.  The set sizes travel to pinned host memory behind
+    an event that backward waits on (it has long completed by then), so the step gains no host synchronisation.  With
+    sparse_grad = 2 the rows of each set are brought up to date (optim.catch_up) before any kernel reads the tables."""
 
     def __init__(self, model: "IntEL", batch: Dict[str, object], dev: torch.device, stream) -> None:
         self.model, self.dev, self.stream = model, dev, stream
@@ -101,6 +102,9 @@ class _RowSets:
             self.tables.append((name, ids, n_rows, rows))
         self.count = torch.empty(len(self.tables), dtype=torch.int64, device=dev)
         self.build()
+        if model.cfg.sparse_grad == 2:
+            for j, (name, _, _, rows) in enumerate(self.tables):
+                optim.catch_up(model.get_parameter(name), rows, self.count[j:j + 1])
         self.host = torch.empty(len(self.tables), dtype=torch.int64, pin_memory=dev.type == "cuda")
         self.host.copy_(self.count, non_blocking=True)
         self.event = torch.cuda.Event() if dev.type == "cuda" else None
@@ -294,7 +298,10 @@ class IntEL(nn.Module):
         parser.add_argument('--buffer', type=int, default=1, help='Whether to buffer feed dicts for dev/test')
         parser.add_argument('--model_num', type=int, default=2, help='Number of base models.')
         parser.add_argument('--sparse_grad', type=int, default=0,
-                            help='Row-sparse gradients for the embedding tables (needs optim.Adam: BaseRunner_b200).')
+                            help='Row-sparse (COO) gradients for the embedding tables; they need optim.Adam (BaseRunner_b200), '
+                                 'since torch.optim.Adam rejects sparse gradients.  1: lazy Adam, the rows a step does not '
+                                 'name keep their values (differs from dense Adam with L2).  2: exact, optim.Adam defers the '
+                                 'updates of those rows and replays them when the rows are next read: bitwise dense Adam.')
         return parser
 
     def __init__(self, args, corpus=None, cfg: Optional[IntelConfig] = None):
@@ -358,6 +365,20 @@ class IntEL(nn.Module):
         shapes = c.param_shapes()
         for n, p in self.named_parameters():
             assert tuple(p.shape) == shapes[n], (n, tuple(p.shape), shapes[n])
+        if c.sparse_grad not in (0, 1, 2):
+            raise ValueError(f"sparse_grad must be 0, 1 or 2, not {c.sparse_grad}")
+        if c.sparse_grad == 2:
+            # optim.Adam defers the zero-gradient updates of these tables: whatever reads them whole sees them current
+            optim.defer_zero_updates(self._deferred_tables())
+            self.register_state_dict_pre_hook(lambda module, *_: module.flush_tables())
+            self.register_load_state_dict_pre_hook(lambda module, *_: module.flush_tables())
+
+    def _deferred_tables(self) -> list:
+        return [self.get_parameter(n) for n, _, _ in SPARSE_TABLES if n in self._param_names] if self.cfg.sparse_grad == 2 else []
+
+    def flush_tables(self) -> None:
+        """sparse_grad = 2: apply the updates optim.Adam deferred on the embedding tables (a no-op when none are pending)."""
+        optim.flush(self._deferred_tables())
 
     def _queue_input_check(self, lib, dims, bt, dev, stream) -> None:
         self.check_inputs(wait=False)
@@ -389,6 +410,8 @@ class IntEL(nn.Module):
     # ---- the hot path ----
     def forward(self, data: Dict[str, object]) -> Dict[str, torch.Tensor]:
         params = [p for _, p in self.named_parameters()]
+        if self.cfg.sparse_grad == 2 and not (torch.is_grad_enabled() and any(p.requires_grad for p in params)):
+            self.flush_tables()      # no row set is built (a training forward pass catches up its rows in _RowSets)
         weights, ens, intents = _IntelFn.apply(self, data, torch.is_grad_enabled(), *params)
         return {"weights": weights, "ens_score": ens, "intents": intents}
 

@@ -130,6 +130,8 @@ def _declare(lib: C.CDLL) -> None:
         "intel_lambdarank_lambdas": (i32, [i64, i64, _p, _p, _p, _p, _p]),
         "intel_adam_step": (i32, [i32, _p, _p, _p, _p, _p, _p, dbl, dbl, dbl, dbl, i64, _p]),
         "intel_adam_rows_step": (i32, [i32, _p, _p, _p, _p, _p, _p, _p, _p, dbl, dbl, dbl, dbl, i64, _p]),
+        "intel_adam_deferred_rows_step": (i32, [i32, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, dbl, dbl, dbl, dbl, i64, _p]),
+        "intel_adam_deferred_catch_up": (i32, [i32, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
         "intel_profile_enable": (i32, [i32]),
         "intel_profile_report": (i32, [C.c_char_p, sz]),
     }
@@ -151,7 +153,7 @@ EXPORTED = ["intel_ensemble_bwd_phase", "intel_reserve_sms", "intel_last_error",
             "intel_linear_fwd_ex", "intel_linear_dx_ex", "intel_linear_dw_ex", "intel_softmax_rows_fwd", "intel_softmax_rows_bwd",
             "intel_batch_validate", "intel_debug_use_tcgen05_stack", "intel_batch_build", "intel_debug_use_tcgen05_gru", "intel_debug_use_rows_gemm", "intel_debug_gru_prep", "intel_debug_use_fused_bert",
             "intel_rowset_workspace_bytes", "intel_rowset_build", "intel_ensemble_bwd_phase_rows", "intel_intent_bwd_rows",
-            "intel_adam_rows_step"]
+            "intel_adam_rows_step", "intel_adam_deferred_rows_step", "intel_adam_deferred_catch_up"]
 
 
 def load(path: Optional[str] = None) -> C.CDLL:

@@ -6,18 +6,29 @@ layout (``step``, ``exp_avg``, ``exp_avg_sq``), so ``state_dict()`` interchanges
 ``torch.optim.lr_scheduler.StepLR`` works on it.  ``step()`` updates all parameters with one kernel launch per 48
 tensors (``intel_adam_step``) instead of ~10 small kernels per tensor.
 
-A group may mix dense and row-sparse (COO, one sparse dimension) gradients: ``IntEL(sparse_grad=1)`` gives its embedding
-tables those.  A sparse gradient updates only the rows it lists (``intel_adam_rows_step``), each with the same per-element
-arithmetic as the dense kernel, the group's L2 and its shared step count; the other rows keep parameter and moments bit
-for bit.  That is not torch.optim.Adam on a dense gradient with zero rows (L2 and the moments' decay move every row there):
-it is the lazy form of Adam, opted into with the model flag.
+A group may mix dense and row-sparse (COO, one sparse dimension) gradients: ``IntEL(sparse_grad=1)`` and
+``IntEL(sparse_grad=2)`` give their embedding tables those.  A sparse gradient updates only the rows it lists
+(``intel_adam_rows_step``), each with the same per-element arithmetic as the dense kernel, the group's L2 and its shared
+step count; the other rows keep parameter and moments bit for bit.  That is not torch.optim.Adam on a dense gradient with
+zero rows (L2 and the moments' decay move every row there): it is the lazy form of Adam, opted into with
+``sparse_grad=1``.
+
+Parameters marked with ``defer_zero_updates`` (``IntEL(sparse_grad=2)`` marks its tables) stay on the dense trajectory
+instead.  The update a dense step gives an unlisted row has a gradient of exactly +0.0, so it depends only on the row and
+that step's scalars: the optimizer records each step's scalars per parameter and defers those updates, and
+``intel_adam_deferred_rows_step`` replays a row's pending ones, in order and with the same arithmetic, before its next
+update.  Rows are brought up to date without a new update by ``catch_up`` (the rows a forward pass is about to read) and
+``flush`` (every row).  After ``flush()`` parameters and moments equal dense Adam's bit for bit; ``state_dict()`` and
+``load_state_dict()`` flush first, so the saved state is torch's and interchanges with every mode.  A marked parameter that
+receives a dense gradient is flushed and then takes the dense step.
 """
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Hashable, Iterable
+from typing import Dict, Hashable, Iterable, Optional
 
 import torch
+from torch.utils.weak import WeakIdKeyDictionary
 
 from . import _lib
 
@@ -29,6 +40,69 @@ _coalesced_rows: Dict[Hashable, torch.Tensor] = {}
 
 def note_coalesced_rows(key: Hashable, rows: torch.Tensor) -> None:
     _coalesced_rows[key] = rows
+
+
+class _Deferred:
+    """Bookkeeping of a marked parameter (intel_adam_deferred_rows_step): ``n`` updates recorded since the last reset, their
+    scalars in ``hist`` [cap, 8] (grown by doubling), ``done[r]`` = how many of them row r has received; ``state`` is the
+    optimizer state (exp_avg, exp_avg_sq) the pending updates belong to."""
+
+    def __init__(self, p: torch.Tensor, state: dict) -> None:
+        self.state, self.n = state, 0
+        self.hist = torch.zeros(16, 8, dtype=torch.float32, device=p.device)
+        self.done = torch.zeros(p.shape[0], dtype=torch.int32, device=p.device)
+
+    def record(self) -> None:
+        """one more update; makes room for its entry in hist"""
+        self.n += 1
+        if self.n > self.hist.shape[0]:
+            hist = torch.zeros(2 * self.hist.shape[0], 8, dtype=torch.float32, device=self.hist.device)
+            hist[: self.n - 1] = self.hist[: self.n - 1]
+            self.hist = hist
+
+
+# parameters whose zero-gradient updates optim.Adam defers (IntEL(sparse_grad=2) marks its tables) -> their bookkeeping,
+# None until the first deferred step
+_deferred = WeakIdKeyDictionary()
+
+
+def defer_zero_updates(params: Iterable[torch.Tensor]) -> None:
+    """Mark parameters whose row-sparse gradients take the exact (deferred) row-wise step."""
+    for p in params:
+        _deferred.setdefault(p, None)
+
+
+def _catch_up(ps, rows, counts) -> None:
+    """intel_adam_deferred_catch_up over the pending parameters of ps (rows None: every row, then the count restarts)"""
+    recs = [(p, _deferred.get(p), r, c) for p, r, c in zip(ps, rows, counts)]
+    recs = [(p, d, r, c) for p, d, r, c in recs if d is not None and d.n > 0]
+    if not recs:
+        return
+    n = len(recs)
+    arr = lambda vals, t=C.c_void_p: (t * n)(*vals)
+    _lib.check(_lib.load().intel_adam_deferred_catch_up(
+        n, arr([_lib.ptr(p) for p, *_ in recs]), arr([_lib.ptr(d.state["exp_avg"]) for _, d, _, _ in recs]),
+        arr([_lib.ptr(d.state["exp_avg_sq"]) for _, d, _, _ in recs]), arr([_lib.ptr(r) for _, _, r, _ in recs]),
+        arr([_lib.ptr(c) for *_, c in recs]),
+        arr([(r.numel() if r is not None else p.shape[0]) for p, _, r, _ in recs], C.c_int64),
+        arr([p[0].numel() for p, *_ in recs], C.c_int32), arr([_lib.ptr(d.done) for _, d, _, _ in recs]),
+        arr([_lib.ptr(d.hist) for _, d, _, _ in recs]), arr([d.n for _, d, _, _ in recs], C.c_int32),
+        _lib.stream_ptr(recs[0][0].device)))
+    for _, d, r, _ in recs:
+        if r is None:
+            d.n = 0
+
+
+def catch_up(p: torch.Tensor, rows: torch.Tensor, count: torch.Tensor) -> None:
+    """Bring the first ``count`` (a device int64 [1]) rows of ``rows`` of a marked parameter up to date, without a host
+    synchronisation."""
+    _catch_up([p], [rows], [count])
+
+
+def flush(params: Iterable[torch.Tensor]) -> None:
+    """Apply every pending update of the given (marked) parameters: they and their moments then equal dense Adam's."""
+    ps = list(params)
+    _catch_up(ps, [None] * len(ps), [None] * len(ps))
 
 
 def _rows_and_values(p: torch.Tensor, g: torch.Tensor):
@@ -86,9 +160,14 @@ class Adam(torch.optim.Optimizer):
             b1, b2 = group["betas"]
             wd = float(group["weight_decay"])
             sparse = [p for p in ps if p.grad.is_sparse]
-            if sparse:
-                self._rows_step(sparse, group, wd, int(step_t))
+            deferred = [p for p in sparse if p in _deferred]
+            if deferred:
+                self._deferred_step(deferred, group, wd, int(step_t))
+            lazy = [p for p in sparse if p not in _deferred]
+            if lazy:
+                self._rows_step(lazy, group, wd, int(step_t))
             ps = [p for p in ps if not p.grad.is_sparse]
+            flush(p for p in ps if p in _deferred)         # a marked parameter with a dense gradient: current, then dense
             if not ps:
                 continue
             n = len(ps)
@@ -122,6 +201,40 @@ class Adam(torch.optim.Optimizer):
             arr([r.numel() for r in rows], C.c_int64), arr([p[0].numel() for p in ps], C.c_int32), arr([wd] * n, C.c_float),
             float(group["lr"]), float(b1), float(b2), float(group["eps"]), step, _lib.stream_ptr(ps[0].device)))
 
+    def _deferred_step(self, ps, group, wd: float, step: int) -> None:
+        n = len(ps)
+        arr = lambda vals, t=C.c_void_p: (t * n)(*vals)
+        rows, vals = zip(*[_rows_and_values(p, p.grad) for p in ps])
+        st = [self.state[p] for p in ps]
+        recs = []
+        for p, s in zip(ps, st):
+            d = _deferred.get(p)
+            if d is not None and d.state is not s:           # pending updates of another optimizer's state: apply them first
+                flush([p])
+                d = None
+            if d is None:
+                d = _deferred[p] = _Deferred(p, s)
+            d.record()
+            recs.append(d)
+        b1, b2 = group["betas"]
+        _lib.check(_lib.load().intel_adam_deferred_rows_step(
+            n, arr([_lib.ptr(p) for p in ps]), arr([_lib.ptr(s["exp_avg"]) for s in st]),
+            arr([_lib.ptr(s["exp_avg_sq"]) for s in st]), arr([_lib.ptr(r) for r in rows]), arr([_lib.ptr(v) for v in vals]),
+            arr([r.numel() for r in rows], C.c_int64), arr([p[0].numel() for p in ps], C.c_int32), arr([wd] * n, C.c_float),
+            arr([_lib.ptr(d.done) for d in recs]), arr([_lib.ptr(d.hist) for d in recs]), arr([d.n for d in recs], C.c_int32),
+            float(group["lr"]), float(b1), float(b2), float(group["eps"]), step, _lib.stream_ptr(ps[0].device)))
+
+    def flush(self, params: Optional[Iterable[torch.Tensor]] = None) -> None:
+        """Apply the deferred updates of ``params`` (default: every parameter of this optimizer).  Afterwards parameters
+        and moments equal what dense Adam would hold, bit for bit.  Call it before reading a marked table directly."""
+        if params is None:
+            params = [p for g in self.param_groups for p in g["params"]]
+        flush(p for p in params if p in _deferred)
+
+    def state_dict(self):
+        self.flush()
+        return super().state_dict()
+
     def _build_cache(self, ps, key):
         """pointer tables of a group's dense-gradient tensors (parameters and moments keep their storage; gradients are
         refreshed every step); the state of every tensor of the group"""
@@ -148,5 +261,10 @@ class Adam(torch.optim.Optimizer):
                 "numel": (C.c_int64 * n)(*[p.numel() for p in ps]), "grads": (C.c_void_p * n)(), "wd": None, "wd_value": None}
 
     def load_state_dict(self, state_dict):
+        self.flush()                 # the pending updates belong to the weights as they are and to the state being replaced
         super().load_state_dict(state_dict)
         self._cache = {}
+        for g in self.param_groups:
+            for p in g["params"]:
+                if _deferred.get(p) is not None:
+                    _deferred[p] = None
