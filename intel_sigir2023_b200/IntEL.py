@@ -417,10 +417,7 @@ class IntEL(nn.Module):
 
     # ---- auxiliary methods kept from BaseModel (BaseModel.py:53-78) ----
     def customize_parameters(self, define_dict={}) -> list:
-        weight_p, bias_p = [], []
-        for name, p in filter(lambda x: x[1].requires_grad, self.named_parameters()):
-            (bias_p if 'bias' in name else weight_p).append(p)
-        return [{'params': weight_p}, {'params': bias_p, 'weight_decay': 0}]
+        return optim.customize_parameters(self)
 
     def save_model(self, model_path=None):
         model_path = model_path or self.model_path

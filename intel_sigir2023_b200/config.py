@@ -36,7 +36,8 @@ class IntelConfig:
     gru_hidden: int = 128     # GRU4RecEncoder(hidden_size=128)  (IntEL.py:105-106)
     bert_layers: int = 2      # BERT4RecEncoder(num_layers=2, num_heads=2) (IntEL.py:108-109)
     bert_heads: int = 2
-    # --sparse_grad 1: the four embedding tables get row-sparse (COO) gradients over the rows a step names
+    # --sparse_grad: 0 dense table gradients; 1 and 2 give the four embedding tables row-sparse (COO) gradients over the
+    # rows a step names, with lazy Adam (1: unnamed rows keep their values) or exact Adam (2: bitwise dense Adam)
     sparse_grad: int = 0
 
     # ---- derived widths ----

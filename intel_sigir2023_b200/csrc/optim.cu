@@ -13,6 +13,21 @@ namespace intel {
 
 static const int ADAM_MAX_TENSORS = 48;
 
+// The float32 scalars of one Adam step.  Every step forms them with adam_scalars only: the deferred row-wise step is
+// bitwise the dense one because its replayed updates use exactly the floats the dense step would have used.
+struct AdamScalars {
+    float lr_over_bc1;      // lr / (1 - beta1^step)
+    float bc2_sqrt;         // sqrt(1 - beta2^step)
+    float beta2, eps;
+    float w1, w2;           // 1 - beta1, 1 - beta2
+};
+
+// computed in double and rounded once, like torch's python-side scalars
+static AdamScalars adam_scalars(double lr, double beta1, double beta2, double eps, int64_t step) {
+    const double bc1 = 1.0 - pow(beta1, (double)step), bc2 = 1.0 - pow(beta2, (double)step);
+    return AdamScalars{(float)(lr / bc1), (float)sqrt(bc2), (float)beta2, (float)eps, (float)(1.0 - beta1), (float)(1.0 - beta2)};
+}
+
 struct AdamTensor {
     float* p;
     const float* g;
@@ -24,10 +39,7 @@ struct AdamTensor {
 struct AdamArgs {
     AdamTensor t[ADAM_MAX_TENSORS];
     int count;
-    float lr_over_bc1;      // lr / (1 - beta1^step)
-    float bc2_sqrt;         // sqrt(1 - beta2^step)
-    float beta2, eps;
-    float w1, w2;           // 1 - beta1, 1 - beta2, rounded from double like torch's python-side scalars
+    AdamScalars s;
 };
 
 __device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, float wd, float w1, float w2, float beta2,
@@ -41,143 +53,63 @@ __device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, 
 
 __global__ void __launch_bounds__(256) adam_kernel(AdamArgs a) {
     const AdamTensor t = a.t[blockIdx.y];
-    const float w1 = a.w1, w2 = a.w2, ns = -a.lr_over_bc1;
+    const AdamScalars& s = a.s;
+    const float w1 = s.w1, w2 = s.w2, ns = -s.lr_over_bc1;
     const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, nth = (int64_t)gridDim.x * blockDim.x;
     const bool vec = ((((uintptr_t)t.p) | ((uintptr_t)t.g) | ((uintptr_t)t.m) | ((uintptr_t)t.v)) & 15) == 0;
     const int64_t n4 = vec ? t.n / 4 : 0;
     for (int64_t i = tid; i < n4; i += nth) {           // 16-byte accesses: 7 streams of 4 floats per thread in flight
         float4 p = reinterpret_cast<float4*>(t.p)[i], m = reinterpret_cast<float4*>(t.m)[i], v = reinterpret_cast<float4*>(t.v)[i];
         const float4 g = reinterpret_cast<const float4*>(t.g)[i];
-        adam_one(p.x, g.x, m.x, v.x, t.wd, w1, w2, a.beta2, a.bc2_sqrt, a.eps, ns);
-        adam_one(p.y, g.y, m.y, v.y, t.wd, w1, w2, a.beta2, a.bc2_sqrt, a.eps, ns);
-        adam_one(p.z, g.z, m.z, v.z, t.wd, w1, w2, a.beta2, a.bc2_sqrt, a.eps, ns);
-        adam_one(p.w, g.w, m.w, v.w, t.wd, w1, w2, a.beta2, a.bc2_sqrt, a.eps, ns);
+        adam_one(p.x, g.x, m.x, v.x, t.wd, w1, w2, s.beta2, s.bc2_sqrt, s.eps, ns);
+        adam_one(p.y, g.y, m.y, v.y, t.wd, w1, w2, s.beta2, s.bc2_sqrt, s.eps, ns);
+        adam_one(p.z, g.z, m.z, v.z, t.wd, w1, w2, s.beta2, s.bc2_sqrt, s.eps, ns);
+        adam_one(p.w, g.w, m.w, v.w, t.wd, w1, w2, s.beta2, s.bc2_sqrt, s.eps, ns);
         reinterpret_cast<float4*>(t.p)[i] = p;
         reinterpret_cast<float4*>(t.m)[i] = m;
         reinterpret_cast<float4*>(t.v)[i] = v;
     }
     for (int64_t i = 4 * n4 + tid; i < t.n; i += nth) {
         float p = t.p[i], m = t.m[i], v = t.v[i];
-        adam_one(p, t.g[i], m, v, t.wd, w1, w2, a.beta2, a.bc2_sqrt, a.eps, ns);
+        adam_one(p, t.g[i], m, v, t.wd, w1, w2, s.beta2, s.bc2_sqrt, s.eps, ns);
         t.p[i] = p;
         t.m[i] = m;
         t.v[i] = v;
     }
 }
 
-// Row-wise step of a sparse (row set) gradient: rows[r] of p / m / v get adam_one with the compact gradient row r; every
-// other row keeps p, m and v bit for bit.  The arithmetic per element is the dense kernel's, so a row updated here equals
-// the same row updated by adam_kernel with that gradient.
-struct AdamRowsTensor {
-    float* p;
-    const float* g;        // [U, d]
-    float* m;
-    float* v;
-    const int64_t* rows;   // [U], distinct
-    int64_t U;
-    int d;
-    float wd;
-};
-struct AdamRowsArgs {
-    AdamRowsTensor t[ADAM_MAX_TENSORS];
-    int count;
-    float lr_over_bc1, bc2_sqrt, beta2, eps, w1, w2;
-};
-
-__global__ void __launch_bounds__(256) adam_rows_kernel(AdamRowsArgs a) {
-    const AdamRowsTensor t = a.t[blockIdx.y];
-    const float w1 = a.w1, w2 = a.w2, ns = -a.lr_over_bc1;
-    const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, nth = (int64_t)gridDim.x * blockDim.x;
-    const bool vec = t.d % 4 == 0 && ((((uintptr_t)t.p) | ((uintptr_t)t.g) | ((uintptr_t)t.m) | ((uintptr_t)t.v)) & 15) == 0;
-    if (vec) {
-        const int per_row = t.d / 4;
-        for (int64_t e = tid; e < t.U * per_row; e += nth) {
-            const int64_t r = e / per_row, row = t.rows[r];
-            const int c = (int)(e % per_row);
-            float4* pp = reinterpret_cast<float4*>(t.p + row * t.d) + c;
-            float4* mp = reinterpret_cast<float4*>(t.m + row * t.d) + c;
-            float4* vp = reinterpret_cast<float4*>(t.v + row * t.d) + c;
-            float4 p = *pp, m = *mp, v = *vp;
-            const float4 g = reinterpret_cast<const float4*>(t.g + r * t.d)[c];
-            adam_one(p.x, g.x, m.x, v.x, t.wd, w1, w2, a.beta2, a.bc2_sqrt, a.eps, ns);
-            adam_one(p.y, g.y, m.y, v.y, t.wd, w1, w2, a.beta2, a.bc2_sqrt, a.eps, ns);
-            adam_one(p.z, g.z, m.z, v.z, t.wd, w1, w2, a.beta2, a.bc2_sqrt, a.eps, ns);
-            adam_one(p.w, g.w, m.w, v.w, t.wd, w1, w2, a.beta2, a.bc2_sqrt, a.eps, ns);
-            *pp = p;
-            *mp = m;
-            *vp = v;
-        }
-    } else {
-        for (int64_t e = tid; e < t.U * t.d; e += nth) {
-            const int64_t r = e / t.d, i = t.rows[r] * t.d + e % t.d;
-            float p = t.p[i], m = t.m[i], v = t.v[i];
-            adam_one(p, t.g[e], m, v, t.wd, w1, w2, a.beta2, a.bc2_sqrt, a.eps, ns);
-            t.p[i] = p;
-            t.m[i] = m;
-            t.v[i] = v;
-        }
-    }
-}
-
-int adam_rows_step(int count, float* const* params, float* const* exp_avg, float* const* exp_avg_sq, const int64_t* const* rows,
-                   const float* const* grads, const int64_t* nrows, const int32_t* dim, const float* weight_decay, double lr,
-                   double beta1_d, double beta2_d, double eps_d, int64_t step, cudaStream_t s) {
-    INTEL_REQUIRE(count >= 0 && step >= 1, INTEL_ERR_ARG, "adam_rows_step: bad count / step");
-    const double bc1 = 1.0 - pow(beta1_d, (double)step), bc2 = 1.0 - pow(beta2_d, (double)step);
-    AdamRowsArgs a;
-    memset(&a, 0, sizeof(a));
-    a.lr_over_bc1 = (float)(lr / bc1);             // the scalars exactly as adam_step forms them
-    a.bc2_sqrt = (float)sqrt(bc2);
-    a.beta2 = (float)beta2_d; a.eps = (float)eps_d;
-    a.w1 = (float)(1.0 - (double)beta1_d);
-    a.w2 = (float)(1.0 - (double)beta2_d);
-    int64_t widest = 1;
-    auto flush = [&]() -> int {
-        if (a.count == 0) return INTEL_OK;
-        int64_t bx = ceil_div(widest, 256 * 4);
-        if (bx > 16 * kNumSMs) bx = 16 * kNumSMs;
-        LAUNCH(adam_rows_kernel, dim3((unsigned)bx, (unsigned)a.count), dim3(256), 0, s, a);
-        double bytes = 0;
-        for (int i = 0; i < a.count; ++i) bytes += (double)a.t[i].U * (28.0 * a.t[i].d + 8.0);
-        a.count = 0;
-        widest = 1;
-        return check_launch("adam_rows", bytes, 0.0);
-    };
-    for (int i = 0; i < count; ++i) {
-        INTEL_REQUIRE(nrows[i] >= 0 && dim[i] > 0 && (nrows[i] == 0 || (params[i] && exp_avg[i] && exp_avg_sq[i] && rows[i] && grads[i])),
-                      INTEL_ERR_ARG, "adam_rows_step: bad tensor %d", i);
-        if (nrows[i] == 0) continue;
-        a.t[a.count++] = AdamRowsTensor{params[i], grads[i], exp_avg[i], exp_avg_sq[i], rows[i], nrows[i], dim[i], weight_decay[i]};
-        if (nrows[i] * dim[i] > widest) widest = nrows[i] * dim[i];
-        if (a.count == ADAM_MAX_TENSORS) INTEL_TRY(flush());
-    }
-    return flush();
-}
-
-// Deferred (exact) row-wise step.  Dense Adam gives every row a step never names a gradient of exactly +0.0, and such an
-// update depends only on the row's own p / m / v and that step's scalars.  So the updates a row skips are deferred and
-// replayed later, in order, through the same adam_one: a row with k pending updates is read and written once, and the
-// result is bitwise the dense one.  Per tensor the caller keeps
+// Row-wise steps of a sparse (row set) gradient, one kernel in four modes.  The listed rows of p / m / v get adam_one per
+// element, the dense kernel's arithmetic; every other row keeps p, m and v bit for bit.
+// LAZY:     listed rows take the update with their compact gradient row (done / hist unused), so a row updated here
+//           equals the same row updated by adam_kernel with that gradient.
+// The other three modes are the deferred (exact) step.  Dense Adam gives every row a step never names a gradient of
+// exactly +0.0, and such an update depends only on the row's own p / m / v and that step's scalars.  So the updates a row
+// skips are deferred and replayed later, in order, through the same adam_one: a row with k pending updates is read and
+// written once, and the result is bitwise the dense one.  Per tensor the caller keeps
 //   hist [>= n, 8] float: entry k holds the scalars of update k + 1 (ADAM_HIST_* below),
 //   done [rows] int32:    how many of the n updates row r has received (the row is current when done[r] == n).
 // STEP:     listed rows replay done[r] .. n-2 with g = +0.0, then take update n with their gradient row; the kernel also
 //           stores update n's scalars (its arguments) to hist[n-1].
 // CATCH_UP: listed rows (the count read from device memory) replay done[r] .. n-1.
 // FLUSH:    every row replays done[r] .. n-1, and done is reset to 0 for the caller to restart its count.
-// A row is handled by one group of G lanes of a warp (G = the power of two >= the row's vectors, at most 32): its lanes
-// read done[r] before the group's first lane writes it, with a __syncwarp in between, so the loop is warp-uniform.
+// A row is handled by one group of G lanes of a warp (G = the power of two >= the row's vectors, at most 32).  In the
+// deferred modes its lanes read done[r] before the group's first lane writes it, with a __syncwarp in between, so the
+// loop is warp-uniform.
 enum { ADAM_HIST_LR_BC1, ADAM_HIST_BC2_SQRT, ADAM_HIST_BETA2, ADAM_HIST_EPS, ADAM_HIST_W1, ADAM_HIST_W2, ADAM_HIST_WD, ADAM_HIST_WIDTH = 8 };
-enum AdamDeferredMode { ADAM_DEFERRED_STEP, ADAM_DEFERRED_CATCH_UP, ADAM_DEFERRED_FLUSH };
+enum AdamRowsMode { ADAM_ROWS_LAZY, ADAM_DEFERRED_STEP, ADAM_DEFERRED_CATCH_UP, ADAM_DEFERRED_FLUSH };
+
+// the modes that apply a new update with a gradient row
+__host__ __device__ constexpr bool adam_rows_take_grad(int mode) { return mode == ADAM_ROWS_LAZY || mode == ADAM_DEFERRED_STEP; }
 
 struct AdamDeferredTensor {
     float* p;
-    const float* g;          // [U, d] (STEP only)
+    const float* g;          // [U, d] (LAZY, STEP)
     float* m;
     float* v;
     const int64_t* rows;     // [U] distinct; NULL: rows 0 .. U-1 (FLUSH)
     const int64_t* count;    // CATCH_UP: device count of rows (<= U)
-    int32_t* done;
-    float* hist;
+    int32_t* done;           // NULL in LAZY
+    float* hist;             // NULL in LAZY
     int64_t U;
     int d;
     int n;
@@ -186,13 +118,13 @@ struct AdamDeferredTensor {
 struct AdamDeferredArgs {
     AdamDeferredTensor t[ADAM_MAX_TENSORS];
     int count;
-    float lr_over_bc1, bc2_sqrt, beta2, eps, w1, w2;     // STEP: the scalars of update n
+    AdamScalars s;           // LAZY, STEP: the scalars of the new update
 };
 
-// V consecutive elements of one row: replay hist[k0 .. k1) with g = +0.0, then (grad != NULL) one update with grad
-template <int V>
-__device__ __forceinline__ void adam_deferred_elems(float* p_, float* m_, float* v_, const float* g_, const float* hist, int k0,
-                                                    int k1, float wd, const AdamDeferredArgs& a) {
+// V consecutive elements of one row: replay hist[k0 .. k1) with g = +0.0 (REPLAY), then one update with the gradient g_ (GRAD)
+template <bool REPLAY, bool GRAD, int V>
+__device__ __forceinline__ void adam_rows_elems(float* p_, float* m_, float* v_, const float* g_, const float* hist, int k0, int k1,
+                                                float wd, const AdamScalars& s) {
     float p[V], m[V], v[V];
     if constexpr (V == 4) {
         const float4 P = *reinterpret_cast<const float4*>(p_), M = *reinterpret_cast<const float4*>(m_),
@@ -203,12 +135,14 @@ __device__ __forceinline__ void adam_deferred_elems(float* p_, float* m_, float*
     } else {
         p[0] = *p_; m[0] = *m_; v[0] = *v_;
     }
-    for (int k = k0; k < k1; ++k) {
-        const float4 h0 = reinterpret_cast<const float4*>(hist)[2 * k], h1 = reinterpret_cast<const float4*>(hist)[2 * k + 1];
+    if constexpr (REPLAY) {
+        for (int k = k0; k < k1; ++k) {
+            const float4 h0 = reinterpret_cast<const float4*>(hist)[2 * k], h1 = reinterpret_cast<const float4*>(hist)[2 * k + 1];
 #pragma unroll
-        for (int j = 0; j < V; ++j) adam_one(p[j], 0.0f, m[j], v[j], h1.z, h1.x, h1.y, h0.z, h0.y, h0.w, -h0.x);
+            for (int j = 0; j < V; ++j) adam_one(p[j], 0.0f, m[j], v[j], h1.z, h1.x, h1.y, h0.z, h0.y, h0.w, -h0.x);
+        }
     }
-    if (g_ != nullptr) {
+    if constexpr (GRAD) {
         float g[V];
         if constexpr (V == 4) {
             const float4 G = *reinterpret_cast<const float4*>(g_);
@@ -217,7 +151,7 @@ __device__ __forceinline__ void adam_deferred_elems(float* p_, float* m_, float*
             g[0] = *g_;
         }
 #pragma unroll
-        for (int j = 0; j < V; ++j) adam_one(p[j], g[j], m[j], v[j], wd, a.w1, a.w2, a.beta2, a.bc2_sqrt, a.eps, -a.lr_over_bc1);
+        for (int j = 0; j < V; ++j) adam_one(p[j], g[j], m[j], v[j], wd, s.w1, s.w2, s.beta2, s.bc2_sqrt, s.eps, -s.lr_over_bc1);
     }
     if constexpr (V == 4) {
         *reinterpret_cast<float4*>(p_) = make_float4(p[0], p[1], p[2], p[3]);
@@ -229,7 +163,8 @@ __device__ __forceinline__ void adam_deferred_elems(float* p_, float* m_, float*
 }
 
 template <int MODE, int V>
-__device__ __forceinline__ void adam_deferred_rows(const AdamDeferredTensor& t, const AdamDeferredArgs& a, int64_t U) {
+__device__ __forceinline__ void adam_rows_groups(const AdamDeferredTensor& t, const AdamScalars& s, int64_t U) {
+    constexpr bool LAZY = MODE == ADAM_ROWS_LAZY, GRAD = adam_rows_take_grad(MODE);
     const int per_row = t.d / V;
     int G = 1;
     while (G < per_row && G < 32) G <<= 1;
@@ -243,55 +178,59 @@ __device__ __forceinline__ void adam_deferred_rows(const AdamDeferredTensor& t, 
         int k0 = last;
         if (live) {
             row = t.rows != nullptr ? t.rows[r] : r;
-            k0 = t.done[row];
+            if constexpr (!LAZY) k0 = t.done[row];
         }
-        if (live && (MODE == ADAM_DEFERRED_STEP || k0 < last)) {
+        if (live && (GRAD || k0 < last)) {
             for (int c = lg; c < per_row; c += G) {
                 const int64_t e = row * t.d + (int64_t)c * V;
-                adam_deferred_elems<V>(t.p + e, t.m + e, t.v + e,
-                                       MODE == ADAM_DEFERRED_STEP ? t.g + r * t.d + (int64_t)c * V : nullptr, t.hist, k0, last,
-                                       t.wd, a);
+                adam_rows_elems<!LAZY, GRAD, V>(t.p + e, t.m + e, t.v + e, GRAD ? t.g + r * t.d + (int64_t)c * V : nullptr, t.hist, k0,
+                                                last, t.wd, s);
             }
         }
-        __syncwarp();
-        if (live && lg == 0) {
-            if (MODE == ADAM_DEFERRED_FLUSH) t.done[row] = 0;
-            else if (MODE == ADAM_DEFERRED_STEP || k0 < last) t.done[row] = t.n;
+        if constexpr (!LAZY) {
+            __syncwarp();
+            if (live && lg == 0) {
+                if (MODE == ADAM_DEFERRED_FLUSH) t.done[row] = 0;
+                else if (MODE == ADAM_DEFERRED_STEP || k0 < last) t.done[row] = t.n;
+            }
         }
     }
 }
 
 template <int MODE>
-__global__ void __launch_bounds__(256) adam_deferred_kernel(AdamDeferredArgs a) {
+__global__ void __launch_bounds__(256) adam_rows_kernel(AdamDeferredArgs a) {
     const AdamDeferredTensor t = a.t[blockIdx.y];
     int64_t U = t.U;
     if (MODE == ADAM_DEFERRED_CATCH_UP) U = min(U, *t.count);
     if (MODE == ADAM_DEFERRED_STEP && blockIdx.x == 0 && threadIdx.x == 0) {
         float* h = t.hist + (int64_t)(t.n - 1) * ADAM_HIST_WIDTH;     // no lane of this launch reads entry n-1
-        h[ADAM_HIST_LR_BC1] = a.lr_over_bc1; h[ADAM_HIST_BC2_SQRT] = a.bc2_sqrt; h[ADAM_HIST_BETA2] = a.beta2;
-        h[ADAM_HIST_EPS] = a.eps; h[ADAM_HIST_W1] = a.w1; h[ADAM_HIST_W2] = a.w2; h[ADAM_HIST_WD] = t.wd; h[7] = 0.f;
+        h[ADAM_HIST_LR_BC1] = a.s.lr_over_bc1; h[ADAM_HIST_BC2_SQRT] = a.s.bc2_sqrt; h[ADAM_HIST_BETA2] = a.s.beta2;
+        h[ADAM_HIST_EPS] = a.s.eps; h[ADAM_HIST_W1] = a.s.w1; h[ADAM_HIST_W2] = a.s.w2; h[ADAM_HIST_WD] = t.wd; h[7] = 0.f;
     }
     const bool vec = t.d % 4 == 0 && ((((uintptr_t)t.p) | ((uintptr_t)t.m) | ((uintptr_t)t.v) |
-                                       (MODE == ADAM_DEFERRED_STEP ? (uintptr_t)t.g : 0)) & 15) == 0;
-    if (vec) adam_deferred_rows<MODE, 4>(t, a, U);
-    else adam_deferred_rows<MODE, 1>(t, a, U);
+                                       (adam_rows_take_grad(MODE) ? (uintptr_t)t.g : 0)) & 15) == 0;
+    if (vec) adam_rows_groups<MODE, 4>(t, a.s, U);
+    else adam_rows_groups<MODE, 1>(t, a.s, U);
 }
 
 // one launch per ADAM_MAX_TENSORS tensors, grid sized for the widest (rows x d).  STEP keeps tensors without rows: their
 // launch still records the update's scalars.
 template <int MODE>
-static int adam_deferred_launch(AdamDeferredArgs& a, const std::vector<AdamDeferredTensor>& ts, cudaStream_t s, const char* name) {
+static int adam_rows_launch(const AdamScalars& sc, const std::vector<AdamDeferredTensor>& ts, cudaStream_t s, const char* name) {
+    const double elem_bytes = adam_rows_take_grad(MODE) ? 28.0 : 24.0, row_bytes = MODE == ADAM_ROWS_LAZY ? 8.0 : 16.0;
+    AdamDeferredArgs a;
+    memset(&a, 0, sizeof(a));
+    a.s = sc;
     int64_t widest = 1;
     double bytes = 0;
-    a.count = 0;
     for (size_t i = 0; i < ts.size(); ++i) {
         a.t[a.count++] = ts[i];
         if (ts[i].U * ts[i].d > widest) widest = ts[i].U * ts[i].d;
-        bytes += (double)ts[i].U * ((MODE == ADAM_DEFERRED_STEP ? 28.0 : 24.0) * ts[i].d + 16.0);
+        bytes += (double)ts[i].U * (elem_bytes * ts[i].d + row_bytes);
         if (a.count < ADAM_MAX_TENSORS && i + 1 < ts.size()) continue;
         int64_t bx = ceil_div(widest, 256 * 4);
         if (bx > 16 * kNumSMs) bx = 16 * kNumSMs;
-        LAUNCH(adam_deferred_kernel<MODE>, dim3((unsigned)bx, (unsigned)a.count), dim3(256), 0, s, a);
+        LAUNCH(adam_rows_kernel<MODE>, dim3((unsigned)bx, (unsigned)a.count), dim3(256), 0, s, a);
         INTEL_TRY(check_launch(name, bytes, 0.0));
         a.count = 0;
         widest = 1;
@@ -300,19 +239,26 @@ static int adam_deferred_launch(AdamDeferredArgs& a, const std::vector<AdamDefer
     return INTEL_OK;
 }
 
+int adam_rows_step(int count, float* const* params, float* const* exp_avg, float* const* exp_avg_sq, const int64_t* const* rows,
+                   const float* const* grads, const int64_t* nrows, const int32_t* dim, const float* weight_decay, double lr,
+                   double beta1_d, double beta2_d, double eps_d, int64_t step, cudaStream_t s) {
+    INTEL_REQUIRE(count >= 0 && step >= 1, INTEL_ERR_ARG, "adam_rows_step: bad count / step");
+    std::vector<AdamDeferredTensor> ts;
+    for (int i = 0; i < count; ++i) {
+        INTEL_REQUIRE(nrows[i] >= 0 && dim[i] > 0 && (nrows[i] == 0 || (params[i] && exp_avg[i] && exp_avg_sq[i] && rows[i] && grads[i])),
+                      INTEL_ERR_ARG, "adam_rows_step: bad tensor %d", i);
+        if (nrows[i] == 0) continue;
+        ts.push_back(AdamDeferredTensor{params[i], grads[i], exp_avg[i], exp_avg_sq[i], rows[i], nullptr, nullptr, nullptr, nrows[i],
+                                        dim[i], 0, weight_decay[i]});
+    }
+    return adam_rows_launch<ADAM_ROWS_LAZY>(adam_scalars(lr, beta1_d, beta2_d, eps_d, step), ts, s, "adam_rows");
+}
+
 int adam_deferred_rows_step(int count, float* const* params, float* const* exp_avg, float* const* exp_avg_sq,
                             const int64_t* const* rows, const float* const* grads, const int64_t* nrows, const int32_t* dim,
                             const float* weight_decay, int32_t* const* done, float* const* hist, const int32_t* n_updates,
                             double lr, double beta1_d, double beta2_d, double eps_d, int64_t step, cudaStream_t s) {
     INTEL_REQUIRE(count >= 0 && step >= 1, INTEL_ERR_ARG, "adam_deferred_rows_step: bad count / step");
-    const double bc1 = 1.0 - pow(beta1_d, (double)step), bc2 = 1.0 - pow(beta2_d, (double)step);
-    AdamDeferredArgs a;
-    memset(&a, 0, sizeof(a));
-    a.lr_over_bc1 = (float)(lr / bc1);             // the scalars exactly as adam_step forms them
-    a.bc2_sqrt = (float)sqrt(bc2);
-    a.beta2 = (float)beta2_d; a.eps = (float)eps_d;
-    a.w1 = (float)(1.0 - (double)beta1_d);
-    a.w2 = (float)(1.0 - (double)beta2_d);
     std::vector<AdamDeferredTensor> ts;
     for (int i = 0; i < count; ++i) {
         INTEL_REQUIRE(nrows[i] >= 0 && dim[i] > 0 && n_updates[i] >= 1 && params[i] && exp_avg[i] && exp_avg_sq[i] && done[i] &&
@@ -321,15 +267,13 @@ int adam_deferred_rows_step(int count, float* const* params, float* const* exp_a
         ts.push_back(AdamDeferredTensor{params[i], grads[i], exp_avg[i], exp_avg_sq[i], rows[i], nullptr, done[i], hist[i], nrows[i],
                                         dim[i], n_updates[i], weight_decay[i]});
     }
-    return adam_deferred_launch<ADAM_DEFERRED_STEP>(a, ts, s, "adam_deferred_step");
+    return adam_rows_launch<ADAM_DEFERRED_STEP>(adam_scalars(lr, beta1_d, beta2_d, eps_d, step), ts, s, "adam_deferred_step");
 }
 
 int adam_deferred_catch_up(int count, float* const* params, float* const* exp_avg, float* const* exp_avg_sq,
                            const int64_t* const* rows, const int64_t* const* row_count, const int64_t* nrows, const int32_t* dim,
                            int32_t* const* done, const float* const* hist, const int32_t* n_updates, cudaStream_t s) {
     INTEL_REQUIRE(count >= 0, INTEL_ERR_ARG, "adam_deferred_catch_up: bad count");
-    AdamDeferredArgs a;
-    memset(&a, 0, sizeof(a));
     std::vector<AdamDeferredTensor> listed, all;
     for (int i = 0; i < count; ++i) {
         INTEL_REQUIRE(nrows[i] >= 0 && dim[i] > 0 && n_updates[i] >= 0, INTEL_ERR_ARG, "adam_deferred_catch_up: bad tensor %d", i);
@@ -340,23 +284,17 @@ int adam_deferred_catch_up(int count, float* const* params, float* const* exp_av
                                                               done[i], const_cast<float*>(hist[i]), nrows[i], dim[i], n_updates[i],
                                                               0.f});
     }
-    INTEL_TRY(adam_deferred_launch<ADAM_DEFERRED_CATCH_UP>(a, listed, s, "adam_deferred_catch_up"));
-    return adam_deferred_launch<ADAM_DEFERRED_FLUSH>(a, all, s, "adam_deferred_flush");
+    INTEL_TRY(adam_rows_launch<ADAM_DEFERRED_CATCH_UP>(AdamScalars{}, listed, s, "adam_deferred_catch_up"));
+    return adam_rows_launch<ADAM_DEFERRED_FLUSH>(AdamScalars{}, all, s, "adam_deferred_flush");
 }
 
 int adam_step(int count, float* const* params, const float* const* grads, float* const* exp_avg, float* const* exp_avg_sq,
               const int64_t* numel, const float* weight_decay, double lr, double beta1_d, double beta2_d, double eps_d, int64_t step,
               cudaStream_t s) {
-    const float beta2 = (float)beta2_d, eps = (float)eps_d;
     INTEL_REQUIRE(count >= 0 && step >= 1, INTEL_ERR_ARG, "adam_step: bad count / step");
-    const double bc1 = 1.0 - pow(beta1_d, (double)step), bc2 = 1.0 - pow(beta2_d, (double)step);
     AdamArgs a;
     memset(&a, 0, sizeof(a));
-    a.lr_over_bc1 = (float)(lr / bc1);
-    a.bc2_sqrt = (float)sqrt(bc2);
-    a.beta2 = beta2; a.eps = eps;
-    a.w1 = (float)(1.0 - (double)beta1_d);
-    a.w2 = (float)(1.0 - (double)beta2_d);
+    a.s = adam_scalars(lr, beta1_d, beta2_d, eps_d, step);
     // big tensors (embedding tables) get a launch of their own with a full grid; all small tensors share launches of
     // up to ADAM_MAX_TENSORS tensors with a short grid (a common grid sized for the largest tensor would schedule tens of
     // thousands of empty blocks)

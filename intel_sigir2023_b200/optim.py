@@ -72,21 +72,25 @@ def defer_zero_updates(params: Iterable[torch.Tensor]) -> None:
         _deferred.setdefault(p, None)
 
 
+def _arr(vals, t=C.c_void_p):
+    """ctypes array of t (default: pointers) over vals"""
+    vals = list(vals)
+    return (t * len(vals))(*vals)
+
+
 def _catch_up(ps, rows, counts) -> None:
     """intel_adam_deferred_catch_up over the pending parameters of ps (rows None: every row, then the count restarts)"""
     recs = [(p, _deferred.get(p), r, c) for p, r, c in zip(ps, rows, counts)]
     recs = [(p, d, r, c) for p, d, r, c in recs if d is not None and d.n > 0]
     if not recs:
         return
-    n = len(recs)
-    arr = lambda vals, t=C.c_void_p: (t * n)(*vals)
     _lib.check(_lib.load().intel_adam_deferred_catch_up(
-        n, arr([_lib.ptr(p) for p, *_ in recs]), arr([_lib.ptr(d.state["exp_avg"]) for _, d, _, _ in recs]),
-        arr([_lib.ptr(d.state["exp_avg_sq"]) for _, d, _, _ in recs]), arr([_lib.ptr(r) for _, _, r, _ in recs]),
-        arr([_lib.ptr(c) for *_, c in recs]),
-        arr([(r.numel() if r is not None else p.shape[0]) for p, _, r, _ in recs], C.c_int64),
-        arr([p[0].numel() for p, *_ in recs], C.c_int32), arr([_lib.ptr(d.done) for _, d, _, _ in recs]),
-        arr([_lib.ptr(d.hist) for _, d, _, _ in recs]), arr([d.n for _, d, _, _ in recs], C.c_int32),
+        len(recs), _arr(_lib.ptr(p) for p, *_ in recs), _arr(_lib.ptr(d.state["exp_avg"]) for _, d, _, _ in recs),
+        _arr(_lib.ptr(d.state["exp_avg_sq"]) for _, d, _, _ in recs), _arr(_lib.ptr(r) for _, _, r, _ in recs),
+        _arr(_lib.ptr(c) for *_, c in recs),
+        _arr(((r.numel() if r is not None else p.shape[0]) for p, _, r, _ in recs), C.c_int64),
+        _arr((p[0].numel() for p, *_ in recs), C.c_int32), _arr(_lib.ptr(d.done) for _, d, _, _ in recs),
+        _arr(_lib.ptr(d.hist) for _, d, _, _ in recs), _arr((d.n for _, d, _, _ in recs), C.c_int32),
         _lib.stream_ptr(recs[0][0].device)))
     for _, d, r, _ in recs:
         if r is None:
@@ -162,10 +166,10 @@ class Adam(torch.optim.Optimizer):
             sparse = [p for p in ps if p.grad.is_sparse]
             deferred = [p for p in sparse if p in _deferred]
             if deferred:
-                self._deferred_step(deferred, group, wd, int(step_t))
+                self._sparse_step(deferred, group, wd, int(step_t), exact=True)
             lazy = [p for p in sparse if p not in _deferred]
             if lazy:
-                self._rows_step(lazy, group, wd, int(step_t))
+                self._sparse_step(lazy, group, wd, int(step_t), exact=False)
             ps = [p for p in ps if not p.grad.is_sparse]
             flush(p for p in ps if p in _deferred)         # a marked parameter with a dense gradient: current, then dense
             if not ps:
@@ -189,40 +193,31 @@ class Adam(torch.optim.Optimizer):
                                            _lib.stream_ptr(ps[0].device)))
         return loss
 
-    def _rows_step(self, ps, group, wd: float, step: int) -> None:
-        n = len(ps)
-        arr = lambda vals, t=C.c_void_p: (t * n)(*vals)
+    def _sparse_step(self, ps, group, wd: float, step: int, exact: bool) -> None:
+        """row-wise step of parameters with sparse gradients: intel_adam_deferred_rows_step for marked parameters (exact),
+        intel_adam_rows_step for the others (lazy)"""
         rows, vals = zip(*[_rows_and_values(p, p.grad) for p in ps])     # (kept alive until the launch is queued)
         st = [self.state[p] for p in ps]
+        cols = [_arr(_lib.ptr(p) for p in ps), _arr(_lib.ptr(s["exp_avg"]) for s in st), _arr(_lib.ptr(s["exp_avg_sq"]) for s in st),
+                _arr(_lib.ptr(r) for r in rows), _arr(_lib.ptr(v) for v in vals), _arr((r.numel() for r in rows), C.c_int64),
+                _arr((p[0].numel() for p in ps), C.c_int32), _arr([wd] * len(ps), C.c_float)]
+        if exact:
+            recs = []
+            for p, s in zip(ps, st):
+                d = _deferred.get(p)
+                if d is not None and d.state is not s:       # pending updates of another optimizer's state: apply them first
+                    flush([p])
+                    d = None
+                if d is None:
+                    d = _deferred[p] = _Deferred(p, s)
+                d.record()
+                recs.append(d)
+            cols += [_arr(_lib.ptr(d.done) for d in recs), _arr(_lib.ptr(d.hist) for d in recs), _arr((d.n for d in recs), C.c_int32)]
+        lib = _lib.load()
+        fn = lib.intel_adam_deferred_rows_step if exact else lib.intel_adam_rows_step
         b1, b2 = group["betas"]
-        _lib.check(_lib.load().intel_adam_rows_step(
-            n, arr([_lib.ptr(p) for p in ps]), arr([_lib.ptr(s["exp_avg"]) for s in st]),
-            arr([_lib.ptr(s["exp_avg_sq"]) for s in st]), arr([_lib.ptr(r) for r in rows]), arr([_lib.ptr(v) for v in vals]),
-            arr([r.numel() for r in rows], C.c_int64), arr([p[0].numel() for p in ps], C.c_int32), arr([wd] * n, C.c_float),
-            float(group["lr"]), float(b1), float(b2), float(group["eps"]), step, _lib.stream_ptr(ps[0].device)))
-
-    def _deferred_step(self, ps, group, wd: float, step: int) -> None:
-        n = len(ps)
-        arr = lambda vals, t=C.c_void_p: (t * n)(*vals)
-        rows, vals = zip(*[_rows_and_values(p, p.grad) for p in ps])
-        st = [self.state[p] for p in ps]
-        recs = []
-        for p, s in zip(ps, st):
-            d = _deferred.get(p)
-            if d is not None and d.state is not s:           # pending updates of another optimizer's state: apply them first
-                flush([p])
-                d = None
-            if d is None:
-                d = _deferred[p] = _Deferred(p, s)
-            d.record()
-            recs.append(d)
-        b1, b2 = group["betas"]
-        _lib.check(_lib.load().intel_adam_deferred_rows_step(
-            n, arr([_lib.ptr(p) for p in ps]), arr([_lib.ptr(s["exp_avg"]) for s in st]),
-            arr([_lib.ptr(s["exp_avg_sq"]) for s in st]), arr([_lib.ptr(r) for r in rows]), arr([_lib.ptr(v) for v in vals]),
-            arr([r.numel() for r in rows], C.c_int64), arr([p[0].numel() for p in ps], C.c_int32), arr([wd] * n, C.c_float),
-            arr([_lib.ptr(d.done) for d in recs]), arr([_lib.ptr(d.hist) for d in recs]), arr([d.n for d in recs], C.c_int32),
-            float(group["lr"]), float(b1), float(b2), float(group["eps"]), step, _lib.stream_ptr(ps[0].device)))
+        _lib.check(fn(len(ps), *cols, float(group["lr"]), float(b1), float(b2), float(group["eps"]), step,
+                      _lib.stream_ptr(ps[0].device)))
 
     def flush(self, params: Optional[Iterable[torch.Tensor]] = None) -> None:
         """Apply the deferred updates of ``params`` (default: every parameter of this optimizer).  Afterwards parameters
