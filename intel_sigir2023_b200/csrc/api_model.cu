@@ -30,39 +30,15 @@ int check_dims(const intel_dims_t* d) {
 // ================================================================================================
 // self-attention stack (IntEL.py:182-197): N iterations sharing one set of weights
 // ================================================================================================
-struct StackWs {
-    float* X[9];       // X[0] = input, X[l+1] = output of iteration l  (layers <= 8)
-    float* QKV[8];
-    float* A[8];
-    float* U[8];
-    float* Z[8];
-    float* st[8];
-};
-
-void stack_layout(Arena& a, int64_t R, int d, int layers, StackWs& w) {
-    w.X[0] = a.take<float>(R * d);
-    for (int l = 0; l < layers; ++l) {
-        w.QKV[l] = a.take<float>(R * 3 * d);
-        w.A[l] = a.take<float>(R * d);
-        w.U[l] = a.take<float>(R * d);
-        w.Z[l] = a.take<float>(R * d);
-        w.st[l] = a.take<float>(R * 2);
-        w.X[l + 1] = a.take<float>(R * d);
-    }
-}
-
 int g_use_fused_stack = 1;
 
-int stack_fwd(int64_t B, int64_t L, int d, int heads, int layers, const intel_selfatt_t& p, StackWs& w, float drop_p,
+int stack_fwd(int64_t B, int64_t L, int d, int heads, int layers, const intel_selfatt_t& p, const StackWs& w, float drop_p,
               uint64_t drop_seed, int stream_id, cudaStream_t s, bool save = true) {
     const int64_t R = B * L;
     // whole stack of a session on chip: tcgen05 kernel (trunk_tc.cu, L <= 128) or the mma.sync kernel (trunk.cu, L <= 64);
     // both leave the same activations behind, which the fused and the staged backward passes read alike
-    if (g_use_fused_stack && d == TD && trunk_fwd_supported(L, heads, layers)) {
-        const StackParams sp{p.wq, p.wk, p.wv, p.w1, p.b1, p.w2, p.b2, p.lnw, p.lnb};
-        const StackSaved sv{w.QKV, w.A, w.U, w.Z, w.st};
-        return trunk_fwd(B, L, heads, layers, sp, w.X, sv, drop_p, drop_seed, stream_id, s, save);
-    }
+    if (g_use_fused_stack && d == TD && trunk_fwd_supported(L, heads, layers))
+        return trunk_fwd(B, L, heads, layers, p, w, drop_p, drop_seed, stream_id, s, save);
     for (int l = 0; l < layers; ++l) {
         INTEL_TRY(linear(R, d, d, w.X[l], d, p.wq, d, nullptr, w.QKV[l], 3 * d, s));
         INTEL_TRY(linear(R, d, d, w.X[l], d, p.wk, d, nullptr, w.QKV[l] + d, 3 * d, s));
@@ -81,16 +57,12 @@ int stack_fwd(int64_t B, int64_t L, int d, int heads, int layers, const intel_se
 }
 
 // dX holds d(loss)/d X[layers] on entry and d(loss)/d X[0] on return.  t1, t2: [R,d] scratch; dqkv: [R,3d].
-int stack_bwd(int64_t B, int64_t L, int d, int heads, int layers, const intel_selfatt_t& p, intel_selfatt_t& g,
-              StackWs& w, float* dX, float* t1, float* t2, float* dqkv, float drop_p, uint64_t drop_seed, int stream_id,
+int stack_bwd(int64_t B, int64_t L, int d, int heads, int layers, const intel_selfatt_t& p, const intel_selfatt_t& g,
+              const StackWs& w, float* dX, float* t1, float* t2, float* dqkv, float drop_p, uint64_t drop_seed, int stream_id,
               cudaStream_t s) {
     const int64_t R = B * L;
-    if (g_use_fused_stack && trunk_supported(L, d, heads, layers)) {
-        const StackParams sp{p.wq, p.wk, p.wv, p.w1, p.b1, p.w2, p.b2, p.lnw, p.lnb};
-        const StackGrads sg{g.wq, g.wk, g.wv, g.w1, g.b1, g.w2, g.b2, g.lnw, g.lnb};
-        const StackSaved sv{w.QKV, w.A, w.U, w.Z, w.st};
-        return trunk_bwd(B, L, heads, layers, sp, sg, w.X, sv, dX, drop_p, drop_seed, stream_id, s);
-    }
+    if (g_use_fused_stack && trunk_supported(L, d, heads, layers))
+        return trunk_bwd(B, L, heads, layers, p, g, w, dX, drop_p, drop_seed, stream_id, s);
     for (int l = layers - 1; l >= 0; --l) {
         float* dZ = t1;
         INTEL_TRY(layernorm_bwd(R, d, dX, w.Z[l], w.st[l], p.lnw, dZ, g.lnw, g.lnb, s));
@@ -120,27 +92,46 @@ int stack_bwd(int64_t B, int64_t L, int d, int heads, int layers, const intel_se
 // ================================================================================================
 // ensemble workspace
 // ================================================================================================
+// The two self-attention streams of predict_ensemble, 0 = item and 1 = score: each has its width d, its column block
+// [off, off + d) of the head input, and its own tensors in the parameters (or the gradients).
+struct Stream {
+    int d, off;
+    const intel_selfatt_t* stack;
+    float *xk, *xv;              // intent_*_attention.{key,value}_layer (cross_attention = 1)
+    float *w0, *b0, *w2;         // intent_*_embeddings.{0,2} (cross_attention = 0)
+};
+void streams_of(const intel_dims_t* d, const intel_tensors_t* T, Stream (&st)[2]) {
+    const int di = d->d_iid + d->d_im;
+    st[0] = {di, 0, &T->item, T->xk_item, T->xv_item, T->gate_item_w0, T->gate_item_b0, T->gate_item_w2};
+    st[1] = {d->d_s, di, &T->score, T->xk_score, T->xv_score, T->gate_score_w0, T->gate_score_b0, T->gate_score_w2};
+}
+
+// The three weights that read the predicted intents (query_layer of each stream, intent_embeddings) already back to back,
+// as the [di + ds + dint, I] matrix Wcat of the one product against the intents
+bool intent_weights_stacked(const intel_tensors_t* T, int di, int ds, int64_t I) {
+    return T->xq_score == T->xq_item + (int64_t)di * I && T->intent_w == T->xq_score + (int64_t)ds * I;
+}
+
 struct EnsWs {
-    StackWs item, score;
+    StackWs stack[2];             // per stream
     float* xs;                    // float copy of the scores [R,K]
-    float *q_i, *q_s, *qk_i, *qk_s, *p_i, *p_s, *xbar_i, *xbar_s;   // cross attention
+    float *q[2], *qk[2], *p[2], *xbar[2];   // cross attention, per stream
     // the three products that read the predicted intents ([B, I] x {query_layer (item), query_layer (score),
     // intent_embeddings}) run as one: Wcat [di + ds + dint, I] = the three weights stacked, qcat / dcat [B, di + ds + dint]
     float *Wcat, *qcat, *dcat;
     float* all;                   // [B, D] head input of the valid rows
     float *w_valid, *w_pad;       // [B,K]
-    float *t_i, *t_s, *m_i, *m_s, *hu, *hint, *all_item;            // cross_attention = 0
+    float *t[2], *m[2], *hu, *hint, *all_item;                      // cross_attention = 0
     // backward scratch
-    float *dall, *dwv, *dwp, *dxbar, *dqk, *dq, *dXa, *dXs, *t1, *t2, *dqkv;   // dXa / dXs: d(stack output) of the item / score stream
+    float *dall, *dwv, *dwp, *dxbar, *dqk, *dq, *dX[2], *t1, *t2, *dqkv;   // dX: d(stack output) of each stream
     float *g, *dall_item, *dm, *dt, *dvec;
 };
 
 void ens_layout(const intel_dims_t* d, Arena& a, EnsWs& w) {
     const int64_t B = d->B, L = d->L, R = B * L;
     const int di = d->d_iid + d->d_im, ds = d->d_s, D = di + ds + d->d_u + d->d_int;
-    const int dmax = di > ds ? di : ds;
-    stack_layout(a, R, di, d->layers, w.item);
-    stack_layout(a, R, ds, d->layers, w.score);
+    const int dmax = di > ds ? di : ds, dst[2] = {di, ds};
+    for (int st = 0; st < 2; ++st) stack_layout(a, R, dst[st], d->layers, w.stack[st]);
     w.xs = a.take<float>(R * d->K);
     w.all = a.take<float>(B * D);
     w.w_valid = a.take<float>(B * d->K);
@@ -148,8 +139,7 @@ void ens_layout(const intel_dims_t* d, Arena& a, EnsWs& w) {
     w.dall = a.take<float>(B * D);
     w.dwv = a.take<float>(B * d->K);
     w.dwp = a.take<float>(B * d->K);
-    w.dXa = a.take<float>(R * dmax);
-    w.dXs = a.take<float>(R * dmax);
+    for (float*& x : w.dX) x = a.take<float>(R * dmax);
     w.t1 = a.take<float>(R * dmax);
     w.t2 = a.take<float>(R * dmax);
     w.dqkv = a.take<float>(R * 3 * dmax);
@@ -158,16 +148,16 @@ void ens_layout(const intel_dims_t* d, Arena& a, EnsWs& w) {
         w.Wcat = a.take<float>((int64_t)dc * d->I);
         w.qcat = a.take<float>(B * dc);
         w.dcat = a.take<float>(B * dc);
-        w.q_i = w.qcat; w.q_s = w.qcat + di;                    // column blocks of qcat (row stride dc)
-        w.qk_i = a.take<float>(B * di); w.qk_s = a.take<float>(B * ds);
-        w.p_i = a.take<float>(B * L); w.p_s = a.take<float>(B * L);
-        w.xbar_i = a.take<float>(B * di); w.xbar_s = a.take<float>(B * ds);
+        w.q[0] = w.qcat; w.q[1] = w.qcat + di;                  // column blocks of qcat (row stride dc)
+        for (int st = 0; st < 2; ++st) w.qk[st] = a.take<float>(B * dst[st]);
+        for (float*& x : w.p) x = a.take<float>(B * L);
+        for (int st = 0; st < 2; ++st) w.xbar[st] = a.take<float>(B * dst[st]);
         w.dxbar = a.take<float>(B * dmax);
         w.dqk = a.take<float>(B * dmax);
         w.dq = a.take<float>(B * dmax);
     } else {
-        w.t_i = a.take<float>(B * d->qsize); w.t_s = a.take<float>(B * d->qsize);
-        w.m_i = a.take<float>(B * di); w.m_s = a.take<float>(B * ds);
+        for (float*& x : w.t) x = a.take<float>(B * d->qsize);
+        for (int st = 0; st < 2; ++st) w.m[st] = a.take<float>(B * dst[st]);
         w.hu = a.take<float>(B * d->d_u); w.hint = a.take<float>(B * d->d_int);
         w.all_item = a.take<float>(R * D);
         w.g = a.take<float>(R * d->K);
@@ -186,7 +176,8 @@ struct BertWs {
     float *QKV[INTEL_MAX_BERT_LAYERS], *Z1[INTEL_MAX_BERT_LAYERS], *st1[INTEL_MAX_BERT_LAYERS], *C[INTEL_MAX_BERT_LAYERS],
         *F[INTEL_MAX_BERT_LAYERS], *Z2[INTEL_MAX_BERT_LAYERS], *st2[INTEL_MAX_BERT_LAYERS];
 };
-struct GruWs { float *gi, *h_all, *gates, *gh, *dh, *dgi, *dgh_all; int32_t *order, *rows_t, *rows_t1, *nlive; bool sorted; };   // sorted: set and read inside one call only
+// packed: the int32 live-row lists can address every row of [B, T + 1, .]; sorted: set and read inside one call only
+struct GruWs { float *gi, *h_all, *gates, *gh, *dh, *dgi, *dgh_all; int32_t *order, *rows_t, *rows_t1, *nlive; bool packed, sorted; };
 struct EncWs {
     int64_t T; int d;
     float* seq;          // [B*T, d] token embeddings (BERT: positions added in place)
@@ -197,10 +188,32 @@ struct EncWs {
 struct IntWs {
     float* Wt;           // [I, d_int] transpose of intent_embeddings.weight
     float* dWt;
-    EncWs e1, e2;
+    EncWs e[2];          // per history
     float *feat, *logits, *dlogits, *dfeat;
     float *t1, *t2, *dqkv;   // bert backward scratch
 };
+
+// The two histories of predict_intent, 0 = session history (encoder), 1 = item history (item_encoder).  A token of a
+// history is [table row of its id | intent embedding of its intents], split at column dtok; the intents are dense float64
+// rows [B*T, I] or, when idx is set, nz compact entries per row.  The encoded history goes to columns [off, off + d) of feat.
+struct History {
+    const float* table; float* gtable; const int64_t* ids; int64_t table_rows; const int32_t* map; int dtok;
+    const double* dense; const char* dense_name; const int32_t* idx; const float* val; int nz;
+    const int64_t* lens;
+    int off;
+    const intel_encoder_t* p; intel_encoder_t* g;
+};
+// G and M may be null (the forward pass)
+void histories_of(const intel_dims_t* d, const intel_tensors_t* P, intel_tensors_t* G, const intel_row_maps_t* M,
+                  const intel_batch_t* bt, History (&h)[2]) {
+    const int off2 = d->d_ctx + d->d_u, off1 = off2 + d->d_iid + d->d_int;   // pred_layer input = [ctx | user | item-history | history]
+    h[0] = {P->ctx_emb, G ? G->ctx_emb : nullptr, bt->his_context, d->ctx_rows, M ? M->ctx : nullptr, d->d_ctx,
+            bt->his_intents, "his_intents", bt->his_intents_idx, bt->his_intents_val, bt->nz1,
+            bt->history_len, off1, &P->enc, G ? &G->enc : nullptr};
+    h[1] = {P->iid_emb, G ? G->iid_emb : nullptr, bt->his_item_id, d->item_rows, M ? M->iid : nullptr, d->d_iid,
+            bt->his_item_int, "his_item_int", bt->his_item_int_idx, bt->his_item_int_val, bt->nz2,
+            bt->history_item_len, off2, &P->item_enc, G ? &G->item_enc : nullptr};
+}
 
 void enc_layout(const intel_dims_t* d, Arena& a, EncWs& e, int64_t T, int dd) {
     const int64_t B = d->B, R = B * T;
@@ -235,6 +248,7 @@ void enc_layout(const intel_dims_t* d, Arena& a, EncWs& e, int64_t T, int dd) {
         e.gru.rows_t = a.take<int32_t>(R);
         e.gru.rows_t1 = a.take<int32_t>(R);
         e.gru.nlive = a.take<int32_t>(4);
+        e.gru.packed = B * (T + 1) < (1LL << 31);
     }
 }
 
@@ -243,8 +257,8 @@ void int_layout(const intel_dims_t* d, Arena& a, IntWs& w) {
     const int Dp = d1 + d2 + d->d_ctx + d->d_u;
     w.Wt = a.take<float>(d->I * d->d_int);
     w.dWt = a.take<float>(d->I * d->d_int);
-    enc_layout(d, a, w.e1, d->H1, d1);
-    enc_layout(d, a, w.e2, d->H2, d2);
+    enc_layout(d, a, w.e[0], d->H1, d1);
+    enc_layout(d, a, w.e[1], d->H2, d2);
     w.feat = a.take<float>(d->B * Dp);
     w.logits = a.take<float>(d->B * pad4(d->I));       // rows padded to 16 bytes: intent_num is odd in every config
     w.dlogits = a.take<float>(d->B * pad4(d->I));
@@ -322,8 +336,7 @@ int bert_bwd(const intel_dims_t* d, const intel_encoder_t& p, intel_encoder_t& g
 // Both GRU encoders of predict_intent (session history, item history) in three stages: input projections, recurrences,
 // output projections.  The recurrences of the two encoders share one launch (gru_tc.cu): each is a chain of T dependent steps
 // that leaves the tensor pipe idle most of the time, so they are overlapped instead of run back to back.
-int gru_fwd_pair(const intel_dims_t* d, const intel_encoder_t* const (&p)[2], EncWs* const (&e)[2], const int64_t* const (&lens)[2],
-                 float* const (&out)[2], int64_t ld_out, cudaStream_t s) {
+int gru_fwd_pair(const intel_dims_t* d, const History (&hs)[2], EncWs (&e)[2], float* feat, int64_t ld_out, cudaStream_t s) {
     const int64_t B = d->B;
     const int h = d->gru_hidden;
     bool fused = h == 128 && gru_tc_supported(h);
@@ -332,10 +345,9 @@ int gru_fwd_pair(const intel_dims_t* d, const intel_encoder_t* const (&p)[2], En
         const int64_t* ls[2];
         int32_t *rt[2], *rt1[2], *cn[2], *od[2];
         for (int i = 0; i < 2; ++i) {
-            GruWs& w = e[i]->gru;
-            Bs[i] = B; Ts[i] = e[i]->T; ls[i] = lens[i];
-            const bool packed = B * (Ts[i] + 1) < (1LL << 31);
-            rt[i] = packed ? w.rows_t : nullptr; rt1[i] = packed ? w.rows_t1 : nullptr; cn[i] = packed ? w.nlive : nullptr;
+            GruWs& w = e[i].gru;
+            Bs[i] = B; Ts[i] = e[i].T; ls[i] = hs[i].lens;
+            rt[i] = w.packed ? w.rows_t : nullptr; rt1[i] = w.packed ? w.rows_t1 : nullptr; cn[i] = w.packed ? w.nlive : nullptr;
             w.sorted = Ts[i] <= 63;
             od[i] = w.sorted ? w.order : nullptr;
             fused = fused && w.sorted;
@@ -343,15 +355,14 @@ int gru_fwd_pair(const intel_dims_t* d, const intel_encoder_t* const (&p)[2], En
         INTEL_TRY(gru_prep(2, Bs, Ts, ls, rt, rt1, cn, od, s));
     }
     for (int i = 0; i < 2; ++i) {
-        const int64_t T = e[i]->T, R = B * T;
-        const int dd = e[i]->d;
-        GruWs& w = e[i]->gru;
+        const int64_t T = e[i].T, R = B * T;
+        const int dd = e[i].d;
+        GruWs& w = e[i].gru;
         // the products over the [B, T] history rows walk the live rows only (about half of them are padding behind a
         // session's length; the reference packs the sequences: GeneralSeq.py:64-71).  gi rows of padding slots stay
         // unwritten: nobody reads them.
-        const bool packed = B * (T + 1) < (1LL << 31);
-        INTEL_TRY(linear(R, 3 * h, dd, e[i]->seq, dd, p[i]->w_ih, dd, p[i]->b_ih, w.gi, 3 * h, s, false, false, nullptr, 0,
-                         packed ? w.rows_t : nullptr, packed ? w.nlive : nullptr));
+        INTEL_TRY(linear(R, 3 * h, dd, e[i].seq, dd, hs[i].p->w_ih, dd, hs[i].p->b_ih, w.gi, 3 * h, s, false, false, nullptr, 0,
+                         w.packed ? w.rows_t : nullptr, w.packed ? w.nlive : nullptr));
         if (h == 128) {
             // the fused kernels write h_all[:, 1..T] of every session themselves: only the initial state h_0 needs clearing
             // (2 MB instead of a 44 MB memset per encoder and step)
@@ -365,35 +376,37 @@ int gru_fwd_pair(const intel_dims_t* d, const intel_encoder_t* const (&p)[2], En
         GruTcPair pr;
         pr.n = 2;
         for (int i = 0; i < 2; ++i) {
-            GruWs& w = e[i]->gru;
-            pr.e[i] = GruTcOne{B, e[i]->T, lens[i], w.gi, p[i]->w_hh, p[i]->b_hh, w.h_all, w.gates, w.order};
+            GruWs& w = e[i].gru;
+            pr.e[i] = GruTcOne{B, e[i].T, hs[i].lens, w.gi, hs[i].p->w_hh, hs[i].p->b_hh, w.h_all, w.gates, w.order};
         }
         INTEL_TRY(gru_tc_fwd_pair(pr, s, d->inference == 0));
     } else {
         for (int i = 0; i < 2; ++i) {
-            const int64_t T = e[i]->T;
-            GruWs& w = e[i]->gru;
+            const int64_t T = e[i].T;
+            const intel_encoder_t& p = *hs[i].p;
+            GruWs& w = e[i].gru;
             if (h == 128) {
-                INTEL_TRY(gru_seq_fwd(B, T, h, lens[i], w.gi, p[i]->w_hh, p[i]->b_hh, w.h_all, w.gates, s, d->inference == 0));
+                INTEL_TRY(gru_seq_fwd(B, T, h, hs[i].lens, w.gi, p.w_hh, p.b_hh, w.h_all, w.gates, s, d->inference == 0));
             } else {
                 for (int64_t t = 0; t < T; ++t) {
-                    INTEL_TRY(linear(B, 3 * h, h, w.h_all + t * h, (T + 1) * h, p[i]->w_hh, h, p[i]->b_hh, w.gh, 3 * h, s));
-                    INTEL_TRY(gru_step_fwd(B, T, h, (int)t, lens[i], w.gi, w.gh, w.h_all, w.gates, s));
+                    INTEL_TRY(linear(B, 3 * h, h, w.h_all + t * h, (T + 1) * h, p.w_hh, h, p.b_hh, w.gh, 3 * h, s));
+                    INTEL_TRY(gru_step_fwd(B, T, h, (int)t, hs[i].lens, w.gi, w.gh, w.h_all, w.gates, s));
                 }
             }
         }
     }
-    if (gru_outproj_pair_ok(h, e[0]->d, e[1]->d)) {          // both output projections in one launch
-        const int n[2] = {e[0]->d, e[1]->d};
-        const float* W[2] = {p[0]->w_out, p[1]->w_out};
-        const float* hl[2] = {e[0]->gru.h_all + e[0]->T * h, e[1]->gru.h_all + e[1]->T * h};
-        const int64_t ldh[2] = {(e[0]->T + 1) * h, (e[1]->T + 1) * h}, ldo[2] = {ld_out, ld_out};
+    if (gru_outproj_pair_ok(h, e[0].d, e[1].d)) {          // both output projections in one launch
+        const int n[2] = {e[0].d, e[1].d};
+        const float* W[2] = {hs[0].p->w_out, hs[1].p->w_out};
+        const float* hl[2] = {e[0].gru.h_all + e[0].T * h, e[1].gru.h_all + e[1].T * h};
+        float* const out[2] = {feat + hs[0].off, feat + hs[1].off};
+        const int64_t ldh[2] = {(e[0].T + 1) * h, (e[1].T + 1) * h}, ldo[2] = {ld_out, ld_out};
         return gru_outproj_pair_fwd(B, n, W, hl, ldh, out, ldo, s);
     }
     for (int i = 0; i < 2; ++i) {
-        const int64_t T = e[i]->T;
-        GruWs& w = e[i]->gru;
-        INTEL_TRY(linear(B, e[i]->d, h, w.h_all + T * h, (T + 1) * h, p[i]->w_out, h, nullptr, out[i], ld_out, s));
+        const int64_t T = e[i].T;
+        GruWs& w = e[i].gru;
+        INTEL_TRY(linear(B, e[i].d, h, w.h_all + T * h, (T + 1) * h, hs[i].p->w_out, h, nullptr, feat + hs[i].off, ld_out, s));
     }
     return INTEL_OK;
 }
@@ -427,11 +440,10 @@ int gru_bwd(const intel_dims_t* d, const intel_encoder_t& p, intel_encoder_t& g,
     }
     // gradient rows of padding slots are zero: the three products below contract / map the live rows only (the list was
     // built by the forward call); d(seq) of the padding slots is cleared for the scatters that read every row
-    const bool packed = B * (T + 1) < (1LL << 31);
-    const int32_t *rt = packed ? w.rows_t : nullptr, *rt1 = packed ? w.rows_t1 : nullptr, *nl = packed ? w.nlive : nullptr;
+    const int32_t *rt = w.packed ? w.rows_t : nullptr, *rt1 = w.packed ? w.rows_t1 : nullptr, *nl = w.packed ? w.nlive : nullptr;
     INTEL_TRY(linear_dw(B * (T + 1), 3 * h, h, w.dgh_all, 3 * h, w.h_all, h, g.w_hh, h, h == 128 ? nullptr : g.b_hh, s, false, rt1, nl));
     INTEL_TRY(linear_dw(R, 3 * h, dd, w.dgi, 3 * h, e.seq, dd, g.w_ih, dd, h == 128 ? nullptr : g.b_ih, s, false, rt, nl));
-    if (packed) INTEL_TRY(fill_zero(e.dseq, (size_t)R * dd * 4, s));
+    if (w.packed) INTEL_TRY(fill_zero(e.dseq, (size_t)R * dd * 4, s));
     return linear_dx(R, 3 * h, dd, w.dgi, 3 * h, p.w_ih, dd, e.dseq, dd, s, 0, nullptr, 0, rt, nl);
 }
 
@@ -511,15 +523,16 @@ int intel_ensemble_fwd(const intel_dims_t* d, const intel_tensors_t* P, const in
     const int64_t B = d->B, L = d->L, R = B * L, I = d->I;
     const int K = (int)d->K, di = d->d_iid + d->d_im, ds = d->d_s, du = d->d_u, dint = d->d_int;
     const int D = di + ds + du + dint, off_u = di + ds, off_h = di + ds + du;
+    Stream ps[2];
+    streams_of(d, P, ps);
 
     // embedding gathers straight into the concatenated item-stream rows (IntEL.py:170-175)
-    INTEL_TRY(gather_rows(R, d->d_iid, P->iid_emb, bt->i_id, w.item.X[0], di, 0, s, d->item_rows));
-    if (d->d_im > 0) INTEL_TRY(gather_rows(R, d->d_im, P->item_emb, bt->i_class, w.item.X[0] + d->d_iid, di, 0, s, d->class_rows));
-    INTEL_TRY(score_embed_fwd(R, K, ds, bt->scores, P->score_w, P->score_b, w.score.X[0], w.xs, s));
-    INTEL_TRY(stack_fwd(B, L, di, d->heads, d->layers, P->item, w.item, d->dropout_p, d->dropout_seed, 0, s, d->inference == 0));
-    INTEL_TRY(stack_fwd(B, L, ds, d->heads, d->layers, P->score, w.score, d->dropout_p, d->dropout_seed, 1, s, d->inference == 0));
-    float* Xi = w.item.X[d->layers];
-    float* Xs = w.score.X[d->layers];
+    INTEL_TRY(gather_rows(R, d->d_iid, P->iid_emb, bt->i_id, w.stack[0].X[0], di, 0, s, d->item_rows));
+    if (d->d_im > 0) INTEL_TRY(gather_rows(R, d->d_im, P->item_emb, bt->i_class, w.stack[0].X[0] + d->d_iid, di, 0, s, d->class_rows));
+    INTEL_TRY(score_embed_fwd(R, K, ds, bt->scores, P->score_w, P->score_b, w.stack[1].X[0], w.xs, s));
+    for (int st = 0; st < 2; ++st)     // stream_id st: the two stacks draw different dropout masks
+        INTEL_TRY(stack_fwd(B, L, ps[st].d, d->heads, d->layers, *ps[st].stack, w.stack[st], d->dropout_p, d->dropout_seed, st, s,
+                            d->inference == 0));
 
     if (d->cross_attention) {
         const float scale = 1.0f / sqrtf((float)d->qsize);
@@ -527,28 +540,25 @@ int intel_ensemble_fwd(const intel_dims_t* d, const intel_tensors_t* P, const in
         // three times); the weights are stacked into Wcat unless the caller already keeps them back to back
         const int dc = di + ds + dint;
         const float* Wc = P->xq_item;
-        if (!(P->xq_score == P->xq_item + (int64_t)di * I && P->intent_w == P->xq_score + (int64_t)ds * I)) {
+        if (!intent_weights_stacked(P, di, ds, I)) {
             INTEL_TRY(copy_d2d(w.Wcat, P->xq_item, (size_t)di * I * 4, s));
             INTEL_TRY(copy_d2d(w.Wcat + (int64_t)di * I, P->xq_score, (size_t)ds * I * 4, s));
             INTEL_TRY(copy_d2d(w.Wcat + (int64_t)(di + ds) * I, P->intent_w, (size_t)dint * I * 4, s));
             Wc = w.Wcat;
         }
         INTEL_TRY(linear(B, dc, I, intents, I, Wc, I, nullptr, w.qcat, dc, s));
-        // item stream, score stream: qk = W_k^T q, the pooling, the value projection into the head input
-        if (cross_full_ok(di, L) && al16(P->xk_item) && al16(P->xv_item)) {
-            INTEL_TRY(cross_full_fwd(B, L, Xi, w.q_i, dc, P->xk_item, P->xv_item, bt->session_len, scale, w.p_i, w.qk_i, w.xbar_i, w.all, D, s));
-        } else {
-            INTEL_TRY(linear_dx(B, di, di, w.q_i, dc, P->xk_item, di, w.qk_i, di, s));            // qk = W_k^T q
-            INTEL_TRY(cross_pool_fwd(B, L, di, Xi, w.qk_i, bt->session_len, scale, w.p_i, w.xbar_i, s));
-            INTEL_TRY(linear(B, di, di, w.xbar_i, di, P->xv_item, di, nullptr, w.all, D, s));
-        }
-        if (cross_full_ok(ds, L) && al16(P->xk_score) && al16(P->xv_score)) {
-            INTEL_TRY(cross_full_fwd(B, L, Xs, w.q_s, dc, P->xk_score, P->xv_score, bt->session_len, scale, w.p_s, w.qk_s, w.xbar_s,
-                                     w.all + di, D, s));
-        } else {
-            INTEL_TRY(linear_dx(B, ds, ds, w.q_s, dc, P->xk_score, ds, w.qk_s, ds, s));
-            INTEL_TRY(cross_pool_fwd(B, L, ds, Xs, w.qk_s, bt->session_len, scale, w.p_s, w.xbar_s, s));
-            INTEL_TRY(linear(B, ds, ds, w.xbar_s, ds, P->xv_score, ds, nullptr, w.all + di, D, s));
+        // per stream: qk = W_k^T q, the pooling, the value projection into the head input
+        for (int st = 0; st < 2; ++st) {
+            const Stream& c = ps[st];
+            const float* X = w.stack[st].X[d->layers];
+            if (cross_full_ok(c.d, L) && al16(c.xk) && al16(c.xv)) {
+                INTEL_TRY(cross_full_fwd(B, L, X, w.q[st], dc, c.xk, c.xv, bt->session_len, scale, w.p[st], w.qk[st], w.xbar[st],
+                                         w.all + c.off, D, s));
+            } else {
+                INTEL_TRY(linear_dx(B, c.d, c.d, w.q[st], dc, c.xk, c.d, w.qk[st], c.d, s));            // qk = W_k^T q
+                INTEL_TRY(cross_pool_fwd(B, L, c.d, X, w.qk[st], bt->session_len, scale, w.p[st], w.xbar[st], s));
+                INTEL_TRY(linear(B, c.d, c.d, w.xbar[st], c.d, c.xv, c.d, nullptr, w.all + c.off, D, s));
+            }
         }
         // user + intent parts of the head input
         INTEL_TRY(gather_rows(B, du, P->uid_emb, bt->u_id, w.all + off_u, D, 1, s, d->user_rows));
@@ -563,12 +573,13 @@ int intel_ensemble_fwd(const intel_dims_t* d, const intel_tensors_t* P, const in
         }
     } else {
         const int q = d->qsize;
-        INTEL_TRY(linear(B, q, I, intents, I, P->gate_item_w0, I, P->gate_item_b0, w.t_i, q, s, false, true));
-        INTEL_TRY(linear(B, di, q, w.t_i, q, P->gate_item_w2, q, nullptr, w.m_i, di, s));
-        INTEL_TRY(linear(B, q, I, intents, I, P->gate_score_w0, I, P->gate_score_b0, w.t_s, q, s, false, true));
-        INTEL_TRY(linear(B, ds, q, w.t_s, q, P->gate_score_w2, q, nullptr, w.m_s, ds, s));
-        INTEL_TRY(gate_fwd(B, L, di, Xi, w.m_i, w.all_item, D, s));
-        INTEL_TRY(gate_fwd(B, L, ds, Xs, w.m_s, w.all_item + di, D, s));
+        for (int st = 0; st < 2; ++st) {
+            const Stream& c = ps[st];
+            INTEL_TRY(linear(B, q, I, intents, I, c.w0, I, c.b0, w.t[st], q, s, false, true));
+            INTEL_TRY(linear(B, c.d, q, w.t[st], q, c.w2, q, nullptr, w.m[st], c.d, s));
+        }
+        for (int st = 0; st < 2; ++st)
+            INTEL_TRY(gate_fwd(B, L, ps[st].d, w.stack[st].X[d->layers], w.m[st], w.all_item + ps[st].off, D, s));
         INTEL_TRY(gather_rows(B, du, P->uid_emb, bt->u_id, w.hu, du, 1, s, d->user_rows));
         INTEL_TRY(bcast_rows(B, L, du, w.hu, du, w.all_item + off_u, D, s));
         INTEL_TRY(linear(B, dint, I, intents, I, P->intent_w, I, P->intent_b, w.hint, dint, s, false, true));
@@ -600,10 +611,10 @@ int intel_ensemble_bwd_phase_rows(const intel_dims_t* d, const intel_tensors_t* 
     const int64_t B = d->B, L = d->L, R = B * L, I = d->I;
     const int K = (int)d->K, di = d->d_iid + d->d_im, ds = d->d_s, du = d->d_u, dint = d->d_int;
     const int D = di + ds + du + dint, off_u = di + ds, off_h = di + ds + du;
-    float* Xi = w.item.X[d->layers];
-    float* Xs = w.score.X[d->layers];
+    Stream ps[2], gs[2];
+    streams_of(d, P, ps);
+    streams_of(d, G, gs);
 
-    float* const dXst[2] = {w.dXa, w.dXs};
     if (d->cross_attention) {
         const float scale = 1.0f / sqrtf((float)d->qsize);
         if (do_head) {
@@ -624,33 +635,26 @@ int intel_ensemble_bwd_phase_rows(const intel_dims_t* d, const intel_tensors_t* 
         INTEL_TRY(scatter_add_rows(B, du, w.dall + off_u, D, bt->u_id, G->uid_emb, P->uid_emb, s, d->user_rows, M.uid));
         // the two pooled cross attentions
         for (int st = 0; st < 2; ++st) {
-            const int dd = st == 0 ? di : ds;
-            const int off = st == 0 ? 0 : di;
-            float* X = st == 0 ? Xi : Xs;
-            float *q = st == 0 ? w.q_i : w.q_s, *qk = st == 0 ? w.qk_i : w.qk_s, *p = st == 0 ? w.p_i : w.p_s;
-            float* xbar = st == 0 ? w.xbar_i : w.xbar_s;
-            const float *xq = st == 0 ? P->xq_item : P->xq_score, *xk = st == 0 ? P->xk_item : P->xk_score,
-                        *xv = st == 0 ? P->xv_item : P->xv_score;
-            float *gxq = st == 0 ? G->xq_item : G->xq_score, *gxk = st == 0 ? G->xk_item : G->xk_score,
-                  *gxv = st == 0 ? G->xv_item : G->xv_score;
+            const int dd = ps[st].d, off = ps[st].off;
+            const float* X = w.stack[st].X[d->layers];
+            const float *xk = ps[st].xk, *xv = ps[st].xv;
             if (cross_full_ok(dd, L) && al16(xk) && al16(xv)) {
-                INTEL_TRY(cross_full_bwd(B, L, X, q, dc, qk, xk, xv, bt->session_len, scale, p, xbar, w.dall + off, D, dXst[st],
-                                         w.dcat + off, dc, gxk, gxv, s));
+                INTEL_TRY(cross_full_bwd(B, L, X, w.q[st], dc, w.qk[st], xk, xv, bt->session_len, scale, w.p[st], w.xbar[st],
+                                         w.dall + off, D, w.dX[st], w.dcat + off, dc, gs[st].xk, gs[st].xv, s));
             } else {
-                INTEL_TRY(linear_dw(B, dd, dd, w.dall + off, D, xbar, dd, gxv, dd, nullptr, s));
+                INTEL_TRY(linear_dw(B, dd, dd, w.dall + off, D, w.xbar[st], dd, gs[st].xv, dd, nullptr, s));
                 INTEL_TRY(linear_dx(B, dd, dd, w.dall + off, D, xv, dd, w.dxbar, dd, s));
-                INTEL_TRY(cross_pool_bwd(B, L, dd, X, qk, bt->session_len, scale, p, w.dxbar, dXst[st], w.dqk, s));
-                INTEL_TRY(linear_dw(B, dd, dd, q, dc, w.dqk, dd, gxk, dd, nullptr, s));            // dW_k[a,c] = sum q_a dqk_c
+                INTEL_TRY(cross_pool_bwd(B, L, dd, X, w.qk[st], bt->session_len, scale, w.p[st], w.dxbar, w.dX[st], w.dqk, s));
+                INTEL_TRY(linear_dw(B, dd, dd, w.q[st], dc, w.dqk, dd, gs[st].xk, dd, nullptr, s));      // dW_k[a,c] = sum q_a dqk_c
                 INTEL_TRY(linear(B, dd, dd, w.dqk, dd, xk, dd, nullptr, w.dcat + off, dc, s));      // dq = W_k dqk -> its block of dcat
             }
-            (void)xq; (void)gxq;
         }
         // the three products against the predicted intents as one: d_intents = dcat Wcat, dWcat += dcat^T intents
         {
             const float* Wc = P->xq_item;
-            if (!(P->xq_score == P->xq_item + (int64_t)di * I && P->intent_w == P->xq_score + (int64_t)ds * I)) Wc = w.Wcat;   // stacked by the forward call
+            if (!intent_weights_stacked(P, di, ds, I)) Wc = w.Wcat;   // stacked by the forward call
             INTEL_TRY(linear_dx(B, dc, I, w.dcat, dc, Wc, I, d_intents_out, I, s, 0));
-            if (G->xq_score == G->xq_item + (int64_t)di * I && G->intent_w == G->xq_score + (int64_t)ds * I) {
+            if (intent_weights_stacked(G, di, ds, I)) {
                 INTEL_TRY(linear_dw(B, dc, I, w.dcat, dc, intents, I, G->xq_item, I, nullptr, s));
             } else {
                 INTEL_TRY(linear_dw(B, di, I, w.dcat, dc, intents, I, G->xq_item, I, nullptr, s));
@@ -674,38 +678,35 @@ int intel_ensemble_bwd_phase_rows(const intel_dims_t* d, const intel_tensors_t* 
         INTEL_TRY(bcast_rows_bwd(B, L, du, w.dall_item + off_u, D, w.dvec, du, 0, s));
         INTEL_TRY(scatter_add_rows(B, du, w.dvec, du, bt->u_id, G->uid_emb, P->uid_emb, s, d->user_rows, M.uid));
         for (int st = 0; st < 2; ++st) {
-            const int dd = st == 0 ? di : ds;
-            const int off = st == 0 ? 0 : di;
-            float* X = st == 0 ? Xi : Xs;
-            float *m = st == 0 ? w.m_i : w.m_s, *t = st == 0 ? w.t_i : w.t_s;
-            const float *w0 = st == 0 ? P->gate_item_w0 : P->gate_score_w0, *w2 = st == 0 ? P->gate_item_w2 : P->gate_score_w2;
-            float *gw0 = st == 0 ? G->gate_item_w0 : G->gate_score_w0, *gb0 = st == 0 ? G->gate_item_b0 : G->gate_score_b0,
-                  *gw2 = st == 0 ? G->gate_item_w2 : G->gate_score_w2;
-            INTEL_TRY(gate_bwd(B, L, dd, X, m, w.dall_item + off, D, dXst[st], w.dm, s));
-            INTEL_TRY(linear_dw(B, dd, q, w.dm, dd, t, q, gw2, q, nullptr, s));
-            INTEL_TRY(linear_dx(B, dd, q, w.dm, dd, w2, q, w.dt, q, s, 0, t, q));       // relu mask (t = relu(.) > 0)
-            INTEL_TRY(linear_dw(B, q, I, w.dt, q, intents, I, gw0, I, gb0, s));
-            INTEL_TRY(linear_dx(B, q, I, w.dt, q, w0, I, d_intents_out, I, s, 1));
+            const int dd = ps[st].d;
+            const float* t = w.t[st];
+            INTEL_TRY(gate_bwd(B, L, dd, w.stack[st].X[d->layers], w.m[st], w.dall_item + ps[st].off, D, w.dX[st], w.dm, s));
+            INTEL_TRY(linear_dw(B, dd, q, w.dm, dd, t, q, gs[st].w2, q, nullptr, s));
+            INTEL_TRY(linear_dx(B, dd, q, w.dm, dd, ps[st].w2, q, w.dt, q, s, 0, t, q));       // relu mask (t = relu(.) > 0)
+            INTEL_TRY(linear_dw(B, q, I, w.dt, q, intents, I, gs[st].w0, I, gs[st].b0, s));
+            INTEL_TRY(linear_dx(B, q, I, w.dt, q, ps[st].w0, I, d_intents_out, I, s, 1));
         }
         }
     }
-    // the self-attention stacks (IntEL.py:182-197) and what feeds them
-    if (do_item) {
-        INTEL_TRY(stack_bwd(B, L, di, d->heads, d->layers, P->item, G->item, w.item, w.dXa, w.t1, w.t2, w.dqkv, d->dropout_p,
-                            d->dropout_seed, 0, s));
-        INTEL_TRY(scatter_add_rows(R, d->d_iid, w.dXa, di, bt->i_id, G->iid_emb, nullptr, s, d->item_rows, M.iid));
-        if (d->d_im > 0)
-            INTEL_TRY(scatter_add_rows(R, d->d_im, w.dXa + d->d_iid, di, bt->i_class, G->item_emb, nullptr, s, d->class_rows, M.item));
-    }
-    if (do_score) {
-        // run on its own, this phase is the one a caller overlaps with its gradient exchange: leave the reserved SMs free
-        trunk_reserve_apply(phases == INTEL_ENS_BWD_SCORE);
-        const int st = stack_bwd(B, L, ds, d->heads, d->layers, P->score, G->score, w.score, w.dXs, w.t1, w.t2, w.dqkv, d->dropout_p,
-                                 d->dropout_seed, 1, s);
-        trunk_reserve_apply(false);
-        INTEL_TRY(st);
-        if (score_embed_bwd_ok(K, ds)) INTEL_TRY(score_embed_bwd(R, K, ds, w.dXs, ds, w.xs, G->score_w, G->score_b, s));
-        else INTEL_TRY(linear_dw(R, ds, K, w.dXs, ds, w.xs, K, G->score_w, K, G->score_b, s));
+    // the self-attention stacks (IntEL.py:182-197) and what feeds them: phase ITEM, then phase SCORE
+    const bool do_stream[2] = {do_item, do_score};
+    for (int st = 0; st < 2; ++st) {
+        if (!do_stream[st]) continue;
+        // run on its own, the score phase is the one a caller overlaps with its gradient exchange: leave the reserved SMs free
+        const bool reserve = st == 1 && phases == INTEL_ENS_BWD_SCORE;
+        if (reserve) trunk_reserve_apply(true);
+        const int r = stack_bwd(B, L, ps[st].d, d->heads, d->layers, *ps[st].stack, *gs[st].stack, w.stack[st], w.dX[st], w.t1, w.t2,
+                                w.dqkv, d->dropout_p, d->dropout_seed, st, s);
+        if (reserve) trunk_reserve_apply(false);
+        INTEL_TRY(r);
+        if (st == 0) {           // item id / class embedding rows
+            INTEL_TRY(scatter_add_rows(R, d->d_iid, w.dX[0], di, bt->i_id, G->iid_emb, nullptr, s, d->item_rows, M.iid));
+            if (d->d_im > 0)
+                INTEL_TRY(scatter_add_rows(R, d->d_im, w.dX[0] + d->d_iid, di, bt->i_class, G->item_emb, nullptr, s, d->class_rows, M.item));
+        } else {                 // score_embeddings
+            if (score_embed_bwd_ok(K, ds)) INTEL_TRY(score_embed_bwd(R, K, ds, w.dX[1], ds, w.xs, G->score_w, G->score_b, s));
+            else INTEL_TRY(linear_dw(R, ds, K, w.dX[1], ds, w.xs, K, G->score_w, K, G->score_b, s));
+        }
     }
     return INTEL_OK;
 }
@@ -745,40 +746,31 @@ int intel_intent_fwd(const intel_dims_t* d, const intel_tensors_t* P, const inte
     INTEL_REQUIRE(workspace && a.ok(), INTEL_ERR_WORKSPACE, "intent workspace too small: need %zu", a.off);
     cudaStream_t s = S(stream);
     const int64_t B = d->B, I = d->I;
-    const int dint = d->d_int, dctx = d->d_ctx, du = d->d_u, diid = d->d_iid;
-    const int d1 = dctx + dint, d2 = diid + dint, Dp = d1 + d2 + dctx + du;
-    const int off_v2 = dctx + du, off_v1 = dctx + du + d2;     // pred_layer input = [ctx | user | item-history | history]
+    const int dint = d->d_int, dctx = d->d_ctx, du = d->d_u;
+    const int Dp = dctx + dint + d->d_iid + dint + dctx + du;
+    History hs[2];
+    histories_of(d, P, nullptr, nullptr, bt, hs);
 
     INTEL_TRY(transpose(dint, I, P->intent_w, w.Wt, 0, s));
-    // session history tokens: [context embedding | intent embedding of the dense history intents]
-    INTEL_TRY(gather_rows(B * d->H1, dctx, P->ctx_emb, bt->his_context, w.e1.seq, d1, 0, s, d->ctx_rows));
-    if (bt->his_intents_idx) {
-        INTEL_TRY(sparse_rows_linear_fwd(B * d->H1, bt->nz1, dint, bt->his_intents_idx, bt->his_intents_val, w.Wt,
-                                         P->intent_b, w.e1.seq + dctx, d1, s));
-    } else {
-        INTEL_REQUIRE(bt->his_intents, INTEL_ERR_ARG, "his_intents is null");
-        INTEL_TRY(dense_rows_linear_fwd(B * d->H1, I, dint, bt->his_intents, w.Wt, P->intent_b, w.e1.seq + dctx, d1,
-                                        w.e1.nz_idx, w.e1.nz_val, w.e1.nz_cnt, NZ_CAP, s, d->H1, bt->history_len));
-    }
-    // item history tokens: [item id embedding | intent embedding of the one-hot item intents]
-    INTEL_TRY(gather_rows(B * d->H2, diid, P->iid_emb, bt->his_item_id, w.e2.seq, d2, 0, s, d->item_rows));
-    if (bt->his_item_int_idx) {
-        INTEL_TRY(sparse_rows_linear_fwd(B * d->H2, bt->nz2, dint, bt->his_item_int_idx, bt->his_item_int_val, w.Wt,
-                                         P->intent_b, w.e2.seq + diid, d2, s));
-    } else {
-        INTEL_REQUIRE(bt->his_item_int, INTEL_ERR_ARG, "his_item_int is null");
-        INTEL_TRY(dense_rows_linear_fwd(B * d->H2, I, dint, bt->his_item_int, w.Wt, P->intent_b, w.e2.seq + diid, d2,
-                                        w.e2.nz_idx, w.e2.nz_val, w.e2.nz_cnt, NZ_CAP, s, d->H2, bt->history_item_len));
+    // history tokens: [context embedding | intent embedding of the dense history intents] of the session history,
+    // [item id embedding | intent embedding of the one-hot item intents] of the item history
+    for (int i = 0; i < 2; ++i) {
+        const History& h = hs[i];
+        EncWs& e = w.e[i];
+        const int64_t R = B * e.T;
+        INTEL_TRY(gather_rows(R, h.dtok, h.table, h.ids, e.seq, e.d, 0, s, h.table_rows));
+        if (h.idx) {
+            INTEL_TRY(sparse_rows_linear_fwd(R, h.nz, dint, h.idx, h.val, w.Wt, P->intent_b, e.seq + h.dtok, e.d, s));
+        } else {
+            INTEL_REQUIRE(h.dense, INTEL_ERR_ARG, "%s is null", h.dense_name);
+            INTEL_TRY(dense_rows_linear_fwd(R, I, dint, h.dense, w.Wt, P->intent_b, e.seq + h.dtok, e.d, e.nz_idx, e.nz_val, e.nz_cnt,
+                                            NZ_CAP, s, e.T, h.lens));
+        }
     }
     if (d->encoder == INTEL_ENCODER_BERT4REC) {
-        INTEL_TRY(bert_fwd(d, P->enc, w.e1, bt->history_len, w.feat + off_v1, Dp, s));
-        INTEL_TRY(bert_fwd(d, P->item_enc, w.e2, bt->history_item_len, w.feat + off_v2, Dp, s));
+        for (int i = 0; i < 2; ++i) INTEL_TRY(bert_fwd(d, *hs[i].p, w.e[i], hs[i].lens, w.feat + hs[i].off, Dp, s));
     } else {
-        const intel_encoder_t* const pe[2] = {&P->enc, &P->item_enc};
-        EncWs* const ee[2] = {&w.e1, &w.e2};
-        const int64_t* const ll[2] = {bt->history_len, bt->history_item_len};
-        float* const oo[2] = {w.feat + off_v1, w.feat + off_v2};
-        INTEL_TRY(gru_fwd_pair(d, pe, ee, ll, oo, Dp, s));
+        INTEL_TRY(gru_fwd_pair(d, hs, w.e, w.feat, Dp, s));
     }
     INTEL_TRY(gather_rows(B, dctx, P->ctx_emb, bt->context_mh, w.feat, Dp, 0, s, d->ctx_rows));
     INTEL_TRY(gather_rows(B, du, P->uid_emb, bt->u_id, w.feat + dctx, Dp, 0, s, d->user_rows));
@@ -798,9 +790,10 @@ int intel_intent_bwd_rows(const intel_dims_t* d, const intel_tensors_t* P, const
     INTEL_REQUIRE(workspace && a.ok(), INTEL_ERR_WORKSPACE, "intent workspace too small: need %zu", a.off);
     cudaStream_t s = S(stream);
     const int64_t B = d->B, I = d->I;
-    const int dint = d->d_int, dctx = d->d_ctx, du = d->d_u, diid = d->d_iid;
-    const int d1 = dctx + dint, d2 = diid + dint, Dp = d1 + d2 + dctx + du;
-    const int off_v2 = dctx + du, off_v1 = dctx + du + d2;
+    const int dint = d->d_int, dctx = d->d_ctx, du = d->d_u;
+    const int Dp = dctx + dint + d->d_iid + dint + dctx + du;
+    History hs[2];
+    histories_of(d, P, G, &M, bt, hs);
 
     INTEL_TRY(softmax_rows_bwd(B, I, intents, d_intents, d_intents_extra, w.dlogits, s, pad4(I)));
     INTEL_TRY(linear_dw(B, I, Dp, w.dlogits, pad4(I), w.feat, Dp, G->pred_w, Dp, G->pred_b, s));
@@ -808,38 +801,35 @@ int intel_intent_bwd_rows(const intel_dims_t* d, const intel_tensors_t* P, const
     INTEL_TRY(scatter_add_rows(B, dctx, w.dfeat, Dp, bt->context_mh, G->ctx_emb, nullptr, s, d->ctx_rows, M.ctx));
     INTEL_TRY(scatter_add_rows(B, du, w.dfeat + dctx, Dp, bt->u_id, G->uid_emb, nullptr, s, d->user_rows, M.uid));
     if (d->encoder == INTEL_ENCODER_BERT4REC) {
-        INTEL_TRY(bert_bwd(d, P->enc, G->enc, w.e1, bt->history_len, w.dfeat + off_v1, Dp, w.t1, w.t2, w.dqkv, s));
-        INTEL_TRY(bert_bwd(d, P->item_enc, G->item_enc, w.e2, bt->history_item_len, w.dfeat + off_v2, Dp, w.t1, w.t2, w.dqkv, s));
+        for (int i = 0; i < 2; ++i)
+            INTEL_TRY(bert_bwd(d, *hs[i].p, *hs[i].g, w.e[i], hs[i].lens, w.dfeat + hs[i].off, Dp, w.t1, w.t2, w.dqkv, s));
     } else {
         bool have_dh = false;
-        if (gru_outproj_pair_ok(d->gru_hidden, w.e1.d, w.e2.d)) {      // d(last state) of both encoders in one launch
-            const int n[2] = {w.e1.d, w.e2.d};
-            const float* W[2] = {P->enc.w_out, P->item_enc.w_out};
-            const float* dv[2] = {w.dfeat + off_v1, w.dfeat + off_v2};
-            float* dh[2] = {w.e1.gru.dh, w.e2.gru.dh};
+        if (gru_outproj_pair_ok(d->gru_hidden, w.e[0].d, w.e[1].d)) {      // d(last state) of both encoders in one launch
+            const int n[2] = {w.e[0].d, w.e[1].d};
+            const float* W[2] = {hs[0].p->w_out, hs[1].p->w_out};
+            const float* dv[2] = {w.dfeat + hs[0].off, w.dfeat + hs[1].off};
+            float* dh[2] = {w.e[0].gru.dh, w.e[1].gru.dh};
             const int64_t ldd[2] = {Dp, Dp}, ldh[2] = {d->gru_hidden, d->gru_hidden};
             INTEL_TRY(gru_outproj_pair_dx(B, n, W, dv, ldd, dh, ldh, s));
             have_dh = true;
         }
-        INTEL_TRY(gru_bwd(d, P->enc, G->enc, w.e1, bt->history_len, w.dfeat + off_v1, Dp, s, have_dh));
-        INTEL_TRY(gru_bwd(d, P->item_enc, G->item_enc, w.e2, bt->history_item_len, w.dfeat + off_v2, Dp, s, have_dh));
+        for (int i = 0; i < 2; ++i)
+            INTEL_TRY(gru_bwd(d, *hs[i].p, *hs[i].g, w.e[i], hs[i].lens, w.dfeat + hs[i].off, Dp, s, have_dh));
     }
     INTEL_TRY(fill_zero(w.dWt, (size_t)I * dint * 4, s));
-    INTEL_TRY(scatter_add_rows(B * d->H1, dctx, w.e1.dseq, d1, bt->his_context, G->ctx_emb, nullptr, s, d->ctx_rows, M.ctx));
-    if (bt->his_intents_idx) {
-        INTEL_TRY(dense_rows_linear_bwd(B * d->H1, I, dint, nullptr, w.e1.dseq + dctx, d1, bt->his_intents_idx,
-                                        bt->his_intents_val, nullptr, bt->nz1, w.dWt, s, G->intent_b));
-    } else {
-        INTEL_TRY(dense_rows_linear_bwd(B * d->H1, I, dint, bt->his_intents, w.e1.dseq + dctx, d1, w.e1.nz_idx, w.e1.nz_val,
-                                        w.e1.nz_cnt, NZ_CAP, w.dWt, s, G->intent_b));      // + the bias gradient (column sums)
-    }
-    INTEL_TRY(scatter_add_rows(B * d->H2, diid, w.e2.dseq, d2, bt->his_item_id, G->iid_emb, nullptr, s, d->item_rows, M.iid));
-    if (bt->his_item_int_idx) {
-        INTEL_TRY(dense_rows_linear_bwd(B * d->H2, I, dint, nullptr, w.e2.dseq + diid, d2, bt->his_item_int_idx,
-                                        bt->his_item_int_val, nullptr, bt->nz2, w.dWt, s, G->intent_b));
-    } else {
-        INTEL_TRY(dense_rows_linear_bwd(B * d->H2, I, dint, bt->his_item_int, w.e2.dseq + diid, d2, w.e2.nz_idx, w.e2.nz_val,
-                                        w.e2.nz_cnt, NZ_CAP, w.dWt, s, G->intent_b));
+    for (int i = 0; i < 2; ++i) {
+        const History& h = hs[i];
+        const EncWs& e = w.e[i];
+        const int64_t R = B * e.T;
+        INTEL_TRY(scatter_add_rows(R, h.dtok, e.dseq, e.d, h.ids, h.gtable, nullptr, s, h.table_rows, h.map));
+        // the intent part, with the bias gradient (column sums)
+        if (h.idx) {
+            INTEL_TRY(dense_rows_linear_bwd(R, I, dint, nullptr, e.dseq + h.dtok, e.d, h.idx, h.val, nullptr, h.nz, w.dWt, s, G->intent_b));
+        } else {
+            INTEL_TRY(dense_rows_linear_bwd(R, I, dint, h.dense, e.dseq + h.dtok, e.d, e.nz_idx, e.nz_val, e.nz_cnt, NZ_CAP, w.dWt, s,
+                                            G->intent_b));
+        }
     }
     return transpose(I, dint, w.dWt, G->intent_w, 1, s);
 }

@@ -500,16 +500,6 @@ int gru_prep(int n, const int64_t* B, const int64_t* T, const int64_t* const* le
     LAUNCH(gru_prep_kernel, dim3((unsigned)(nb + 1), (unsigned)n), dim3(1024), 0, s, a);
     return check_launch("gru_prep");
 }
-int gru_live_rows(int64_t B, int64_t T, const int64_t* lens, int32_t* rows_t, int32_t* rows_t1, int32_t* count, cudaStream_t s) {
-    if (B <= 0) return INTEL_OK;
-    int32_t* none = nullptr;
-    return gru_prep(1, &B, &T, &lens, &rows_t, &rows_t1, &count, &none, s);
-}
-int gru_order_by_len(int64_t B, int64_t T, const int64_t* lens, int32_t* order, cudaStream_t s) {
-    if (B <= 0) return INTEL_OK;
-    int32_t* none = nullptr;
-    return gru_prep(1, &B, &T, &lens, &none, &none, &none, &order, s);
-}
 
 // Backward recurrence.  dh [B,128] holds d(loss)/d h_T on entry.  Writes dgi [B,T,384] and
 // dgh_all [B,T+1,384] (slot T untouched: the caller clears the buffer) for the weight-gradient GEMMs.

@@ -63,7 +63,6 @@ struct ValidateArgs {
     int nz1, nz2;
 };
 int batch_validate(const ValidateArgs& a, int32_t* flags, cudaStream_t s);
-// out[b, l, :] += table[idx[b]]-style broadcast helpers are not needed: per-session rows are gathered once.
 
 // Dense float64 rows X[R, I] times the intent_embeddings weight, exploiting that the rows are (nearly)
 // one-hot / few-hot: Y[r, :] = sum_i float(X[r,i]) * Wt[i, :] + bias.  Wt is the [I, d] transpose.
@@ -164,7 +163,7 @@ int gru_seq_fwd(int64_t B, int64_t T, int h, const int64_t* lens, const float* g
 bool gru_tc_supported(int h);
 int gru_tc_fwd(int64_t B, int64_t T, const int64_t* lens, const float* gi, const float* w_hh, const float* b_hh, float* h_all,
                float* gates, cudaStream_t s, bool save_gates = true, const int32_t* order = nullptr);
-// one launch for the recurrences of up to two encoders; order (nullable): sessions by decreasing length (gru_order_by_len)
+// one launch for the recurrences of up to two encoders; order (nullable): sessions by decreasing length (gru_prep)
 struct GruTcOne {
     int64_t B, T;
     const int64_t* lens;
@@ -178,28 +177,44 @@ void gru_debug_use_tcgen05(int on);
 int gru_seq_bwd(int64_t B, int64_t T, int h, const int64_t* lens, const float* w_hh, const float* h_all,
                 const float* gates, const float* dh_in, float* dgi, float* dgh_all, float* db_ih, float* db_hh, cudaStream_t s,
                 int32_t* order = nullptr);
-// order [B + 1]: order[i] = session with the i-th longest history (stable; T <= 63), order[B] = 0 (the tile counter).  With it the backward recurrence walks tiles of
-// equally long sessions and stops each tile at its own last step (the reference packs the sequences: GeneralSeq.py:64-71).
-int gru_order_by_len(int64_t B, int64_t T, const int64_t* lens, int32_t* order, cudaStream_t s);
-// the live (session, step) pairs of a padded [B, T] history as row numbers, in (b, t) order: rows_t[i] = b T + t into the
-// [B, T, .] tensors, rows_t1[i] = b (T + 1) + t into the [B, T + 1, .] ones; *count = sum of the (clamped) lengths
-int gru_live_rows(int64_t B, int64_t T, const int64_t* lens, int32_t* rows_t, int32_t* rows_t1, int32_t* count, cudaStream_t s);
 // output projections (Linear(128 -> d <= 64), no bias) of both encoders in one launch, and their input gradients
 bool gru_outproj_pair_ok(int h, int n0, int n1);
 int gru_outproj_pair_fwd(int64_t B, const int* n, const float* const* W, const float* const* h_last, const int64_t* ldh,
                          float* const* out, const int64_t* ldo, cudaStream_t s);
 int gru_outproj_pair_dx(int64_t B, const int* n, const float* const* W, const float* const* dout, const int64_t* ldd,
                         float* const* dh, const int64_t* ldh, cudaStream_t s);
-// both of the above for up to two encoders in one launch (null pointers skip a part)
+// For up to two encoders in one launch (null pointers skip a part):
+// - the live (session, step) pairs of a padded [B, T] history as row numbers, in (b, t) order: rows_t[i] = b T + t into the
+//   [B, T, .] tensors, rows_t1[i] = b (T + 1) + t into the [B, T + 1, .] ones; *count = sum of the (clamped) lengths;
+// - order [B + 1]: order[i] = session with the i-th longest history (stable; T <= 63), order[B] = 0 (the tile counter).  With
+//   it the backward recurrence walks tiles of equally long sessions and stops each tile at its own last step (the reference
+//   packs the sequences: GeneralSeq.py:64-71).
 int gru_prep(int n, const int64_t* B, const int64_t* T, const int64_t* const* lens, int32_t* const* rows_t, int32_t* const* rows_t1,
              int32_t* const* count, int32_t* const* order, cudaStream_t s);
 
 // ---- trunk.cu: fused self-attention stack (d = 32, L <= 64): all layers of a session on chip -----
-struct StackParams { const float *wq, *wk, *wv, *w1, *b1, *w2, *b2, *lnw, *lnb; };
-struct StackGrads { float *wq, *wk, *wv, *w1, *b1, *w2, *b2, *lnw, *lnb; };
-// per-layer activations the forward kernel leaves for the backward kernel: q|k|v [B*L,96], attention output,
-// FFN hidden (pre-relu), pre-LN sum [B*L,32] each, LN mean / rstd [B*L,2]
-struct StackSaved { float* const* QKV; float* const* A; float* const* U; float* const* Z; float* const* ST; };
+// The activations of one self-attention stack (IntEL.py:182-197) over R = B*L rows of width d, as the forward pass leaves
+// them for the backward pass: X[0] = input, X[l+1] = output of layer l (layers <= 8); per layer q|k|v [R,3d], attention
+// output, FFN hidden (pre-relu), pre-LN sum [R,d] each, LN mean / rstd [R,2].  The fused and the staged paths read them alike.
+struct StackWs {
+    float* X[9];
+    float* QKV[8];
+    float* A[8];
+    float* U[8];
+    float* Z[8];
+    float* st[8];
+};
+inline void stack_layout(Arena& a, int64_t R, int d, int layers, StackWs& w) {
+    w.X[0] = a.take<float>(R * d);
+    for (int l = 0; l < layers; ++l) {
+        w.QKV[l] = a.take<float>(R * 3 * d);
+        w.A[l] = a.take<float>(R * d);
+        w.U[l] = a.take<float>(R * d);
+        w.Z[l] = a.take<float>(R * d);
+        w.st[l] = a.take<float>(R * 2);
+        w.X[l + 1] = a.take<float>(R * d);
+    }
+}
 int adam_step(int count, float* const* params, const float* const* grads, float* const* exp_avg, float* const* exp_avg_sq,
               const int64_t* numel, const float* weight_decay, double lr, double beta1, double beta2, double eps, int64_t step,
               cudaStream_t s);
@@ -235,12 +250,12 @@ void trunk_reserve_apply(bool on);  // ... in the launches made while this is on
 void gemm_debug_use_umma(int on);
 bool trunk_supported(int64_t L, int d, int heads, int layers);      // mma.sync kernels, forward and backward
 bool trunk_fwd_supported(int64_t L, int heads, int layers);         // any fused forward kernel (d = 32)
-// X[0] = stack input [B*L,32]; X[l+1] receives the output of layer l
-int trunk_fwd(int64_t B, int64_t L, int heads, int layers, const StackParams& p, float* const* X, const StackSaved& sv,
-              float drop_p, uint64_t drop_seed, int stream_id, cudaStream_t s, bool save = true);
+// w.X[0] = stack input [B*L,32]; w.X[l+1] receives the output of layer l
+int trunk_fwd(int64_t B, int64_t L, int heads, int layers, const intel_selfatt_t& p, const StackWs& w, float drop_p,
+              uint64_t drop_seed, int stream_id, cudaStream_t s, bool save = true);
 // dX: d loss / d X[layers] on entry, d loss / d X[0] on return; weight gradients are accumulated into g
-int trunk_bwd(int64_t B, int64_t L, int heads, int layers, const StackParams& p, const StackGrads& g, float* const* X,
-              const StackSaved& sv, float* dX, float drop_p, uint64_t drop_seed, int stream_id, cudaStream_t s);
+int trunk_bwd(int64_t B, int64_t L, int heads, int layers, const intel_selfatt_t& p, const intel_selfatt_t& g, const StackWs& w,
+              float* dX, float drop_p, uint64_t drop_seed, int stream_id, cudaStream_t s);
 
 // ---- fuse.cu ------------------------------------------------------------------------------------
 // weights[b,l,:] = l < n_b ? w_valid[b] : w_pad[b];  ens[b,l] = sum_k weights * float(scores)

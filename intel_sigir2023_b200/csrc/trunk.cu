@@ -1055,31 +1055,31 @@ int trunk_run(const TrunkArgs& a, bool bwd, cudaStream_t s) {
     return INTEL_ERR_UNSUPPORTED;
 }
 
-static TrunkArgs trunk_args(int64_t B, int64_t L, int heads, int layers, const StackParams& p, float* const* X,
-                            const StackSaved& sv, float drop_p, uint64_t drop_seed, int stream_id) {
+static TrunkArgs trunk_args(int64_t B, int64_t L, int heads, int layers, const intel_selfatt_t& p, const StackWs& w,
+                            float drop_p, uint64_t drop_seed, int stream_id) {
     TrunkArgs a;
     memset(&a, 0, sizeof(a));
     for (int l = 0; l < 8; ++l) a.drop[l] = make_dropout(drop_p, drop_seed, stream_id, l);
     for (int l = 0; l < layers && l < 8; ++l) {
-        a.QKV[l] = sv.QKV[l]; a.A[l] = sv.A[l]; a.U[l] = sv.U[l]; a.Z[l] = sv.Z[l]; a.ST[l] = sv.ST[l];
+        a.QKV[l] = w.QKV[l]; a.A[l] = w.A[l]; a.U[l] = w.U[l]; a.Z[l] = w.Z[l]; a.ST[l] = w.st[l];
     }
     a.save = 1;
     a.B = B; a.L = (int)L; a.heads = heads; a.layers = layers;
     a.wq = p.wq; a.wk = p.wk; a.wv = p.wv; a.w1 = p.w1; a.b1 = p.b1; a.w2 = p.w2; a.b2 = p.b2; a.lnw = p.lnw; a.lnb = p.lnb;
-    for (int l = 0; l <= layers && l < 9; ++l) a.X[l] = X[l];
+    for (int l = 0; l <= layers && l < 9; ++l) a.X[l] = w.X[l];
     return a;
 }
 
-int trunk_fwd(int64_t B, int64_t L, int heads, int layers, const StackParams& p, float* const* X, const StackSaved& sv,
-              float drop_p, uint64_t drop_seed, int stream_id, cudaStream_t s, bool save) {
-    TrunkArgs a = trunk_args(B, L, heads, layers, p, X, sv, drop_p, drop_seed, stream_id);
+int trunk_fwd(int64_t B, int64_t L, int heads, int layers, const intel_selfatt_t& p, const StackWs& w, float drop_p,
+              uint64_t drop_seed, int stream_id, cudaStream_t s, bool save) {
+    TrunkArgs a = trunk_args(B, L, heads, layers, p, w, drop_p, drop_seed, stream_id);
     a.save = save ? 1 : 0;
     return trunk_run(a, false, s);
 }
 
-int trunk_bwd(int64_t B, int64_t L, int heads, int layers, const StackParams& p, const StackGrads& g, float* const* X,
-              const StackSaved& sv, float* dX, float drop_p, uint64_t drop_seed, int stream_id, cudaStream_t s) {
-    TrunkArgs a = trunk_args(B, L, heads, layers, p, X, sv, drop_p, drop_seed, stream_id);
+int trunk_bwd(int64_t B, int64_t L, int heads, int layers, const intel_selfatt_t& p, const intel_selfatt_t& g, const StackWs& w,
+              float* dX, float drop_p, uint64_t drop_seed, int stream_id, cudaStream_t s) {
+    TrunkArgs a = trunk_args(B, L, heads, layers, p, w, drop_p, drop_seed, stream_id);
     a.dX = dX;
     a.gwq = g.wq; a.gwk = g.wk; a.gwv = g.wv; a.gw1 = g.w1; a.gb1 = g.b1; a.gw2 = g.w2; a.gb2 = g.b2; a.glnw = g.lnw; a.glnb = g.lnb;
     return trunk_run(a, true, s);
