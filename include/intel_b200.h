@@ -48,6 +48,9 @@ typedef struct {
     int32_t heads, layers;   /* num_heads, num_layers of the two self-attention stacks */
     int32_t cross_attention; /* 1: CrossAtt pooling (default); 0: intent MLP gate */
     int32_t encoder;         /* INTEL_ENCODER_* */
+    /* gru_hidden: GRU4Rec hidden size; must be 128, the size the reference fixes (GRU4RecEncoder(hidden_size=128),
+     * IntEL.py:105-106): other values make every call with encoder = INTEL_ENCODER_GRU4REC fail with
+     * INTEL_ERR_UNSUPPORTED (and *_workspace_bytes return 0).  BERT4Rec ignores it. */
     int32_t gru_hidden, bert_layers, bert_heads, history_max;
     /* nn.Dropout of the two self-attention stacks (IntEL.py:187,196), training mode only: p = 0 disables it.
      * Masks come from a counter-based hash of (seed, stream, layer, row, channel); pass a new seed per step. */

@@ -23,6 +23,8 @@ int check_dims(const intel_dims_t* d) {
                   "stream widths not divisible by num_heads");
     INTEL_REQUIRE(d->encoder == INTEL_ENCODER_BERT4REC || d->encoder == INTEL_ENCODER_GRU4REC, INTEL_ERR_ARG,
                   "Invalid sequence encoder.");
+    INTEL_REQUIRE(d->encoder != INTEL_ENCODER_GRU4REC || d->gru_hidden == 128, INTEL_ERR_UNSUPPORTED,
+                  "GRU4Rec needs gru_hidden = 128, the reference's GRU4RecEncoder(hidden_size=128)");
     INTEL_REQUIRE(d->bert_layers <= INTEL_MAX_BERT_LAYERS, INTEL_ERR_UNSUPPORTED, "too many BERT4Rec layers");
     return INTEL_OK;
 }
@@ -176,8 +178,9 @@ struct BertWs {
     float *QKV[INTEL_MAX_BERT_LAYERS], *Z1[INTEL_MAX_BERT_LAYERS], *st1[INTEL_MAX_BERT_LAYERS], *C[INTEL_MAX_BERT_LAYERS],
         *F[INTEL_MAX_BERT_LAYERS], *Z2[INTEL_MAX_BERT_LAYERS], *st2[INTEL_MAX_BERT_LAYERS];
 };
-// packed: the int32 live-row lists can address every row of [B, T + 1, .]; sorted: set and read inside one call only
-struct GruWs { float *gi, *h_all, *gates, *gh, *dh, *dgi, *dgh_all; int32_t *order, *rows_t, *rows_t1, *nlive; bool packed, sorted; };
+// rows_t / rows_t1 / nlive: the live-row lists (gru_prep), null when int32 cannot address every row of [B, T + 1, .];
+// order: the length-sorted sessions, null when T > 63
+struct GruWs { float *gi, *h_all, *gates, *dh, *dgi, *dgh_all; int32_t *order, *rows_t, *rows_t1, *nlive; };
 struct EncWs {
     int64_t T; int d;
     float* seq;          // [B*T, d] token embeddings (BERT: positions added in place)
@@ -240,15 +243,14 @@ void enc_layout(const intel_dims_t* d, Arena& a, EncWs& e, int64_t T, int dd) {
         e.gru.gi = a.take<float>(R * 3 * h);
         e.gru.h_all = a.take<float>(B * (T + 1) * h);
         e.gru.gates = a.take<float>(R * 4 * h);
-        e.gru.gh = a.take<float>(B * 3 * h);
         e.gru.dh = a.take<float>(B * h);
         e.gru.dgi = a.take<float>(R * 3 * h);
         e.gru.dgh_all = a.take<float>(B * (T + 1) * 3 * h);
-        e.gru.order = a.take<int32_t>(B + 1);
-        e.gru.rows_t = a.take<int32_t>(R);
-        e.gru.rows_t1 = a.take<int32_t>(R);
-        e.gru.nlive = a.take<int32_t>(4);
-        e.gru.packed = B * (T + 1) < (1LL << 31);
+        e.gru.order = T <= 63 ? a.take<int32_t>(B + 1) : nullptr;
+        const bool packed = B * (T + 1) < (1LL << 31);
+        e.gru.rows_t = packed ? a.take<int32_t>(R) : nullptr;
+        e.gru.rows_t1 = packed ? a.take<int32_t>(R) : nullptr;
+        e.gru.nlive = packed ? a.take<int32_t>(4) : nullptr;
     }
 }
 
@@ -339,21 +341,12 @@ int bert_bwd(const intel_dims_t* d, const intel_encoder_t& p, intel_encoder_t& g
 int gru_fwd_pair(const intel_dims_t* d, const History (&hs)[2], EncWs (&e)[2], float* feat, int64_t ld_out, cudaStream_t s) {
     const int64_t B = d->B;
     const int h = d->gru_hidden;
-    bool fused = h == 128 && gru_tc_supported(h);
-    {   // live rows and length order of both encoders: one launch
-        int64_t Bs[2], Ts[2];
-        const int64_t* ls[2];
-        int32_t *rt[2], *rt1[2], *cn[2], *od[2];
-        for (int i = 0; i < 2; ++i) {
-            GruWs& w = e[i].gru;
-            Bs[i] = B; Ts[i] = e[i].T; ls[i] = hs[i].lens;
-            rt[i] = w.packed ? w.rows_t : nullptr; rt1[i] = w.packed ? w.rows_t1 : nullptr; cn[i] = w.packed ? w.nlive : nullptr;
-            w.sorted = Ts[i] <= 63;
-            od[i] = w.sorted ? w.order : nullptr;
-            fused = fused && w.sorted;
-        }
-        INTEL_TRY(gru_prep(2, Bs, Ts, ls, rt, rt1, cn, od, s));
+    GruPrepOne prep[2];         // live rows and length order of both encoders: one launch
+    for (int i = 0; i < 2; ++i) {
+        const GruWs& w = e[i].gru;
+        prep[i] = GruPrepOne{B, (int)e[i].T, hs[i].lens, w.rows_t, w.rows_t1, w.nlive, w.order};
     }
+    INTEL_TRY(gru_prep(2, prep, s));
     for (int i = 0; i < 2; ++i) {
         const int64_t T = e[i].T, R = B * T;
         const int dd = e[i].d;
@@ -362,40 +355,27 @@ int gru_fwd_pair(const intel_dims_t* d, const History (&hs)[2], EncWs (&e)[2], f
         // session's length; the reference packs the sequences: GeneralSeq.py:64-71).  gi rows of padding slots stay
         // unwritten: nobody reads them.
         INTEL_TRY(linear(R, 3 * h, dd, e[i].seq, dd, hs[i].p->w_ih, dd, hs[i].p->b_ih, w.gi, 3 * h, s, false, false, nullptr, 0,
-                         w.packed ? w.rows_t : nullptr, w.packed ? w.nlive : nullptr));
-        if (h == 128) {
-            // the fused kernels write h_all[:, 1..T] of every session themselves: only the initial state h_0 needs clearing
-            // (2 MB instead of a 44 MB memset per encoder and step)
-            cudaError_t ce = cudaMemset2DAsync(w.h_all, (size_t)(T + 1) * h * 4, 0, (size_t)h * 4, (size_t)B, s);
-            INTEL_REQUIRE(ce == cudaSuccess, INTEL_ERR_CUDA, "cudaMemset2DAsync: %s", cudaGetErrorString(ce));
-        } else {
-            INTEL_TRY(fill_zero(w.h_all, (size_t)B * (T + 1) * h * 4, s));
-        }
+                         w.rows_t, w.nlive));
+        // the recurrence kernels write h_all[:, 1..T] of every session themselves: only the initial state h_0 needs clearing
+        cudaError_t ce = cudaMemset2DAsync(w.h_all, (size_t)(T + 1) * h * 4, 0, (size_t)h * 4, (size_t)B, s);
+        INTEL_REQUIRE(ce == cudaSuccess, INTEL_ERR_CUDA, "cudaMemset2DAsync: %s", cudaGetErrorString(ce));
     }
-    if (fused) {
+    if (gru_tc_supported()) {
         GruTcPair pr;
         pr.n = 2;
+        pr.save_gates = d->inference == 0;
         for (int i = 0; i < 2; ++i) {
             GruWs& w = e[i].gru;
             pr.e[i] = GruTcOne{B, e[i].T, hs[i].lens, w.gi, hs[i].p->w_hh, hs[i].p->b_hh, w.h_all, w.gates, w.order};
         }
-        INTEL_TRY(gru_tc_fwd_pair(pr, s, d->inference == 0));
+        INTEL_TRY(gru_tc_fwd_pair(pr, s));
     } else {
         for (int i = 0; i < 2; ++i) {
-            const int64_t T = e[i].T;
-            const intel_encoder_t& p = *hs[i].p;
             GruWs& w = e[i].gru;
-            if (h == 128) {
-                INTEL_TRY(gru_seq_fwd(B, T, h, hs[i].lens, w.gi, p.w_hh, p.b_hh, w.h_all, w.gates, s, d->inference == 0));
-            } else {
-                for (int64_t t = 0; t < T; ++t) {
-                    INTEL_TRY(linear(B, 3 * h, h, w.h_all + t * h, (T + 1) * h, p.w_hh, h, p.b_hh, w.gh, 3 * h, s));
-                    INTEL_TRY(gru_step_fwd(B, T, h, (int)t, hs[i].lens, w.gi, w.gh, w.h_all, w.gates, s));
-                }
-            }
+            INTEL_TRY(gru_seq_fwd(B, e[i].T, hs[i].lens, w.gi, hs[i].p->w_hh, hs[i].p->b_hh, w.h_all, w.gates, s));
         }
     }
-    if (gru_outproj_pair_ok(h, e[0].d, e[1].d)) {          // both output projections in one launch
+    if (gru_outproj_pair_ok(e[0].d, e[1].d)) {          // both output projections in one launch
         const int n[2] = {e[0].d, e[1].d};
         const float* W[2] = {hs[0].p->w_out, hs[1].p->w_out};
         const float* hl[2] = {e[0].gru.h_all + e[0].T * h, e[1].gru.h_all + e[1].T * h};
@@ -411,40 +391,28 @@ int gru_fwd_pair(const intel_dims_t* d, const History (&hs)[2], EncWs (&e)[2], f
     return INTEL_OK;
 }
 
-// have_dh: d(last state) was already formed (for both encoders at once, gru_outproj_pair_dx)
+// w.dh holds d(last state) on entry (intel_intent_bwd_rows forms it for both encoders)
 int gru_bwd(const intel_dims_t* d, const intel_encoder_t& p, intel_encoder_t& g, EncWs& e, const int64_t* lens,
-            const float* dout, int64_t ld, cudaStream_t s, bool have_dh = false) {
+            const float* dout, int64_t ld, cudaStream_t s) {
     const int64_t B = d->B, T = e.T, R = B * T;
     const int dd = e.d, h = d->gru_hidden;
     GruWs& w = e.gru;
     INTEL_TRY(linear_dw(B, dd, h, dout, ld, w.h_all + T * h, (T + 1) * h, g.w_out, h, nullptr, s));
-    if (!have_dh) INTEL_TRY(linear_dx(B, dd, h, dout, ld, p.w_out, h, w.dh, h, s));
-    if (h == 128) {
-        // the fused kernel writes dgh_all[:, 0..T-1] of every session (zeros behind a session's end): only slot T, which
-        // pairs with the final state in the weight-gradient product below, needs clearing (6 MB instead of 132 MB)
-        cudaError_t ce = cudaMemset2DAsync(w.dgh_all + T * 3 * h, (size_t)(T + 1) * 3 * h * 4, 0, (size_t)3 * h * 4, (size_t)B, s);
-        INTEL_REQUIRE(ce == cudaSuccess, INTEL_ERR_CUDA, "cudaMemset2DAsync: %s", cudaGetErrorString(ce));
-        // the fused kernel also sums the bias gradients (column sums of dgi / dgh) on its way
-        int32_t* order = nullptr;
-        if (T <= 63) {               // tiles of equally long sessions: a tile stops at its own last step
-            INTEL_TRY(fill_zero(w.order + B, sizeof(int32_t), s));     // the order is the forward call's; reset the tile counter
-            order = w.order;
-        }
-        INTEL_TRY(gru_seq_bwd(B, T, h, lens, p.w_hh, w.h_all, w.gates, w.dh, w.dgi, w.dgh_all, g.b_ih, g.b_hh, s, order));
-    } else {
-        INTEL_TRY(fill_zero(w.dgh_all, (size_t)B * (T + 1) * 3 * h * 4, s));
-        for (int64_t t = T - 1; t >= 0; --t) {
-            INTEL_TRY(gru_step_bwd(B, T, h, (int)t, lens, w.h_all, w.gates, w.dh, w.dgi, w.dgh_all, s));
-            INTEL_TRY(linear_dx(B, 3 * h, h, w.dgh_all + t * 3 * h, (T + 1) * 3 * h, p.w_hh, h, w.dh, h, s, 1));
-        }
-    }
+    // the recurrence kernel writes dgh_all[:, 0..T-1] of every session (zeros behind a session's end): only slot T, which
+    // pairs with the final state in the weight-gradient product below, needs clearing (6 MB instead of 132 MB)
+    cudaError_t ce = cudaMemset2DAsync(w.dgh_all + T * 3 * h, (size_t)(T + 1) * 3 * h * 4, 0, (size_t)3 * h * 4, (size_t)B, s);
+    INTEL_REQUIRE(ce == cudaSuccess, INTEL_ERR_CUDA, "cudaMemset2DAsync: %s", cudaGetErrorString(ce));
+    // with the length order, tiles of equally long sessions stop at their own last step; the order is the forward call's,
+    // its tile counter is reset here
+    if (w.order) INTEL_TRY(fill_zero(w.order + B, sizeof(int32_t), s));
+    // the kernel also sums the bias gradients (column sums of dgi / dgh) on its way
+    INTEL_TRY(gru_seq_bwd(B, T, lens, p.w_hh, w.h_all, w.gates, w.dh, w.dgi, w.dgh_all, g.b_ih, g.b_hh, s, w.order));
     // gradient rows of padding slots are zero: the three products below contract / map the live rows only (the list was
     // built by the forward call); d(seq) of the padding slots is cleared for the scatters that read every row
-    const int32_t *rt = w.packed ? w.rows_t : nullptr, *rt1 = w.packed ? w.rows_t1 : nullptr, *nl = w.packed ? w.nlive : nullptr;
-    INTEL_TRY(linear_dw(B * (T + 1), 3 * h, h, w.dgh_all, 3 * h, w.h_all, h, g.w_hh, h, h == 128 ? nullptr : g.b_hh, s, false, rt1, nl));
-    INTEL_TRY(linear_dw(R, 3 * h, dd, w.dgi, 3 * h, e.seq, dd, g.w_ih, dd, h == 128 ? nullptr : g.b_ih, s, false, rt, nl));
-    if (w.packed) INTEL_TRY(fill_zero(e.dseq, (size_t)R * dd * 4, s));
-    return linear_dx(R, 3 * h, dd, w.dgi, 3 * h, p.w_ih, dd, e.dseq, dd, s, 0, nullptr, 0, rt, nl);
+    INTEL_TRY(linear_dw(B * (T + 1), 3 * h, h, w.dgh_all, 3 * h, w.h_all, h, g.w_hh, h, nullptr, s, false, w.rows_t1, w.nlive));
+    INTEL_TRY(linear_dw(R, 3 * h, dd, w.dgi, 3 * h, e.seq, dd, g.w_ih, dd, nullptr, s, false, w.rows_t, w.nlive));
+    if (w.rows_t) INTEL_TRY(fill_zero(e.dseq, (size_t)R * dd * 4, s));
+    return linear_dx(R, 3 * h, dd, w.dgi, 3 * h, p.w_ih, dd, e.dseq, dd, s, 0, nullptr, 0, w.rows_t, w.nlive);
 }
 
 }  // namespace
@@ -470,7 +438,9 @@ int intel_debug_use_rows_gemm(int on) {
 int intel_debug_gru_prep(int64_t B, int64_t T, const int64_t* lens, int32_t* order, int32_t* rows_t, int32_t* rows_t1,
                          int32_t* count, intel_stream_t stream) {
     INTEL_REQUIRE(lens && order && rows_t && rows_t1 && count, INTEL_ERR_ARG, "gru_prep: null argument");
-    return gru_prep(1, &B, &T, &lens, &rows_t, &rows_t1, &count, &order, S(stream));
+    INTEL_REQUIRE(T >= 0 && T < (1LL << 31), INTEL_ERR_ARG, "gru_prep: bad history length %lld", (long long)T);
+    const GruPrepOne one{B, (int)T, lens, rows_t, rows_t1, count, order};
+    return gru_prep(1, &one, S(stream));
 }
 
 int intel_debug_use_fused_bert(int on) {
@@ -804,18 +774,20 @@ int intel_intent_bwd_rows(const intel_dims_t* d, const intel_tensors_t* P, const
         for (int i = 0; i < 2; ++i)
             INTEL_TRY(bert_bwd(d, *hs[i].p, *hs[i].g, w.e[i], hs[i].lens, w.dfeat + hs[i].off, Dp, w.t1, w.t2, w.dqkv, s));
     } else {
-        bool have_dh = false;
-        if (gru_outproj_pair_ok(d->gru_hidden, w.e[0].d, w.e[1].d)) {      // d(last state) of both encoders in one launch
+        const int h = d->gru_hidden;
+        if (gru_outproj_pair_ok(w.e[0].d, w.e[1].d)) {      // d(last state) of both encoders in one launch
             const int n[2] = {w.e[0].d, w.e[1].d};
             const float* W[2] = {hs[0].p->w_out, hs[1].p->w_out};
             const float* dv[2] = {w.dfeat + hs[0].off, w.dfeat + hs[1].off};
             float* dh[2] = {w.e[0].gru.dh, w.e[1].gru.dh};
-            const int64_t ldd[2] = {Dp, Dp}, ldh[2] = {d->gru_hidden, d->gru_hidden};
+            const int64_t ldd[2] = {Dp, Dp}, ldh[2] = {h, h};
             INTEL_TRY(gru_outproj_pair_dx(B, n, W, dv, ldd, dh, ldh, s));
-            have_dh = true;
+        } else {
+            for (int i = 0; i < 2; ++i)
+                INTEL_TRY(linear_dx(B, w.e[i].d, h, w.dfeat + hs[i].off, Dp, hs[i].p->w_out, h, w.e[i].gru.dh, h, s));
         }
         for (int i = 0; i < 2; ++i)
-            INTEL_TRY(gru_bwd(d, *hs[i].p, *hs[i].g, w.e[i], hs[i].lens, w.dfeat + hs[i].off, Dp, s, have_dh));
+            INTEL_TRY(gru_bwd(d, *hs[i].p, *hs[i].g, w.e[i], hs[i].lens, w.dfeat + hs[i].off, Dp, s));
     }
     INTEL_TRY(fill_zero(w.dWt, (size_t)I * dint * 4, s));
     for (int i = 0; i < 2; ++i) {

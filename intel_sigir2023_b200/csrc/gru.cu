@@ -1,91 +1,12 @@
-// GRU4RecEncoder recurrence (GeneralSeq.py:58-78 -> torch.nn.GRU, gate order r,z,n), one masked time
-// step per launch; the two projections per step (W_ih x, W_hh h) are GEMMs issued by the caller.
+// GRU4RecEncoder recurrence (GeneralSeq.py:58-78 -> torch.nn.GRU, gate order r,z,n) for hidden size 128, the size the
+// reference hard-codes (GRU4RecEncoder(hidden_size=128), IntEL.py:105-106).  The input projections W_ih x are one GEMM over
+// all live history rows, issued by the caller; the recurrence itself is ONE kernel per direction: a CTA owns a tile of
+// sessions for all T steps, W_hh (384x128 fp32 = 192 KB) stays in shared memory for the whole kernel, the hidden
+// state of the tile lives in shared memory / registers, gh = W_hh h is formed by 3xTF32 tensor-core MMAs and the gate math
+// runs in the MMA epilogue on the accumulator fragments (each warp owns 16 hidden units: its r, z and n columns of a unit
+// land in the same lane).  HBM traffic is just gi in, h_all / gates out.  gru_tc.cu has the tcgen05 forward kernel.
 // Packed-sequence semantics: a session stops updating once t >= len, so h_all[:, T] is its last state.
 #include "kernels.h"
-
-namespace intel {
-
-__global__ void __launch_bounds__(256) gru_step_fwd_kernel(int64_t B, int64_t T, int h, int t,
-                                                           const int64_t* __restrict__ lens,
-                                                           const float* __restrict__ gi, const float* __restrict__ gh,
-                                                           float* h_all, float* __restrict__ gates) {
-    const int64_t total = B * h;
-    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t b = e / h;
-        const int c = (int)(e % h);
-        const float hp = h_all[(b * (T + 1) + t) * h + c];
-        float hn = hp;
-        if (t < lens[b]) {
-            const float* gib = gi + (b * T + t) * 3 * h;
-            const float* ghb = gh + b * 3 * h;
-            const float r = sigmoidf_(gib[c] + ghb[c]);
-            const float z = sigmoidf_(gib[h + c] + ghb[h + c]);
-            const float ghn = ghb[2 * h + c];
-            const float n = tanhf(gib[2 * h + c] + r * ghn);
-            hn = (1.f - z) * n + z * hp;
-            float* gt = gates + (b * T + t) * 4 * h;
-            gt[c] = r; gt[h + c] = z; gt[2 * h + c] = n; gt[3 * h + c] = ghn;
-        }
-        h_all[(b * (T + 1) + t + 1) * h + c] = hn;
-    }
-}
-
-int gru_step_fwd(int64_t B, int64_t T, int h, int t, const int64_t* lens, const float* gi, const float* gh,
-                 float* h_all, float* gates, cudaStream_t s) {
-    if (B <= 0) return INTEL_OK;
-    unsigned grid = stream_grid(ceil_div(B * h, 256), 8);
-    LAUNCH(gru_step_fwd_kernel, dim3(grid), dim3(256), 0, s, B, T, h, t, lens, gi, gh, h_all, gates);
-    return check_launch("gru_step_fwd");
-}
-
-__global__ void __launch_bounds__(256) gru_step_bwd_kernel(int64_t B, int64_t T, int h, int t,
-                                                           const int64_t* __restrict__ lens,
-                                                           const float* __restrict__ h_all,
-                                                           const float* __restrict__ gates, float* dh,
-                                                           float* __restrict__ dgi, float* __restrict__ dgh_all) {
-    const int64_t total = B * h;
-    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t b = e / h;
-        const int c = (int)(e % h);
-        float* di = dgi + (b * T + t) * 3 * h;
-        float* dg = dgh_all + (b * (T + 1) + t) * 3 * h;   // [B, T+1, 3h]: row layout of h_all (slot T stays 0)
-        if (t < lens[b]) {
-            const float* gt = gates + (b * T + t) * 4 * h;
-            const float r = gt[c], z = gt[h + c], n = gt[2 * h + c], ghn = gt[3 * h + c];
-            const float hp = h_all[(b * (T + 1) + t) * h + c];
-            const float g = dh[e];
-            const float dn = g * (1.f - z) * (1.f - n * n);
-            const float dz = g * (hp - n) * z * (1.f - z);
-            const float dr = dn * ghn * r * (1.f - r);
-            di[c] = dr; di[h + c] = dz; di[2 * h + c] = dn;
-            dg[c] = dr; dg[h + c] = dz; dg[2 * h + c] = dn * r;
-            dh[e] = g * z;
-        } else {
-            di[c] = 0.f; di[h + c] = 0.f; di[2 * h + c] = 0.f;
-            dg[c] = 0.f; dg[h + c] = 0.f; dg[2 * h + c] = 0.f;
-        }
-    }
-}
-
-int gru_step_bwd(int64_t B, int64_t T, int h, int t, const int64_t* lens, const float* h_all, const float* gates,
-                 float* dh, float* dgi, float* dgh_all, cudaStream_t s) {
-    if (B <= 0) return INTEL_OK;
-    unsigned grid = stream_grid(ceil_div(B * h, 256), 8);
-    LAUNCH(gru_step_bwd_kernel, dim3(grid), dim3(256), 0, s, B, T, h, t, lens, h_all, gates, dh, dgi, dgh_all);
-    return check_launch("gru_step_bwd");
-}
-
-}  // namespace intel
-
-// =================================================================================================
-// Fused recurrence for hidden size 128 (the reference hard-codes GRU4RecEncoder(hidden_size=128),
-// IntEL.py:105-106).  The per-step formulation above needs 2 launches per time step and runs its
-// [B,128]x[128,384] products on a few hundred CTAs; here ONE persistent CTA owns a tile of sessions for all
-// T steps: W_hh (384x128 fp32 = 192 KB) stays in shared memory for the whole kernel, the hidden state of the
-// tile lives in shared memory / registers, gh = W_hh h is formed by 3xTF32 tensor-core MMAs and the gate
-// math runs in the MMA epilogue on the accumulator fragments (each warp owns 16 hidden units: its r, z and n
-// columns of a unit land in the same lane).  HBM traffic is just gi in, h_all / gates out.
-// =================================================================================================
 #include "mma.cuh"
 
 namespace intel {
@@ -238,11 +159,9 @@ __global__ void __launch_bounds__(256, 1) gru_seq_fwd_kernel(int64_t B, int64_t 
 }
 
 // h_all[:, 0] must be zero (the caller clears it); h_all [B, T+1, 128], gates [B, T, 512]
-int gru_seq_fwd(int64_t B, int64_t T, int h, const int64_t* lens, const float* gi, const float* w_hh,
-                const float* b_hh, float* h_all, float* gates, cudaStream_t s, bool save_gates) {
+int gru_seq_fwd(int64_t B, int64_t T, const int64_t* lens, const float* gi, const float* w_hh, const float* b_hh, float* h_all,
+                float* gates, cudaStream_t s) {
     if (B <= 0 || T <= 0) return INTEL_OK;
-    INTEL_REQUIRE(h == GH, INTEL_ERR_UNSUPPORTED, "fused GRU needs hidden size 128");
-    if (gru_tc_supported(h)) return gru_tc_fwd(B, T, lens, gi, w_hh, b_hh, h_all, gates, s, save_gates);
     const size_t smem = (size_t)(3 * GH * GW + GF_SB * GW) * 4;
     ensure_smem(gru_seq_fwd_kernel, smem);
     LAUNCH(gru_seq_fwd_kernel, dim3((unsigned)ceil_div(B, GF_SB)), dim3(256), smem, s, B, T, lens, gi, w_hh, b_hh, h_all,
@@ -340,7 +259,7 @@ __global__ void __launch_bounds__(OP_WARPS * 32) gru_outproj_dx_kernel(OutProjAr
     }
 }
 
-bool gru_outproj_pair_ok(int h, int n0, int n1) { return h == OP_H && n0 >= 1 && n0 <= OP_NMAX && n1 >= 1 && n1 <= OP_NMAX; }
+bool gru_outproj_pair_ok(int n0, int n1) { return n0 >= 1 && n0 <= OP_NMAX && n1 >= 1 && n1 <= OP_NMAX; }
 
 static int gru_outproj_launch(bool dx, int64_t B, const int* n, const float* const* W, const float* const* x, const int64_t* ldx,
                               float* const* y, const int64_t* ldy, cudaStream_t s) {
@@ -470,11 +389,11 @@ __device__ void gru_order_body(int64_t B, int T, const int64_t* __restrict__ len
 }
 // One launch prepares both encoders: blocks [0, nb) of row y list the live rows of encoder y, block nb sorts its sessions.
 struct GruPrepArgs {
-    struct One { int64_t B; int T; const int64_t* lens; int32_t *rows_t, *rows_t1, *count, *order; } e[2];
+    GruPrepOne e[2];
     int n;
 };
 __global__ void __launch_bounds__(1024) gru_prep_kernel(GruPrepArgs a) {
-    const GruPrepArgs::One& E = a.e[blockIdx.y];
+    const GruPrepOne& E = a.e[blockIdx.y];
     const int nb = (int)((E.B + 1023) / 1024);
     if ((int)blockIdx.x < nb) {
         if (E.rows_t) gru_live_rows_body((int)blockIdx.x, nb, E.B, E.T, E.lens, E.rows_t, E.rows_t1, E.count);
@@ -482,18 +401,16 @@ __global__ void __launch_bounds__(1024) gru_prep_kernel(GruPrepArgs a) {
         if (E.order) gru_order_body(E.B, E.T, E.lens, E.order);
     }
 }
-int gru_prep(int n, const int64_t* B, const int64_t* T, const int64_t* const* lens, int32_t* const* rows_t, int32_t* const* rows_t1,
-             int32_t* const* count, int32_t* const* order, cudaStream_t s) {
+int gru_prep(int n, const GruPrepOne* e, cudaStream_t s) {
     GruPrepArgs a;
     memset(&a, 0, sizeof(a));
     a.n = n;
     int64_t nb = 0;
     for (int i = 0; i < n; ++i) {
-        INTEL_REQUIRE(B[i] * (T[i] + 1) < (1LL << 31) || !rows_t[i], INTEL_ERR_UNSUPPORTED, "gru_prep: more than 2^31 history rows");
-        INTEL_REQUIRE(!order[i] || (T[i] >= 1 && T[i] <= 63), INTEL_ERR_UNSUPPORTED, "gru_prep: sorting needs T in [1, 63]");
-        a.e[i].B = B[i]; a.e[i].T = (int)T[i]; a.e[i].lens = lens[i];
-        a.e[i].rows_t = rows_t[i]; a.e[i].rows_t1 = rows_t1[i]; a.e[i].count = count[i]; a.e[i].order = order[i];
-        const int64_t x = ceil_div(B[i], 1024);
+        INTEL_REQUIRE(e[i].B * (e[i].T + 1) < (1LL << 31) || !e[i].rows_t, INTEL_ERR_UNSUPPORTED, "gru_prep: more than 2^31 history rows");
+        INTEL_REQUIRE(!e[i].order || (e[i].T >= 1 && e[i].T <= 63), INTEL_ERR_UNSUPPORTED, "gru_prep: sorting needs T in [1, 63]");
+        a.e[i] = e[i];
+        const int64_t x = ceil_div(e[i].B, 1024);
         nb = x > nb ? x : nb;
     }
     if (n <= 0 || nb <= 0) return INTEL_OK;
@@ -708,11 +625,9 @@ __global__ void __launch_bounds__(256, 1) gru_seq_bwd_kernel(int64_t B, int64_t 
     }
 }
 
-int gru_seq_bwd(int64_t B, int64_t T, int h, const int64_t* lens, const float* w_hh, const float* h_all,
-                const float* gates, const float* dh_in, float* dgi, float* dgh_all, float* db_ih, float* db_hh, cudaStream_t s,
-                int32_t* order) {
+int gru_seq_bwd(int64_t B, int64_t T, const int64_t* lens, const float* w_hh, const float* h_all, const float* gates,
+                const float* dh_in, float* dgi, float* dgh_all, float* db_ih, float* db_hh, cudaStream_t s, int32_t* order) {
     if (B <= 0 || T <= 0) return INTEL_OK;
-    INTEL_REQUIRE(h == GH, INTEL_ERR_UNSUPPORTED, "fused GRU needs hidden size 128");
     const size_t smem = (size_t)(3 * GH * GW + GB_SB * GD) * 4;
     ensure_smem(gru_seq_bwd_kernel, smem);
     // persistent: one CTA per SM (W_hh fills its shared memory), tiles drawn from the counter behind `order` (order[B])

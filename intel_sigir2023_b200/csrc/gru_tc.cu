@@ -68,25 +68,13 @@ __device__ __forceinline__ bool elect_lane() {
 // hands out the clusters in blockIdx order = by decreasing length of both encoders interleaved, a cluster stops at the last
 // live step of its tile, and the SMs it frees take the next cluster: the two recurrences, each a chain of T dependent steps,
 // overlap instead of running back to back.
-struct GruTcEnc {
-    int64_t B, T;
-    const int64_t* lens;
-    const float *gi, *w_hh, *b_hh;
-    float *h_all, *gates;
-    const int32_t* order;        // nullable: sessions by decreasing length
-};
-struct GruTcArgs {
-    GruTcEnc e[2];
-    int nenc, save_gates;
-};
-
-__global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(128, 1) gru_tc_fwd_kernel(GruTcArgs args) {
+__global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(128, 1) gru_tc_fwd_kernel(GruTcPair args) {
     extern __shared__ __align__(1024) uint8_t gsm[];
     const int t = threadIdx.x, warp = t >> 5;
     const uint32_t c = cluster_rank();                              // hidden-unit slice of this CTA
     const int cq = (int)(blockIdx.x >> 2);
-    const GruTcEnc& E = args.e[cq % args.nenc];
-    const int64_t tile = cq / args.nenc;
+    const GruTcOne& E = args.e[cq % args.n];
+    const int64_t tile = cq / args.n;
     const int64_t B = E.B, T = E.T;
     if (tile * 128 >= B) return;                                     // the whole cluster leaves (no barrier was touched)
     const int64_t* __restrict__ lens = E.lens;
@@ -266,35 +254,22 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(128, 1) gru_tc_fwd_k
 
 static int g_use_gru_tc = 1;
 void gru_debug_use_tcgen05(int on) { g_use_gru_tc = on ? 1 : 0; }
-bool gru_tc_supported(int h) { return g_use_gru_tc && h == GT_H; }
+bool gru_tc_supported() { return g_use_gru_tc; }
 
-int gru_tc_fwd(int64_t B, int64_t T, const int64_t* lens, const float* gi, const float* w_hh, const float* b_hh, float* h_all,
-               float* gates, cudaStream_t s, bool save_gates, const int32_t* order) {
-    GruTcPair p;
-    p.n = 1;
-    p.e[0] = GruTcOne{B, T, lens, gi, w_hh, b_hh, h_all, gates, order};
-    return gru_tc_fwd_pair(p, s, save_gates);
-}
-
-int gru_tc_fwd_pair(const GruTcPair& p, cudaStream_t s, bool save_gates) {
-    GruTcArgs a;
-    memset(&a, 0, sizeof(a));
-    a.nenc = p.n;
-    a.save_gates = save_gates ? 1 : 0;
+int gru_tc_fwd_pair(const GruTcPair& p, cudaStream_t s) {
     int64_t tiles = 0;
     double bytes = 0.0, flops = 0.0;
     for (int i = 0; i < p.n; ++i) {
         const GruTcOne& o = p.e[i];
-        a.e[i] = GruTcEnc{o.B, o.T, o.lens, o.gi, o.w_hh, o.b_hh, o.h_all, o.gates, o.order};
         const int64_t ti = ceil_div(o.B, 128);
         tiles = ti > tiles ? ti : tiles;
-        bytes += (double)o.B * o.T * (3 + (save_gates ? 4 : 0) + 1) * GT_H * 4.0;
+        bytes += (double)o.B * o.T * (3 + (p.save_gates ? 4 : 0) + 1) * GT_H * 4.0;
         flops += 2.0 * o.B * o.T * 3 * GT_H * GT_H;
     }
     if (tiles <= 0) return INTEL_OK;
     const unsigned grid = (unsigned)(4 * tiles * p.n);
     ensure_smem(gru_tc_fwd_kernel, (size_t)GT_BYTES);
-    LAUNCH(gru_tc_fwd_kernel, dim3(grid), dim3(128), (size_t)GT_BYTES, s, a);
+    LAUNCH(gru_tc_fwd_kernel, dim3(grid), dim3(128), (size_t)GT_BYTES, s, p);
     return check_launch("gru_seq_fwd", bytes, flops);
 }
 
@@ -302,11 +277,7 @@ int gru_tc_fwd_pair(const GruTcPair& p, cudaStream_t s, bool save_gates) {
 #else
 namespace intel {
 void gru_debug_use_tcgen05(int) {}
-bool gru_tc_supported(int) { return false; }
-int gru_tc_fwd(int64_t, int64_t, const int64_t*, const float*, const float*, const float*, float*, float*, cudaStream_t, bool,
-               const int32_t*) {
-    return INTEL_ERR_UNSUPPORTED;
-}
-int gru_tc_fwd_pair(const GruTcPair&, cudaStream_t, bool) { return INTEL_ERR_UNSUPPORTED; }
+bool gru_tc_supported() { return false; }
+int gru_tc_fwd_pair(const GruTcPair&, cudaStream_t) { return INTEL_ERR_UNSUPPORTED; }
 }  // namespace intel
 #endif

@@ -144,26 +144,14 @@ int bert_fused_fwd(int64_t B, int64_t T, int heads, int layers, const int64_t* l
                    float* const* Z2, float* const* st2, bool save, float* out, int64_t ld_out, cudaStream_t s);
 
 // ---- gru.cu -------------------------------------------------------------------------------------
-// One masked GRU step for all sessions (gate order r,z,n; torch.nn.GRU equations).
-// gi [B, T, 3h] (input projections incl. b_ih), gh [B, 3h] (= W_hh h_{t-1} + b_hh),
-// h_all [B, T+1, h] with h_all[:,0] = 0;  saves gates [B, T, 4h] = (r, z, n, gh_n).
-int gru_step_fwd(int64_t B, int64_t T, int h, int t, const int64_t* lens, const float* gi, const float* gh,
-                 float* h_all, float* gates, cudaStream_t s);
-// dh [B,h] is updated in place to d h_{t-1} (without the W_hh term, which the caller adds by GEMM);
-// dgi[:, t] and dgh_t [B, 3h] are written.
-int gru_step_bwd(int64_t B, int64_t T, int h, int t, const int64_t* lens, const float* h_all,
-                 const float* gates, float* dh, float* dgi, float* dgh_all, cudaStream_t s);
-
-// Fused recurrence for hidden size 128: one persistent CTA per tile of sessions walks all T steps with W_hh
-// resident in shared memory (see gru.cu).  h_all [B,T+1,h] (slot 0 pre-zeroed), gates [B,T,4h],
-// dgi [B,T,3h], dgh_all [B,T+1,3h] (pre-zeroed), dh_in [B,h] = d loss / d h_T.
-int gru_seq_fwd(int64_t B, int64_t T, int h, const int64_t* lens, const float* gi, const float* w_hh,
-                const float* b_hh, float* h_all, float* gates, cudaStream_t s, bool save_gates = true);
-// tcgen05 forward recurrence (gru_tc.cu): clusters of four CTAs, W_hh slices resident as UMMA B operands; same outputs
-bool gru_tc_supported(int h);
-int gru_tc_fwd(int64_t B, int64_t T, const int64_t* lens, const float* gi, const float* w_hh, const float* b_hh, float* h_all,
-               float* gates, cudaStream_t s, bool save_gates = true, const int32_t* order = nullptr);
-// one launch for the recurrences of up to two encoders; order (nullable): sessions by decreasing length (gru_prep)
+// GRU recurrence for hidden size 128 (gate order r,z,n; torch.nn.GRU equations): one CTA per tile of sessions walks all T
+// steps with W_hh resident in shared memory (see gru.cu).  gi [B,T,3h] (input projections incl. b_ih), h_all [B,T+1,h]
+// (slot 0 pre-zeroed), gates [B,T,4h] = (r, z, n, gh_n), dgi [B,T,3h], dgh_all [B,T+1,3h] (slot T pre-zeroed),
+// dh_in [B,h] = d loss / d h_T.
+int gru_seq_fwd(int64_t B, int64_t T, const int64_t* lens, const float* gi, const float* w_hh, const float* b_hh, float* h_all,
+                float* gates, cudaStream_t s);
+// tcgen05 forward recurrence (gru_tc.cu) of up to two encoders in one launch: clusters of four CTAs, W_hh slices resident as
+// UMMA B operands; same outputs.  order (nullable): sessions by decreasing length (gru_prep)
 struct GruTcOne {
     int64_t B, T;
     const int64_t* lens;
@@ -171,26 +159,26 @@ struct GruTcOne {
     float *h_all, *gates;
     const int32_t* order;
 };
-struct GruTcPair { GruTcOne e[2]; int n; };
-int gru_tc_fwd_pair(const GruTcPair& p, cudaStream_t s, bool save_gates);
+struct GruTcPair { GruTcOne e[2]; int n, save_gates; };    // save_gates = 0: forward only, gates are not written
+bool gru_tc_supported();
+int gru_tc_fwd_pair(const GruTcPair& p, cudaStream_t s);
 void gru_debug_use_tcgen05(int on);
-int gru_seq_bwd(int64_t B, int64_t T, int h, const int64_t* lens, const float* w_hh, const float* h_all,
-                const float* gates, const float* dh_in, float* dgi, float* dgh_all, float* db_ih, float* db_hh, cudaStream_t s,
-                int32_t* order = nullptr);
+int gru_seq_bwd(int64_t B, int64_t T, const int64_t* lens, const float* w_hh, const float* h_all, const float* gates,
+                const float* dh_in, float* dgi, float* dgh_all, float* db_ih, float* db_hh, cudaStream_t s, int32_t* order);
 // output projections (Linear(128 -> d <= 64), no bias) of both encoders in one launch, and their input gradients
-bool gru_outproj_pair_ok(int h, int n0, int n1);
+bool gru_outproj_pair_ok(int n0, int n1);
 int gru_outproj_pair_fwd(int64_t B, const int* n, const float* const* W, const float* const* h_last, const int64_t* ldh,
                          float* const* out, const int64_t* ldo, cudaStream_t s);
 int gru_outproj_pair_dx(int64_t B, const int* n, const float* const* W, const float* const* dout, const int64_t* ldd,
                         float* const* dh, const int64_t* ldh, cudaStream_t s);
-// For up to two encoders in one launch (null pointers skip a part):
+// For up to two encoders in one launch, one entry each (null pointers skip a part):
 // - the live (session, step) pairs of a padded [B, T] history as row numbers, in (b, t) order: rows_t[i] = b T + t into the
 //   [B, T, .] tensors, rows_t1[i] = b (T + 1) + t into the [B, T + 1, .] ones; *count = sum of the (clamped) lengths;
 // - order [B + 1]: order[i] = session with the i-th longest history (stable; T <= 63), order[B] = 0 (the tile counter).  With
 //   it the backward recurrence walks tiles of equally long sessions and stops each tile at its own last step (the reference
 //   packs the sequences: GeneralSeq.py:64-71).
-int gru_prep(int n, const int64_t* B, const int64_t* T, const int64_t* const* lens, int32_t* const* rows_t, int32_t* const* rows_t1,
-             int32_t* const* count, int32_t* const* order, cudaStream_t s);
+struct GruPrepOne { int64_t B; int T; const int64_t* lens; int32_t *rows_t, *rows_t1, *count, *order; };
+int gru_prep(int n, const GruPrepOne* e, cudaStream_t s);
 
 // ---- trunk.cu: fused self-attention stack (d = 32, L <= 64): all layers of a session on chip -----
 // The activations of one self-attention stack (IntEL.py:182-197) over R = B*L rows of width d, as the forward pass leaves

@@ -502,14 +502,15 @@ def check_tc_stack(device, cases=((10, 30, 2, 2), (7, 50, 2, 2), (5, 64, 1, 1), 
             assert_grad_close(a[2][k].cpu().numpy(), g.cpu().numpy(), gmax, f"{k} {(B, L, heads, layers)}", rtol=2e-4, afrac=3e-6)
 
 
-def check_gru_tc(device, B=300, L=9):
+def check_gru_tc(device, B=300, L=9, history_max=11):
     """the tcgen05 cluster kernel of the GRU recurrence (gru_tc.cu) against the mma.sync kernel (gru.cu): several session
-    tiles with a ragged tail, history lengths 1..H, outputs and every parameter gradient"""
+    tiles with a ragged tail, history lengths 1..H, outputs and every parameter gradient.  Histories longer than 63 slots
+    run without the length-sorted order, forward and backward."""
     from intel_sigir2023_b200 import _lib, synthetic
     from intel_sigir2023_b200.config import IntelConfig
-    corpus = synthetic.CorpusSpec(n_item=200, n_class=9, n_user=30, n_ctx=19, model_num=3, intent_num=40, history_max=11)
+    corpus = synthetic.CorpusSpec(n_item=200, n_class=9, n_user=30, n_ctx=19, model_num=3, intent_num=40, history_max=history_max)
     cfg = IntelConfig(item_rows=corpus.item_rows, class_rows=corpus.n_class, user_rows=corpus.user_rows, ctx_rows=corpus.n_ctx,
-                      intent_num=corpus.intent_num, model_num=3, history_max=11, encoder="GRU4Rec", num_heads=2, num_layers=1,
+                      intent_num=corpus.intent_num, model_num=3, history_max=history_max, encoder="GRU4Rec", num_heads=2, num_layers=1,
                       context_emb_size=32, intent_emb_size=32)
     batch = synthetic.make_batch(corpus, synthetic.BatchSpec(batch_size=B, max_len=L, min_len=2), seed=21)
     batch = {k: (v.to(device) if torch.is_tensor(v) else v) for k, v in batch.items()}

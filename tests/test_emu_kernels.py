@@ -157,6 +157,26 @@ def test_gru_prep_index_kernels():
     P.check_gru_prep("cpu")
 
 
+def test_gru_hidden_other_than_128_is_rejected():
+    """GRU4Rec runs at hidden size 128 only, the size the reference fixes (IntEL.py:105-106); BERT4Rec ignores gru_hidden"""
+    import ctypes
+    from intel_sigir2023_b200 import _lib
+    from intel_sigir2023_b200.config import IntelConfig
+    lib = _lib.load()
+    for encoder in ("GRU4Rec", "BERT4Rec"):
+        cfg = IntelConfig(item_rows=50, class_rows=7, user_rows=5, ctx_rows=5, intent_num=12, encoder=encoder, gru_hidden=64)
+        dims = _lib.make_dims(cfg, B=4, L=6, H1=3, H2=3)
+        nbytes = lib.intel_intent_workspace_bytes(ctypes.byref(dims))
+        status = lib.intel_intent_fwd(ctypes.byref(dims), None, None, None, None, 0, None)
+        if encoder == "GRU4Rec":
+            assert nbytes == 0
+            assert status == 4, status                  # INTEL_ERR_UNSUPPORTED
+            assert b"gru_hidden = 128" in lib.intel_last_error()
+        else:
+            assert nbytes > 0
+            assert status == 1, status                  # INTEL_ERR_ARG: the dims pass, the null tensors do not
+
+
 def test_bert_fused_vs_staged():
     P.check_bert_fused_vs_staged("cpu", names=("default_bert",))
 

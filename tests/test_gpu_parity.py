@@ -143,5 +143,9 @@ def test_tcgen05_gru_matches_mma_sync_gru():
     P.check_gru_tc(DEV)
 
 
+def test_tcgen05_gru_matches_mma_sync_gru_long_histories():
+    P.check_gru_tc(DEV, history_max=70)
+
+
 def test_dropout():
     P.check_dropout(DEV)
