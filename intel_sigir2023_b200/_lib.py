@@ -171,8 +171,6 @@ def load(path: Optional[str] = None) -> C.CDLL:
         raise RuntimeError("libintel_b200 ABI version mismatch")
     if os.environ.get("INTEL_STACK_SESSIONS"):       # tuning knob for the fused stack kernels (1..4 sessions per CTA)
         lib.intel_debug_stack_sessions_per_cta(int(os.environ["INTEL_STACK_SESSIONS"]))
-    if os.environ.get("INTEL_TCGEN05_GEMM"):
-        lib.intel_debug_use_tcgen05_gemm(int(os.environ["INTEL_TCGEN05_GEMM"]))
     _lib = lib
     return lib
 

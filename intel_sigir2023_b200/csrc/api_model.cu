@@ -425,13 +425,12 @@ int intel_debug_use_fused_stack(int on) {
 }
 
 int intel_debug_use_tcgen05_gemm(int on) {
-    gemm_debug_use_umma(on);
+    gemm_debug_use_tcgen05(on);
     return INTEL_OK;
 }
 
 int intel_debug_use_rows_gemm(int on) {
-    gemm_debug_use_rows_tc(on);
-    gemm_debug_use_wgrad_tc(on);
+    gemm_debug_use_rows_gemm(on);
     return INTEL_OK;
 }
 

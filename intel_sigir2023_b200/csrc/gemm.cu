@@ -7,7 +7,7 @@
 // All shapes here have a tiny inner dimension (32..384, 1071 at most) or a tiny output, so tiles are
 // 128 x {32,64} x 32 with register-staged prefetch of the next k-tile; operands may be stored k-major or
 // row-major (the three nn.Linear passes), selected at compile time.
-#include <stdlib.h>
+#include <stdarg.h>
 
 #include "kernels.h"
 #include "mma.cuh"
@@ -26,16 +26,14 @@ struct GemmDev {
     int64_t kchunk;
 };
 
-static const int BK = 32;
-static int g_use_umma = 1;
-void gemm_debug_use_umma(int on) { g_use_umma = on ? 1 : 0; }
+static const int BK = 32;     // k depth of a gemm_tc_kernel stage
 
 // Global -> register staging of one operand tile.  TR = operand stored [K][rows] (rows contiguous),
 // otherwise [rows][K] (k contiguous).  Two modes: 16-byte chunks when the operand is 16-byte aligned with a
 // leading dimension that is a multiple of 4, otherwise element-wise with consecutive lanes on consecutive
 // addresses (I = 1071 makes every operand with that leading dimension misaligned; a per-thread 4-float
-// fallback there cost 4x the transactions).
-template <int ROWS, int NT, bool TR>
+// fallback there cost 4x the transactions).  BK: k depth of the tile.
+template <int ROWS, int NT, bool TR, int BK>
 struct TileLoader {
     static constexpr int CH = ROWS * BK / 4;                 // float4 chunks per tile
     static constexpr int NV = (CH + NT - 1) / NT;
@@ -180,8 +178,8 @@ template <int BM, int BN, int WM, int WN, bool AT, bool BT>
 __global__ void __launch_bounds__(WM * WN * 32) gemm_tc_kernel(GemmDev g) {
     constexpr int NT = WM * WN * 32;
     constexpr int TM = BM / WM / 16, TN = BN / WN / 8;
-    using LA = TileLoader<BM, NT, AT>;
-    using LB = TileLoader<BN, NT, BT>;
+    using LA = TileLoader<BM, NT, AT, BK>;
+    using LB = TileLoader<BN, NT, BT, BK>;
     constexpr int SA = LA::LD, SB = LB::LD;
     __shared__ __align__(16) float sA[AT ? BK * SA : BM * SA];
     __shared__ __align__(16) float sB[BT ? BK * SB : BN * SB];
@@ -290,14 +288,21 @@ __global__ void __launch_bounds__(WM * WN * 32) gemm_tc_kernel(GemmDev g) {
         }
 }
 
-// Weight-gradient shape: small output tile (32x32 per CTA), very long inner dimension.  The eight warps
-// of a CTA take different k-slices of each staged tile (split-K inside the CTA), partial tiles are summed
-// through shared memory, one atomicAdd per output element and CTA.  A stored [K][M], B stored [K][N].
-static const int WG_WARPS = 8, WG_BK = 16 * WG_WARPS;
-__global__ void __launch_bounds__(WG_WARPS * 32) gemm_wgrad_kernel(GemmDev g) {
-    constexpr int LD = 32 + 8;
-    __shared__ __align__(16) float sA[WG_BK * LD];
-    __shared__ __align__(16) float sB[WG_BK * LD];
+// Split-warp 32 x 32 kernel for products whose output fills too few 128-row tiles while the inner dimension is long:
+// tall outputs with few columns (the intent-side projections [B x 1071] x [1071 -> 32]: a 128 x 32 tiling leaves 32-64 CTAs
+// walking 34 k-tiles one after the other; A [M][K], B [N][K] or, BT, [K][N]) and weight gradients with a small output
+// (AT = BT = true, split-K over blockIdx.z, atomicAdd epilogue).  The eight warps of a CTA take 16 k each of every staged
+// 128-deep slab; their partial tiles are summed through shared memory.
+static const int SW_BK = 128;
+template <bool AT, bool BT>
+__global__ void __launch_bounds__(256) gemm_warpsplit_kernel(GemmDev g) {
+    using LA = TileLoader<32, 256, AT, SW_BK>;
+    using LB = TileLoader<32, 256, BT, SW_BK>;
+    constexpr int SA = LA::LD, SB = LB::LD;
+    constexpr int NA = AT ? SW_BK * SA : 32 * SA, NB = BT ? SW_BK * SB : 32 * SB;
+    __shared__ __align__(16) float sm[NA + NB > 8 * 1024 ? NA + NB : 8 * 1024];     // A slab | B slab, then the 8 partial tiles
+    float* sA = sm;
+    float* sB = sm + NA;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int gq = lane >> 2, tq = lane & 3;
     const int64_t m0 = (int64_t)blockIdx.x * 32, n0 = (int64_t)blockIdx.y * 32;
@@ -311,69 +316,20 @@ __global__ void __launch_bounds__(WG_WARPS * 32) gemm_wgrad_kernel(GemmDev g) {
 #pragma unroll
             for (int c = 0; c < 4; ++c) acc[i][j][c] = 0.f;
 
-    // register staging of the next [WG_BK][32] tile of each operand: 16-byte chunks when aligned, else
-    // element-wise with consecutive lanes on consecutive addresses (see TileLoader)
-    float pa[16], pb[16];
-    auto fetch_one = [&](const float* __restrict__ P, int64_t ld, int64_t c0, int64_t cmax, int vec, int relu, int64_t k0,
-                         float (&dst)[16]) {
-        if (vec) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const int e = tid + i * (WG_WARPS * 32);
-                const int kk = e >> 3, r4 = (e & 7) * 4;
-                const int64_t gk = k0 + kk;
-                float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (gk < kend) {
-                    const float* p = P + gk * ld + c0 + r4;
-                    if (c0 + r4 + 3 < cmax) x = *reinterpret_cast<const float4*>(p);
-                    else {
-                        if (c0 + r4 < cmax) x.x = p[0];
-                        if (c0 + r4 + 1 < cmax) x.y = p[1];
-                        if (c0 + r4 + 2 < cmax) x.z = p[2];
-                    }
-                }
-                dst[4 * i] = x.x; dst[4 * i + 1] = x.y; dst[4 * i + 2] = x.z; dst[4 * i + 3] = x.w;
-            }
-        } else {
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-                const int e = tid + i * (WG_WARPS * 32);
-                const int kk = e >> 5, r = e & 31;
-                const int64_t gk = k0 + kk;
-                dst[i] = (gk < kend && c0 + r < cmax) ? P[gk * ld + c0 + r] : 0.f;
-            }
-        }
-        if (relu) {
-#pragma unroll
-            for (int i = 0; i < 16; ++i) dst[i] = fmaxf(dst[i], 0.f);
-        }
-    };
-    auto stash = [&](float* sdst, int vec, const float (&src)[16]) {
-        if (vec) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const int e = tid + i * (WG_WARPS * 32);
-                *reinterpret_cast<float4*>(sdst + (e >> 3) * LD + (e & 7) * 4) =
-                    make_float4(src[4 * i], src[4 * i + 1], src[4 * i + 2], src[4 * i + 3]);
-            }
-        } else {
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-                const int e = tid + i * (WG_WARPS * 32);
-                sdst[(e >> 5) * LD + (e & 31)] = src[i];
-            }
-        }
-    };
-    auto fetch = [&](int64_t k0) {
-        fetch_one(g.A, g.lda, m0, g.M, g.vec_a, g.relu_a, k0, pa);
-        fetch_one(g.B, g.ldb, n0, g.N, g.vec_b, g.relu_b, k0, pb);
-    };
-    if (kbeg < kend) fetch(kbeg);
-    for (int64_t k0 = kbeg; k0 < kend; k0 += WG_BK) {
-        stash(sA, g.vec_a, pa);
-        stash(sB, g.vec_b, pb);
+    LA la;
+    LB lb;
+    if (kbeg < kend) {
+        la.load(g.A, g.lda, m0, g.M, kbeg, kend, g.vec_a, g.relu_a, tid);
+        lb.load(g.B, g.ldb, n0, g.N, kbeg, kend, g.vec_b, g.relu_b, tid);
+    }
+    for (int64_t k0 = kbeg; k0 < kend; k0 += SW_BK) {
+        la.store(sA, g.vec_a, tid);
+        lb.store(sB, g.vec_b, tid);
         __syncthreads();
-        if (k0 + WG_BK < kend) fetch(k0 + WG_BK);     // next tile in flight while this one is consumed
+        if (k0 + SW_BK < kend) {     // next slab in flight while this one is consumed
+            la.load(g.A, g.lda, m0, g.M, k0 + SW_BK, kend, g.vec_a, g.relu_a, tid);
+            lb.load(g.B, g.ldb, n0, g.N, k0 + SW_BK, kend, g.vec_b, g.relu_b, tid);
+        }
         float part[2][4][4];     // per-slab partial sums, folded into acc with a rounded add (see gemm_tc_kernel)
 #pragma unroll
         for (int i = 0; i < 2; ++i)
@@ -388,207 +344,16 @@ __global__ void __launch_bounds__(WG_WARPS * 32) gemm_wgrad_kernel(GemmDev g) {
 #pragma unroll
             for (int i = 0; i < 2; ++i) {
                 const int r = i * 16 + gq;
-                af[i][0] = sA[(kb + tq) * LD + r];
-                af[i][1] = sA[(kb + tq) * LD + r + 8];
-                af[i][2] = sA[(kb + tq + 4) * LD + r];
-                af[i][3] = sA[(kb + tq + 4) * LD + r + 8];
+                af[i][0] = tile_at<AT, SA>(sA, r, kb + tq);
+                af[i][1] = tile_at<AT, SA>(sA, r + 8, kb + tq);
+                af[i][2] = tile_at<AT, SA>(sA, r, kb + tq + 4);
+                af[i][3] = tile_at<AT, SA>(sA, r + 8, kb + tq + 4);
             }
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
                 const int c = j * 8 + gq;
-                bf[j][0] = sB[(kb + tq) * LD + c];
-                bf[j][1] = sB[(kb + tq + 4) * LD + c];
-            }
-#pragma unroll
-            for (int i = 0; i < 2; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) mma_3xtf32(part[i][j], af[i], bf[j]);
-        }
-#pragma unroll
-        for (int i = 0; i < 2; ++i)
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-#pragma unroll
-                for (int c = 0; c < 4; ++c) acc[i][j][c] += part[i][j][c];
-        __syncthreads();
-    }
-    // cross-warp reduction through shared memory (8 partial 32x32 tiles fit in the staging buffers)
-    float* red = (warp < 4) ? sA + warp * 1024 : sB + (warp - 4) * 1024;
-#pragma unroll
-    for (int i = 0; i < 2; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const int r = i * 16 + gq, c = j * 8 + 2 * tq;
-            red[r * 32 + c] = acc[i][j][0];
-            red[r * 32 + c + 1] = acc[i][j][1];
-            red[(r + 8) * 32 + c] = acc[i][j][2];
-            red[(r + 8) * 32 + c + 1] = acc[i][j][3];
-        }
-    __syncthreads();
-    const bool first = (blockIdx.z == 0);
-    for (int e = tid; e < 1024; e += WG_WARPS * 32) {
-        float v = 0.f;
-#pragma unroll
-        for (int w = 0; w < 4; ++w) v += sA[w * 1024 + e] + sB[w * 1024 + e];
-        gemm_store(g, m0 + (e >> 5), n0 + (e & 31), v, first);
-    }
-}
-
-// Tall output with few columns and a LONG inner dimension (the intent-side projections:
-// [B x 1071] x [1071 -> 32]): a 128 x 32 tiling leaves 32-64 CTAs walking 34 k-tiles one after the other.  Here a
-// CTA owns 32 rows x 32 columns and its eight warps split every staged 128-wide k slab between them; the eight
-// partial tiles are reduced through shared memory.  A is [M][K] (k contiguous); B is [N][K] or, BT, [K][N].
-static const int SK_BK = 128, SK_LD = SK_BK + 4, SK_LDT = 32 + 8;
-
-// [32 rows][128 k] slab of a k-contiguous operand -> 16 registers per thread (and back to shared memory)
-__device__ __forceinline__ void sk_load_kmajor(const float* __restrict__ P, int64_t ld, int64_t r0, int64_t rmax, int64_t k0,
-                                               int64_t kend, int vec, int relu, int tid, float (&dst)[16]) {
-    if (vec) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const int e = tid + i * 256;
-            const int rr = e >> 5, k4 = (e & 31) * 4;
-            float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (r0 + rr < rmax) {
-                const float* p = P + (r0 + rr) * ld + k0 + k4;
-                if (k0 + k4 + 3 < kend) x = *reinterpret_cast<const float4*>(p);
-                else {
-                    if (k0 + k4 < kend) x.x = p[0];
-                    if (k0 + k4 + 1 < kend) x.y = p[1];
-                    if (k0 + k4 + 2 < kend) x.z = p[2];
-                }
-            }
-            dst[4 * i] = x.x; dst[4 * i + 1] = x.y; dst[4 * i + 2] = x.z; dst[4 * i + 3] = x.w;
-        }
-    } else {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            const int e = tid + i * 256;
-            const int rr = e >> 7, k = e & 127;
-            dst[i] = (r0 + rr < rmax && k0 + k < kend) ? P[(r0 + rr) * ld + k0 + k] : 0.f;
-        }
-    }
-    if (relu) {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) dst[i] = fmaxf(dst[i], 0.f);
-    }
-}
-__device__ __forceinline__ void sk_stash_kmajor(float* s, int vec, int tid, const float (&src)[16]) {
-    if (vec) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const int e = tid + i * 256;
-            *reinterpret_cast<float4*>(s + (e >> 5) * SK_LD + (e & 31) * 4) = make_float4(src[4 * i], src[4 * i + 1], src[4 * i + 2], src[4 * i + 3]);
-        }
-    } else {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            const int e = tid + i * 256;
-            s[(e >> 7) * SK_LD + (e & 127)] = src[i];
-        }
-    }
-}
-// [128 k][32 cols] slab of a column-contiguous operand
-__device__ __forceinline__ void sk_load_cmajor(const float* __restrict__ P, int64_t ld, int64_t c0, int64_t cmax, int64_t k0,
-                                               int64_t kend, int vec, int relu, int tid, float (&dst)[16]) {
-    if (vec) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const int e = tid + i * 256;
-            const int kk = e >> 3, r4 = (e & 7) * 4;
-            float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (k0 + kk < kend) {
-                const float* p = P + (k0 + kk) * ld + c0 + r4;
-                if (c0 + r4 + 3 < cmax) x = *reinterpret_cast<const float4*>(p);
-                else {
-                    if (c0 + r4 < cmax) x.x = p[0];
-                    if (c0 + r4 + 1 < cmax) x.y = p[1];
-                    if (c0 + r4 + 2 < cmax) x.z = p[2];
-                }
-            }
-            dst[4 * i] = x.x; dst[4 * i + 1] = x.y; dst[4 * i + 2] = x.z; dst[4 * i + 3] = x.w;
-        }
-    } else {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            const int e = tid + i * 256;
-            const int kk = e >> 5, r = e & 31;
-            dst[i] = (k0 + kk < kend && c0 + r < cmax) ? P[(k0 + kk) * ld + c0 + r] : 0.f;
-        }
-    }
-    if (relu) {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) dst[i] = fmaxf(dst[i], 0.f);
-    }
-}
-__device__ __forceinline__ void sk_stash_cmajor(float* s, int vec, int tid, const float (&src)[16]) {
-    if (vec) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const int e = tid + i * 256;
-            *reinterpret_cast<float4*>(s + (e >> 3) * SK_LDT + (e & 7) * 4) = make_float4(src[4 * i], src[4 * i + 1], src[4 * i + 2], src[4 * i + 3]);
-        }
-    } else {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            const int e = tid + i * 256;
-            s[(e >> 5) * SK_LDT + (e & 31)] = src[i];
-        }
-    }
-}
-
-template <bool BT>
-__global__ void __launch_bounds__(256) gemm_skinny_kernel(GemmDev g) {
-    __shared__ __align__(16) float sm[32 * SK_LD + SK_BK * SK_LDT];     // A slab | B slab; reused for the reduction (>= 8192)
-    float* sA = sm;
-    float* sB = sm + 32 * SK_LD;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int gq = lane >> 2, tq = lane & 3;
-    const int64_t m0 = (int64_t)blockIdx.x * 32, n0 = (int64_t)blockIdx.y * 32;
-    float acc[2][4][4];
-#pragma unroll
-    for (int i = 0; i < 2; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-#pragma unroll
-            for (int c = 0; c < 4; ++c) acc[i][j][c] = 0.f;
-    float pa[16], pb[16];
-    auto fetch = [&](int64_t k0) {
-        sk_load_kmajor(g.A, g.lda, m0, g.M, k0, g.K, g.vec_a, g.relu_a, tid, pa);
-        if (BT) sk_load_cmajor(g.B, g.ldb, n0, g.N, k0, g.K, g.vec_b, g.relu_b, tid, pb);
-        else sk_load_kmajor(g.B, g.ldb, n0, g.N, k0, g.K, g.vec_b, g.relu_b, tid, pb);
-    };
-    fetch(0);
-    for (int64_t k0 = 0; k0 < g.K; k0 += SK_BK) {
-        sk_stash_kmajor(sA, g.vec_a, tid, pa);
-        if (BT) sk_stash_cmajor(sB, g.vec_b, tid, pb);
-        else sk_stash_kmajor(sB, g.vec_b, tid, pb);
-        __syncthreads();
-        if (k0 + SK_BK < g.K) fetch(k0 + SK_BK);
-        float part[2][4][4];     // per-slab partial sums, folded into acc with a rounded add (see gemm_tc_kernel)
-#pragma unroll
-        for (int i = 0; i < 2; ++i)
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-#pragma unroll
-                for (int c = 0; c < 4; ++c) part[i][j][c] = 0.f;
-#pragma unroll
-        for (int ks = 0; ks < 2; ++ks) {
-            const int kb = warp * 16 + ks * 8;
-            float af[2][4], bf[4][2];
-#pragma unroll
-            for (int i = 0; i < 2; ++i) {
-                const int r = i * 16 + gq;
-                af[i][0] = sA[r * SK_LD + kb + tq];
-                af[i][1] = sA[(r + 8) * SK_LD + kb + tq];
-                af[i][2] = sA[r * SK_LD + kb + tq + 4];
-                af[i][3] = sA[(r + 8) * SK_LD + kb + tq + 4];
-            }
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const int c = j * 8 + gq;
-                bf[j][0] = BT ? sB[(kb + tq) * SK_LDT + c] : sB[c * SK_LD + kb + tq];
-                bf[j][1] = BT ? sB[(kb + tq + 4) * SK_LDT + c] : sB[c * SK_LD + kb + tq + 4];
+                bf[j][0] = tile_at<BT, SB>(sB, c, kb + tq);
+                bf[j][1] = tile_at<BT, SB>(sB, c, kb + tq + 4);
             }
 #pragma unroll
             for (int i = 0; i < 2; ++i)
@@ -615,11 +380,12 @@ __global__ void __launch_bounds__(256) gemm_skinny_kernel(GemmDev g) {
             red[(r + 8) * 32 + c + 1] = acc[i][j][3];
         }
     __syncthreads();
+    const bool first = (blockIdx.z == 0);
     for (int e = tid; e < 1024; e += 256) {
         float v = 0.f;
 #pragma unroll
         for (int w = 0; w < 8; ++w) v += sm[w * 1024 + e];
-        gemm_store(g, m0 + (e >> 5), n0 + (e & 31), v, true);
+        gemm_store(g, m0 + (e >> 5), n0 + (e & 31), v, first);
     }
 }
 
@@ -716,21 +482,156 @@ __global__ void __launch_bounds__(256) gemm_stream32_kernel(GemmDev g) {
     }
 }
 
-template <int BM, int BN, int WM, int WN>
-static void launch_tc(const GemmDev& d, bool at, bool bt, cudaStream_t s) {
-    dim3 grid((unsigned)ceil_div(d.M, BM), (unsigned)ceil_div(d.N, BN), (unsigned)d.splits);
-    dim3 block(WM * WN * 32);
-    if (!at && !bt) { auto k = gemm_tc_kernel<BM, BN, WM, WN, false, false>; LAUNCH(k, grid, block, 0, s, d); }
-    else if (!at && bt) { auto k = gemm_tc_kernel<BM, BN, WM, WN, false, true>; LAUNCH(k, grid, block, 0, s, d); }
-    else { auto k = gemm_tc_kernel<BM, BN, WM, WN, true, true>; LAUNCH(k, grid, block, 0, s, d); }
-}
+// How gemm() computes one product.  gemm_plan() makes every choice; the launch below follows it.
+struct GemmPlan {
+    enum Kernel { UMMA, WARPSPLIT, STREAM32, TC } kernel;
+    bool prezero;              // C is cleared first and the split partial products are added with atomics
+    int splits;                // CTAs along the inner dimension (blockIdx.z), kchunk deep each
+    int64_t kchunk;
+    int cfg;                   // mma.sync kernels: 0: 128x64  1: 128x32  2: 64x64  3: 64x32  (TC tiles)  4: 32x32 weight gradient
+    int bn, nraw, vec_c4;      // UMMA: N tile, raw fp32 stages, 16-byte aligned rows of C / add / mask / bias
+    bool multi;                // UMMA: the k range spans several accumulation chunks
+    size_t smem;               // UMMA: dynamic shared memory
+};
+
+static int g_tcgen05 = 1, g_rows_gemm = 1;
+void gemm_debug_use_tcgen05(int on) { g_tcgen05 = on ? 1 : 0; }
+void gemm_debug_use_rows_gemm(int on) { g_rows_gemm = on ? 1 : 0; }
 
 static inline bool vec_ok(const float* p, int64_t ld) { return (((uintptr_t)p) % 16 == 0) && (ld % 4 == 0); }
+
+// splits of the inner dimension: enough CTAs for `waves` waves of the SMs, no split shallower than 4 granules; kchunk is a
+// multiple of the granule
+static void split_k(GemmPlan& p, int64_t K, int64_t tiles, int waves, int granule, bool can_split) {
+    int64_t n = 1;
+    if (can_split) {
+        const int64_t want = ceil_div(waves * kNumSMs, tiles), maxs = ceil_div(K, 4 * granule);
+        n = want < maxs ? want : maxs;
+        if (n < 1) n = 1;
+    }
+    p.splits = (int)n;
+    p.kchunk = ceil_div(ceil_div(K, n), granule) * granule;
+    if (p.kchunk <= 0) p.kchunk = granule;
+}
+
+static GemmPlan gemm_plan(const Gemm& g) {
+    GemmPlan p{};
+    const bool wgrad = g.pass == GemmPass::WGRAD;
+    auto ctas = [&](int bm, int bn) { return ceil_div(g.M, bm) * ceil_div(g.N, bn); };
+    // plain outputs with a long inner dimension and too few tiles to fill the GPU are split like the weight gradients: the
+    // output is cleared first and the partial products are accumulated with atomics
+    p.prezero = g.accumulate == 0 && !g.relu_out && !g.mask && g.K >= 512 && g.N > 64 && ctas(128, 64) < kNumSMs;
+    const bool can_split = wgrad || p.prezero;
+    // tall outputs with few columns and a long inner dimension fill too few 128-row tiles: the warp-split kernel
+    const bool skinny = !wgrad && !p.prezero && g.N <= 64 && g.K >= 256 && ctas(128, 32) < 2 * kNumSMs;
+#ifndef INTEL_EMU
+    // large products: tcgen05 kernel (gemm_umma.cuh), 128 x bn tiles, TMEM accumulators
+    if (g_tcgen05 && !skinny && g.M >= 128 && g.N >= 16 && g.K >= 16 && (double)g.M * g.N * g.K >= 134217728.0) {
+        p.kernel = GemmPlan::UMMA;
+        p.bn = (int)(g.N >= 128 ? 128 : ceil_div(g.N, 16) * 16);
+        split_k(p, g.K, ceil_div(g.M, umma::UM) * ceil_div(g.N, p.bn), 3, umma::UBK, can_split);
+        // short inner dimension: the epilogue dominates; a 2-deep raw ring keeps two CTAs per SM
+        // (up to 256 inner columns the forward layout keeps the 2-deep ring as well - 121 registers, two CTAs per SM: 54 -> 39 us
+        // for the pred_layer product; the transposing variants need 154+ registers, one CTA per SM either way)
+        p.nraw = (p.kchunk <= 128 || (p.kchunk <= 256 && g.pass == GemmPass::FWD)) ? 2 : 4;
+        p.multi = p.kchunk > (int64_t)umma::UCH * umma::UBK;
+        p.smem = (size_t)umma::USTAGES * 2 * (umma::plane_bytes(umma::UM) + umma::plane_bytes(p.bn)) +
+                 (size_t)p.nraw * (umma::raw_bytes(umma::UM) + umma::raw_bytes(p.bn));
+        const size_t tile_bytes = (size_t)umma::UM * (p.bn + 4) * 4;      // epilogue staging tile reuses the operand stages
+        if (p.smem < tile_bytes) p.smem = tile_bytes;
+        auto al16 = [](const float* q, int64_t ld) { return q == nullptr || vec_ok(q, ld); };
+        p.vec_c4 = al16(g.C, g.ldc) && al16(g.add, g.ldadd) && al16(g.mask, g.ldmask) && al16(g.bias, 4);
+        return p;
+    }
+#endif
+    // mma.sync kernels: the largest tile that still yields ~2 waves of CTAs on the SMs; weight gradients with a small output
+    // take the warp-split kernel
+    if (wgrad && (g.M < 64 || g.N < 64)) p.cfg = 4;
+    else if (g.N <= 32) p.cfg = (ctas(128, 32) >= 2 * kNumSMs || can_split) ? 1 : 3;
+    else if (ctas(128, 64) >= 2 * kNumSMs || can_split) p.cfg = 0;
+    else if (ctas(64, 64) >= 2 * kNumSMs) p.cfg = 2;
+    else p.cfg = 3;
+    const int bm = p.cfg == 4 ? 32 : (p.cfg <= 1 ? 128 : 64), bn = (p.cfg == 0 || p.cfg == 2) ? 64 : 32;
+    split_k(p, g.K, ctas(bm, bn), 2, p.cfg == 4 ? SW_BK : BK, can_split);
+    if (skinny || p.cfg == 4) p.kernel = GemmPlan::WARPSPLIT;
+    else if (!wgrad && g.K == 32 && g.N <= 32 && vec_ok(g.A, g.lda) && g.accumulate != 2 && g.M >= 2048) p.kernel = GemmPlan::STREAM32;
+    else p.kernel = GemmPlan::TC;
+    return p;
+}
+
+template <int BM, int BN, int WM, int WN, bool AT, bool BT>
+static void launch_tc(const GemmDev& d, cudaStream_t s) {
+    auto k = gemm_tc_kernel<BM, BN, WM, WN, AT, BT>;
+    LAUNCH(k, dim3((unsigned)ceil_div(d.M, BM), (unsigned)ceil_div(d.N, BN), (unsigned)d.splits), dim3(WM * WN * 32), 0, s, d);
+}
+
+// AT / BT: the operand layouts of the pass
+template <bool AT, bool BT>
+static void gemm_launch(const GemmDev& d, const GemmPlan& p, cudaStream_t s) {
+    switch (p.kernel) {
+#ifndef INTEL_EMU
+    case GemmPlan::UMMA: {
+        using K = void (*)(GemmDev, int, int);
+        // [NACC = 32, 64, 128][one accumulation chunk; several chunks with 2 / 4 raw stages]
+        static const K kernels[3][3] = {
+            {umma::gemm_umma_kernel<AT, BT, 32, false, 2>, umma::gemm_umma_kernel<AT, BT, 32, true, 2>, umma::gemm_umma_kernel<AT, BT, 32, true, 4>},
+            {umma::gemm_umma_kernel<AT, BT, 64, false, 2>, umma::gemm_umma_kernel<AT, BT, 64, true, 2>, umma::gemm_umma_kernel<AT, BT, 64, true, 4>},
+            {umma::gemm_umma_kernel<AT, BT, 128, false, 2>, umma::gemm_umma_kernel<AT, BT, 128, true, 2>, umma::gemm_umma_kernel<AT, BT, 128, true, 4>}};
+        const K k = kernels[p.bn <= 32 ? 0 : (p.bn <= 64 ? 1 : 2)][!p.multi ? 0 : (p.nraw == 2 ? 1 : 2)];
+        ensure_smem(k, p.smem);
+        const dim3 grid((unsigned)ceil_div(d.M, umma::UM), (unsigned)ceil_div(d.N, p.bn), (unsigned)d.splits);
+        LAUNCH(k, grid, dim3(umma::UTHREADS), p.smem, s, d, p.bn, p.vec_c4);
+        break;
+    }
+#endif
+    case GemmPlan::WARPSPLIT: {
+        auto k = gemm_warpsplit_kernel<AT, BT>;
+        LAUNCH(k, dim3((unsigned)ceil_div(d.M, 32), (unsigned)ceil_div(d.N, 32), (unsigned)d.splits), dim3(256), 0, s, d);
+        break;
+    }
+    case GemmPlan::STREAM32: {
+        auto k = gemm_stream32_kernel<BT>;
+        LAUNCH(k, dim3(stream_grid(ceil_div(d.M, 16 * 8), 3)), dim3(256), 0, s, d);
+        break;
+    }
+    default:
+        if (p.cfg == 0) launch_tc<128, 64, 4, 2, AT, BT>(d, s);
+        else if (p.cfg == 1) launch_tc<128, 32, 4, 1, AT, BT>(d, s);
+        else if (p.cfg == 2) launch_tc<64, 64, 2, 2, AT, BT>(d, s);
+        else launch_tc<64, 32, 2, 1, AT, BT>(d, s);
+    }
+}
+
+int gemm_check_launch(const Gemm& g, const char* tag_fmt, ...) {
+    static const char* const names[] = {"gemm_fwd", "gemm_dgrad", "gemm_wgrad"};
+    const char* what = names[(int)g.pass];
+    if (prof_detail()) {
+        char tag[64], name[160];
+        va_list ap;
+        va_start(ap, tag_fmt);
+        vsnprintf(tag, sizeof(tag), tag_fmt, ap);
+        va_end(ap);
+        snprintf(name, sizeof(name), "%s[%lldx%lldx%lld,%s]", what, (long long)g.M, (long long)g.N, (long long)g.K, tag);
+        what = prof_intern(name);
+    }
+    const double bytes = 4.0 * ((double)g.M * g.K + (double)g.N * g.K +
+                                (double)g.M * g.N * (1 + (g.add != nullptr) + (g.mask != nullptr)));
+    return check_launch(what, bytes, 2.0 * g.M * g.N * g.K);
+}
 
 int gemm(const Gemm& g, cudaStream_t s) {
     if (g.M <= 0 || g.N <= 0) return INTEL_OK;
     INTEL_REQUIRE(g.A && g.B && g.C, INTEL_ERR_ARG, "gemm: null operand");
     INTEL_REQUIRE(g.M <= 0x7fffffffLL * 32 && g.N < (65535LL * 32), INTEL_ERR_ARG, "gemm: shape too large");
+    const GemmPlan p = gemm_plan(g);
+#ifndef INTEL_EMU
+    // tall products with a small resident weight operand, and weight gradients over tens of thousands of rows: the persistent
+    // warp-specialised tcgen05 kernels (gemm_rows_tc.cu, gemm_wgrad_tc.cu), when the shape fits them
+    if (g_tcgen05 && g_rows_gemm && !p.prezero) {
+        int st = 0;
+        if (gemm_rows_tc_try(g, s, &st) || gemm_wgrad_tc_try(g, s, &st)) return st;
+    }
+#endif
     GemmDev d;
     d.M = g.M; d.N = g.N; d.K = g.K;
     d.A = g.A; d.lda = g.lda; d.B = g.B; d.ldb = g.ldb; d.C = g.C; d.ldc = g.ldc;
@@ -738,148 +639,29 @@ int gemm(const Gemm& g, cudaStream_t s) {
     d.relu_a = g.relu_a; d.relu_b = g.relu_b; d.relu_out = g.relu_out; d.accumulate = g.accumulate;
     d.vec_a = vec_ok(g.A, g.lda);
     d.vec_b = vec_ok(g.B, g.ldb);
-    auto even = [](const float* p, int64_t ld) { return p == nullptr || ((((uintptr_t)p) % 8 == 0) && (ld % 2 == 0)); };
+    auto even = [](const float* q, int64_t ld) { return q == nullptr || ((((uintptr_t)q) % 8 == 0) && (ld % 2 == 0)); };
     d.vec_c = even(g.C, g.ldc) && even(g.add, g.ldadd) && even(g.mask, g.ldmask) && even(g.bias, 2);
-    INTEL_REQUIRE(g.a_t == false || g.b_t == true, INTEL_ERR_UNSUPPORTED, "gemm: A^T B layout is not used by this path");
-    const bool wgrad = g.a_t && g.b_t;
-    // tile choice: the largest tile that still yields ~2 waves of CTAs on the 148 SMs; weight gradients with a
-    // small output use the warp-split-K kernel, everything else the tiled kernel (with split-K when allowed)
-    // plain outputs with a long inner dimension and too few tiles to fill the GPU are also split: the output is
-    // cleared first and the partial products are accumulated with atomics
-    const bool prezero = (g.accumulate == 0 && !g.relu_out && !g.mask && g.splits == 1 && g.K >= 512 && g.N > 64 &&
-                          ceil_div(g.M, 128) * ceil_div(g.N, 64) < kNumSMs);
-    if (prezero) {
+    d.splits = p.splits;
+    d.kchunk = p.kchunk;
+    if (p.prezero) {
         cudaError_t e = cudaMemset2DAsync(g.C, (size_t)g.ldc * 4, 0, (size_t)g.N * 4, (size_t)g.M, s);
         INTEL_REQUIRE(e == cudaSuccess, INTEL_ERR_CUDA, "cudaMemset2DAsync: %s", cudaGetErrorString(e));
         d.accumulate = 2;
     }
-    const bool can_split = ((g.accumulate == 2 && !g.relu_out && !g.mask && g.splits <= 0) || prezero);
-    auto ctas = [&](int bm, int bn) { return ceil_div(g.M, bm) * ceil_div(g.N, bn); };
-    const char* what = wgrad ? "gemm_wgrad" : (g.b_t ? "gemm_dgrad" : "gemm_fwd");
-    const double bytes = 4.0 * ((double)d.M * d.K + (double)d.N * d.K +
-                                (double)d.M * d.N * (1 + (d.add != nullptr) + (d.mask != nullptr)));
-    {   // tall products with a small resident weight operand: persistent warp-specialised tcgen05 kernel (gemm_rows_tc.cu)
-        int st = 0;
-        if (g_use_umma && !prezero && gemm_rows_tc_try(g, s, what, &st)) return st;
-        if (g_use_umma && !prezero && gemm_wgrad_tc_try(g, s, what, &st)) return st;       // gemm_wgrad_tc.cu
+    switch (g.pass) {
+    case GemmPass::FWD: gemm_launch<false, false>(d, p, s); break;
+    case GemmPass::DGRAD: gemm_launch<false, true>(d, p, s); break;
+    case GemmPass::WGRAD: gemm_launch<true, true>(d, p, s); break;
     }
-#ifndef INTEL_EMU
-    // large products with 16-byte aligned operands: tcgen05 path (gemm_umma.cuh), 128 x bn tiles, TMEM accumulators
-    // (tall outputs with few columns and a long inner dimension fill too few 128-row tiles: the skinny kernel below)
-    const bool skinny = !g.a_t && g.splits == 1 && !prezero && g.N <= 64 && g.K >= 256 && ctas(128, 32) < 2 * kNumSMs;
-    if (g_use_umma && !skinny && g.M >= 128 && g.N >= 16 && g.K >= 16 && (double)g.M * g.N * g.K >= 134217728.0) {
-        static const int bn_cap = getenv("INTEL_UMMA_BN") ? atoi(getenv("INTEL_UMMA_BN")) : 128;      // tuning knob
-        const int bn_max = (g.K > 128 && bn_cap < 128) ? bn_cap : 128;
-        const int bn = (int)(g.N >= bn_max ? bn_max : ceil_div(g.N, 16) * 16);
-        const int64_t tiles = ceil_div(g.M, umma::UM) * ceil_div(g.N, bn);
-        int splits = prezero ? 0 : g.splits;
-        if (splits <= 0) {
-            splits = 1;
-            if (can_split) {
-                const int64_t want = ceil_div(3 * kNumSMs, tiles), maxs = ceil_div(g.K, 4 * umma::UBK);
-                splits = (int)(want < 1 ? 1 : (want > maxs ? maxs : want));
-            }
-        }
-        INTEL_REQUIRE(splits == 1 || (d.accumulate == 2 && !g.relu_out && !g.mask), INTEL_ERR_ARG,
-                      "gemm: split-K needs atomic accumulation and a linear epilogue");
-        INTEL_REQUIRE(splits <= 65535, INTEL_ERR_ARG, "gemm: too many splits");
-        d.splits = splits;
-        d.kchunk = ceil_div(ceil_div(g.K, splits), umma::UBK) * umma::UBK;
-        // short inner dimension: the epilogue dominates; a 2-deep raw ring keeps two CTAs per SM
-        // (up to 256 inner columns the forward layout keeps the 2-deep ring as well - 121 registers, two CTAs per SM: 54 -> 39 us
-        // for the pred_layer product; the transposing variants need 154+ registers, one CTA per SM either way)
-        const int nraw = (d.kchunk <= 128 || (d.kchunk <= 256 && !g.a_t && !g.b_t)) ? 2 : 4;
-        size_t smem = (size_t)umma::USTAGES * 2 * (umma::plane_bytes(umma::UM) + umma::plane_bytes(bn)) +
-                      (size_t)nraw * (umma::raw_bytes(umma::UM) + umma::raw_bytes(bn));
-        const size_t tile_bytes = (size_t)umma::UM * (bn + 4) * 4;      // epilogue staging tile reuses the operand stages
-        if (smem < tile_bytes) smem = tile_bytes;
-        dim3 grid((unsigned)ceil_div(g.M, umma::UM), (unsigned)ceil_div(g.N, bn), (unsigned)splits);
-        auto al16 = [](const float* p, int64_t ld) { return p == nullptr || ((((uintptr_t)p) % 16 == 0) && (ld % 4 == 0)); };
-        const int vec_c4 = al16(g.C, g.ldc) && al16(g.add, g.ldadd) && al16(g.mask, g.ldmask) && al16(g.bias, 4);
-        const bool multi = d.kchunk > (int64_t)umma::UCH * umma::UBK;
-#define INTEL_UMMA_N(ATR, BTR, NACC)                                                                                  \
-    do {                                                                                                              \
-        if (multi && nraw == 2) { auto k = umma::gemm_umma_kernel<ATR, BTR, NACC, true, 2>; ensure_smem(k, smem); LAUNCH(k, grid, dim3(umma::UTHREADS), smem, s, d, bn, vec_c4); }   \
-        else if (multi) { auto k = umma::gemm_umma_kernel<ATR, BTR, NACC, true, 4>; ensure_smem(k, smem); LAUNCH(k, grid, dim3(umma::UTHREADS), smem, s, d, bn, vec_c4); }   \
-        else { auto k = umma::gemm_umma_kernel<ATR, BTR, NACC, false, 2>; ensure_smem(k, smem); LAUNCH(k, grid, dim3(umma::UTHREADS), smem, s, d, bn, vec_c4); }       \
-    } while (0)
-#define INTEL_UMMA(ATR, BTR)                                                                                          \
-    do {                                                                                                              \
-        if (bn <= 32) INTEL_UMMA_N(ATR, BTR, 32);                                                                     \
-        else if (bn <= 64) INTEL_UMMA_N(ATR, BTR, 64);                                                                \
-        else INTEL_UMMA_N(ATR, BTR, 128);                                                                             \
-    } while (0)
-        if (!g.a_t && !g.b_t) INTEL_UMMA(false, false);
-        else if (!g.a_t) INTEL_UMMA(false, true);
-        else INTEL_UMMA(true, true);
-#undef INTEL_UMMA_N
-#undef INTEL_UMMA
-        if (prof_detail()) {
-            char name[128];
-            snprintf(name, sizeof(name), "%s[%lldx%lldx%lld,umma,bn%d,splits%d]", what, (long long)d.M, (long long)d.N, (long long)d.K, bn, splits);
-            what = prof_intern(name);
-        }
-        return check_launch(what, bytes, 2.0 * d.M * d.N * d.K);
-    }
-#endif
-    int cfg;   // 0: 128x64  1: 128x32  2: 64x64  3: 64x32  4: warp-split-K 32x32
-    if (wgrad && (g.M < 64 || g.N < 64)) cfg = 4;
-    else if (g.N <= 32) cfg = (ctas(128, 32) >= 2 * kNumSMs || can_split) ? 1 : 3;
-    else if (ctas(128, 64) >= 2 * kNumSMs || can_split) cfg = 0;
-    else if (ctas(64, 64) >= 2 * kNumSMs) cfg = 2;
-    else cfg = 3;
-    const int bm = cfg == 4 ? 32 : (cfg <= 1 ? 128 : 64), bn = (cfg == 0 || cfg == 2) ? 64 : 32;
-    const int bk = cfg == 4 ? WG_BK : BK;
-    int splits = prezero ? 0 : g.splits;
-    if (splits <= 0) {
-        splits = 1;
-        if (can_split) {
-            // few output tiles and a very long inner dimension: split it to fill ~2 waves of the 148 SMs
-            const int64_t want = ceil_div(2 * kNumSMs, ctas(bm, bn));
-            const int64_t maxs = ceil_div(g.K, 4 * bk);
-            splits = (int)(want < 1 ? 1 : (want > maxs ? maxs : want));
-            if (splits < 1) splits = 1;
-        }
-    }
-    INTEL_REQUIRE(splits == 1 || (d.accumulate == 2 && !g.relu_out && !g.mask), INTEL_ERR_ARG,
-                  "gemm: split-K needs atomic accumulation and a linear epilogue");
-    INTEL_REQUIRE(splits <= 65535, INTEL_ERR_ARG, "gemm: too many splits");
-    d.splits = splits;
-    d.kchunk = ceil_div(ceil_div(g.K, splits), bk) * bk;
-    if (d.kchunk <= 0) d.kchunk = bk;
-    if (!g.a_t && splits == 1 && g.N <= 64 && g.K >= 256 && ctas(128, 32) < 2 * kNumSMs) {
-        dim3 grid((unsigned)ceil_div(d.M, 32), (unsigned)ceil_div(d.N, 32));
-        if (g.b_t) { auto k = gemm_skinny_kernel<true>; LAUNCH(k, grid, dim3(256), 0, s, d); }
-        else { auto k = gemm_skinny_kernel<false>; LAUNCH(k, grid, dim3(256), 0, s, d); }
-    } else if (!g.a_t && g.K == 32 && g.N <= 32 && d.vec_a && g.accumulate != 2 && splits == 1 && g.M >= 2048) {
-        const unsigned grid = stream_grid(ceil_div(g.M, 16 * 8), 3);
-        if (g.b_t) { auto k = gemm_stream32_kernel<true>; LAUNCH(k, dim3(grid), dim3(256), 0, s, d); }
-        else { auto k = gemm_stream32_kernel<false>; LAUNCH(k, dim3(grid), dim3(256), 0, s, d); }
-    } else if (cfg == 4) {
-        dim3 grid((unsigned)ceil_div(d.M, 32), (unsigned)ceil_div(d.N, 32), (unsigned)d.splits);
-        LAUNCH(gemm_wgrad_kernel, grid, dim3(WG_WARPS * 32), 0, s, d);
-    } else if (cfg == 0) {
-        launch_tc<128, 64, 4, 2>(d, g.a_t, g.b_t, s);
-    } else if (cfg == 1) {
-        launch_tc<128, 32, 4, 1>(d, g.a_t, g.b_t, s);
-    } else if (cfg == 2) {
-        launch_tc<64, 64, 2, 2>(d, g.a_t, g.b_t, s);
-    } else {
-        launch_tc<64, 32, 2, 1>(d, g.a_t, g.b_t, s);
-    }
-    if (prof_detail()) {
-        char name[128];
-        snprintf(name, sizeof(name), "%s[%lldx%lldx%lld,cfg%d,splits%d,vec%d%d%d]", what, (long long)d.M, (long long)d.N,
-                 (long long)d.K, cfg, splits, d.vec_a, d.vec_b, d.vec_c);
-        what = prof_intern(name);
-    }
-    return check_launch(what, bytes, 2.0 * d.M * d.N * d.K);
+    if (p.kernel == GemmPlan::UMMA) return gemm_check_launch(g, "umma,bn%d,splits%d", p.bn, p.splits);
+    return gemm_check_launch(g, "cfg%d,splits%d,vec%d%d%d", p.cfg, p.splits, d.vec_a, d.vec_b, d.vec_c);
 }
 
 int linear(int64_t M, int64_t N, int64_t K, const float* A, int64_t lda, const float* W, int64_t ldw,
            const float* bias, float* C, int64_t ldc, cudaStream_t s, bool relu_a, bool relu_out,
            const float* add, int64_t ldadd, const int32_t* rows, const int32_t* nrows) {
     Gemm g;
+    g.pass = GemmPass::FWD;
     g.M = M; g.N = N; g.K = K; g.A = A; g.lda = lda; g.B = W; g.ldb = ldw; g.C = C; g.ldc = ldc;
     g.bias = bias; g.relu_a = relu_a; g.relu_out = relu_out; g.add = add; g.ldadd = ldadd; g.rows = rows; g.nrows = nrows;
     return gemm(g, s);
@@ -889,8 +671,9 @@ int linear_dx(int64_t M, int64_t N, int64_t K, const float* dY, int64_t lddy, co
               float* dX, int64_t lddx, cudaStream_t s, int accumulate, const float* mask, int64_t ldmask,
               const int32_t* rows, const int32_t* nrows) {
     Gemm g;   // dX[M,K] = dY[M,N] * W[N,K]: inner dimension N, B operand stored [inner][out]
+    g.pass = GemmPass::DGRAD;
     g.rows = rows; g.nrows = nrows;
-    g.M = M; g.N = K; g.K = N; g.A = dY; g.lda = lddy; g.B = W; g.ldb = ldw; g.b_t = true;
+    g.M = M; g.N = K; g.K = N; g.A = dY; g.lda = lddy; g.B = W; g.ldb = ldw;
     g.C = dX; g.ldc = lddx; g.accumulate = accumulate; g.mask = mask; g.ldmask = ldmask;
     return gemm(g, s);
 }
@@ -899,9 +682,10 @@ int linear_dw(int64_t M, int64_t N, int64_t K, const float* dY, int64_t lddy, co
               float* dW, int64_t lddw, float* db, cudaStream_t s, bool relu_x, const int32_t* rows, const int32_t* nrows) {
     if (dW) {
         Gemm g;   // dW[N,K] += sum_m dY[m,n] X[m,k]: both operands stored [inner][out]
+        g.pass = GemmPass::WGRAD;
         g.rows = rows; g.nrows = nrows;
-        g.M = N; g.N = K; g.K = M; g.A = dY; g.lda = lddy; g.a_t = true; g.B = X; g.ldb = ldx; g.b_t = true;
-        g.C = dW; g.ldc = lddw; g.accumulate = 2; g.splits = 0; g.relu_b = relu_x;
+        g.M = N; g.N = K; g.K = M; g.A = dY; g.lda = lddy; g.B = X; g.ldb = ldx;
+        g.C = dW; g.ldc = lddw; g.accumulate = 2; g.relu_b = relu_x;
         INTEL_TRY(gemm(g, s));
     }
     if (db) INTEL_TRY(colsum(M, N, dY, lddy, db, s));

@@ -37,15 +37,6 @@ struct RowsArgs {
     const int32_t* rows;                  // optional: the rows of A / C to process (Gemm::rows), *nrows of them
     const int32_t* nrows;
 };
-
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc05::smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool elect1() {
-    uint32_t p;
-    asm volatile("{\n.reg .pred P;\nelect.sync _|P, 0xffffffff;\nselp.u32 %0, 1, 0, P;\n}" : "=r"(p));
-    return p != 0;
-}
 }  // namespace
 
 __global__ void __launch_bounds__(RT_THREADS, 1) gemm_rows_tc_kernel(RowsArgs a) {
@@ -151,13 +142,13 @@ __global__ void __launch_bounds__(RT_THREADS, 1) gemm_rows_tc_kernel(RowsArgs a)
             }
             tc05::wait_st();
             tc05::fence_before();
-            mbar_arrive(&a_full[buf]);
+            tc05::mbar_arrive(&a_full[buf]);
 #pragma unroll
             for (int j = 0; j < RT_KC / 4; ++j) v[j] = nx[j];
         }
     } else if (warp == 8) {
         // ================= MMA issuer =================
-        if (elect1()) {
+        if (tc05::elect_one()) {
             const uint32_t lbo = (uint32_t)Np * 16;
             const uint64_t d_hi = tc05::make_desc(tc05::smem_u32(w_hi), lbo, 128), d_lo = tc05::make_desc(tc05::smem_u32(w_lo), lbo, 128);
             uint32_t ia = 0, id = 0;
@@ -239,7 +230,7 @@ __global__ void __launch_bounds__(RT_THREADS, 1) gemm_rows_tc_kernel(RowsArgs a)
                     if (Np > 32) tc05::ld32(tl + cD + bd * 128 + 32, v);
                     tc05::wait_ld();
                     tc05::fence_before();
-                    mbar_arrive(&d_empty[bd]);
+                    tc05::mbar_arrive(&d_empty[bd]);
 #pragma unroll
                     for (int j = 0; j < 32; ++j) {
                         acc[j] += __uint_as_float(u[j]);
@@ -304,7 +295,7 @@ __global__ void __launch_bounds__(RT_THREADS, 1) gemm_rows_tc_kernel(RowsArgs a)
                     __syncwarp();
                 }
                 tc05::fence_before();
-                mbar_arrive(&d_empty[bd]);
+                tc05::mbar_arrive(&d_empty[bd]);
             }
         }
     }
@@ -313,15 +304,12 @@ __global__ void __launch_bounds__(RT_THREADS, 1) gemm_rows_tc_kernel(RowsArgs a)
     if (warp == 8) tc05::tmem_free(tm, 512);
 }
 
-static int g_rows_tc = 1;
-void gemm_debug_use_rows_tc(int on) { g_rows_tc = on ? 1 : 0; }
-
 // returns true when the product was taken (status = launch status)
-bool gemm_rows_tc_try(const Gemm& g, cudaStream_t s, const char* what, int* status) {
-    if (!g_rows_tc || g.a_t || g.relu_a || g.relu_b || g.relu_out || g.add || g.mask || g.accumulate != 0 || g.splits > 1) return false;
+bool gemm_rows_tc_try(const Gemm& g, cudaStream_t s, int* status) {
+    if (g.pass == GemmPass::WGRAD || g.relu_a || g.relu_b || g.relu_out || g.add || g.mask || g.accumulate != 0) return false;
     if (g.M < 16384 || g.N < 16 || g.N % 4 || g.K % 4 || g.lda % 4 || g.ldc % 4) return false;
     if ((((uintptr_t)g.A) | ((uintptr_t)g.C)) % 16) return false;
-    if (g.b_t && g.bias) return false;
+    if (g.pass == GemmPass::DGRAD && g.bias) return false;
     const int Np = (int)((g.N + 15) / 16 * 16);
     const int nkc = (int)((g.K + RT_KC - 1) / RT_KC), nnc = (Np + RT_NB - 1) / RT_NB;
     if (nkc > 1 && (nnc > 1 || Np > 64)) return false;
@@ -329,25 +317,15 @@ bool gemm_rows_tc_try(const Gemm& g, cudaStream_t s, const char* what, int* stat
     const size_t smem = 2 * plane + 4 * 4096 + (size_t)((Np + 31) / 32 * 32) * 4 + 128;
     if (smem > 225 * 1024) return false;
     RowsArgs a;
-    a.M = g.M; a.N = (int)g.N; a.K = (int)g.K; a.A = g.A; a.lda = g.lda; a.W = g.B; a.ldw = g.ldb; a.w_t = g.b_t ? 1 : 0;
+    a.M = g.M; a.N = (int)g.N; a.K = (int)g.K; a.A = g.A; a.lda = g.lda; a.W = g.B; a.ldw = g.ldb; a.w_t = g.pass == GemmPass::DGRAD;
     a.bias = g.bias; a.C = g.C; a.ldc = g.ldc; a.nkc = nkc; a.nnc = nnc;
     a.rows = (g.rows && g.nrows) ? g.rows : nullptr; a.nrows = g.nrows;
     ensure_smem(gemm_rows_tc_kernel, smem);
     const unsigned grid = stream_grid((g.M + 127) / 128, 1);
     LAUNCH(gemm_rows_tc_kernel, dim3(grid), dim3(RT_THREADS), smem, s, a);
-    if (prof_detail()) {
-        char name[96];
-        snprintf(name, sizeof(name), "%s[%lldx%lldx%lld,rows_tc]", what, (long long)g.M, (long long)g.N, (long long)g.K);
-        what = prof_intern(name);
-    }
-    *status = check_launch(what, 4.0 * ((double)g.M * g.K + (double)g.N * g.K + (double)g.M * g.N), 2.0 * g.M * g.N * g.K);
+    *status = gemm_check_launch(g, "rows_tc");
     return true;
 }
 
-}  // namespace intel
-#else
-namespace intel {
-void gemm_debug_use_rows_tc(int) {}
-bool gemm_rows_tc_try(const Gemm&, cudaStream_t, const char*, int*) { return false; }
 }  // namespace intel
 #endif

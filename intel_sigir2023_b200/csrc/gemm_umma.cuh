@@ -16,6 +16,7 @@
 // TMEM tile is drained into fp32 registers with a rounded add and the next MMA starts a fresh sum.
 #pragma once
 #ifndef INTEL_EMU
+#include "tc05.cuh"
 
 namespace intel {
 namespace umma {
@@ -28,50 +29,6 @@ static const int USTAGES = 2;          // plane stages (MMA of tile i overlaps t
 static const int USBO = 144;           // stride of an 8-row core-matrix group: 128 + 16 keeps the transposing stores conflict-free
 static const int UCH = 8;            // k-tiles per accumulation chunk (drained into registers with rounded adds)
 static const int UTHREADS = 256;       // 8 warps: copy / convert work is spread over all of them, warps w and w + 4 share TMEM lanes
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred P1;\n"
-        "LAB_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-        "@P1 bra DONE;\n"
-        "bra LAB_WAIT;\n"
-        "DONE:\n"
-        "}" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-// the mbarrier receives one arrival when every tcgen05.mma issued so far by this thread has completed
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "setp.ne.b32 p, %4, 0;\n"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n"
-        "}" ::"r"(tmem_d),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
-    uint32_t r[16];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
 
 // Shared-memory plane of one operand and stage: ROWS x 16 TF32 words, K-major no-swizzle canonical layout:
 // 16-byte unit (row r, k-chunk c) at c * LBO + (r / 8) * USBO + (r % 8) * 16;  LBO == 64 (mod 128) spreads the four
@@ -90,14 +47,6 @@ __device__ __forceinline__ void cp_async4(uint32_t dst, const void* src, int byt
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-    uint64_t d = (uint64_t)((saddr >> 4) & 0x3FFFu);
-    d |= (uint64_t)((lbo >> 4) & 0x3FFFu) << 16;
-    d |= (uint64_t)((sbo >> 4) & 0x3FFFu) << 32;
-    d |= (uint64_t)1 << 46;                          // descriptor version of sm_100
-    return d;                                        // base offset 0, no swizzle
-}
 
 __device__ __forceinline__ void put_unit(uint8_t* hi, uint8_t* lo, int off, float a, float b, float c, float d, int relu) {
     if (relu) { a = fmaxf(a, 0.f); b = fmaxf(b, 0.f); c = fmaxf(c, 0.f); d = fmaxf(d, 0.f); }
@@ -231,26 +180,21 @@ __global__ void __launch_bounds__(UTHREADS) gemm_umma_kernel(GemmDev g, int bn, 
     const int stage_bytes = 2 * pa + 2 * pb;
     const int ra = raw_bytes(UM), rb = raw_bytes(bn);
     uint8_t* planes = umma_smem + NRAW * (ra + rb);
-    const uint32_t raw_base = smem_u32(umma_smem);
+    const uint32_t raw_base = tc05::smem_u32(umma_smem);
 
     if (tid == 0) {
 #pragma unroll
-        for (int s = 0; s < USTAGES; ++s) mbar_init(&empty_bar[s], 1);
-        mbar_init(&chunk_bar, 1);
+        for (int s = 0; s < USTAGES; ++s) tc05::mbar_init(&empty_bar[s], 1);
+        tc05::mbar_init(&chunk_bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)), "r"(NACC)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    if (warp == 0) tc05::tmem_alloc(&tmem_base_s, NACC);
+    tc05::fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tc05::fence_after();
     const uint32_t tmem_d = tmem_base_s;
 
-    // instruction descriptor: D = f32 (bit 4), A = B = tf32 (bits 7, 10), both K-major, N >> 3 at bit 17, M >> 4 at bit 24
-    const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(bn >> 3) << 17) | ((uint32_t)(UM >> 4) << 24);
+    const uint32_t idesc = tc05::make_idesc(UM, bn);
     const uint32_t a_lbo = lbo_k(UM), b_lbo = lbo_k(bn);
 
     // warps w and w + 4 read the same 32 TMEM lanes (= output rows) and take alternate 16-column chunks
@@ -278,7 +222,7 @@ __global__ void __launch_bounds__(UTHREADS) gemm_umma_kernel(GemmDev g, int bn, 
         const int s = i % USTAGES;
         uint8_t* st = planes + s * stage_bytes;
         cp_async_wait<NRAW - 2>();                                                        // this thread's chunks of k-tile i have landed
-        if (i >= USTAGES) mbar_wait(&empty_bar[s], (uint32_t)((i / USTAGES) - 1) & 1u);   // MMAs of k-tile i - USTAGES are done
+        if (i >= USTAGES) tc05::mbar_wait(&empty_bar[s], (uint32_t)((i / USTAGES) - 1) & 1u);   // MMAs of k-tile i - USTAGES are done
         const uint8_t* rw = umma_smem + (i % NRAW) * (ra + rb);
         la.convert(rw, st, st + pa, g.relu_a);
         lb.convert(rw + ra, st + 2 * pa, st + 2 * pa + pb, g.relu_b);
@@ -290,39 +234,40 @@ __global__ void __launch_bounds__(UTHREADS) gemm_umma_kernel(GemmDev g, int bn, 
             lb.issue(dst + ra, t, k0, kend);
         }
         cp_async_commit();
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // generic-proxy writes -> visible to the tensor core
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");  // orders the drain's tcgen05.ld before the next MMA
+        tc05::fence_smem_to_mma();
+        tc05::fence_before();           // orders the drain's tcgen05.ld before the next MMA
         __syncthreads();
         const bool chunk_end = (i % UCH == UCH - 1) || (i == nk - 1);
         if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const uint32_t sa = smem_u32(st), sb = smem_u32(st + 2 * pa);
+            tc05::fence_after();
+            const uint32_t sa = tc05::smem_u32(st), sb = tc05::smem_u32(st + 2 * pa);
 #pragma unroll
             for (int ks = 0; ks < UBK / 8; ++ks) {
-                const uint64_t ah = make_desc(sa + ks * 2 * a_lbo, a_lbo, USBO), al = make_desc(sa + pa + ks * 2 * a_lbo, a_lbo, USBO);
-                const uint64_t bh = make_desc(sb + ks * 2 * b_lbo, b_lbo, USBO), bl = make_desc(sb + pb + ks * 2 * b_lbo, b_lbo, USBO);
-                umma_tf32(tmem_d, al, bh, idesc, ((i % UCH) | ks) ? 1u : 0u);      // a chunk starts a fresh sum
-                umma_tf32(tmem_d, ah, bl, idesc, 1u);
-                umma_tf32(tmem_d, ah, bh, idesc, 1u);
+                const uint64_t ah = tc05::make_desc(sa + ks * 2 * a_lbo, a_lbo, USBO), al = tc05::make_desc(sa + pa + ks * 2 * a_lbo, a_lbo, USBO);
+                const uint64_t bh = tc05::make_desc(sb + ks * 2 * b_lbo, b_lbo, USBO), bl = tc05::make_desc(sb + pb + ks * 2 * b_lbo, b_lbo, USBO);
+                tc05::mma_ss(tmem_d, al, bh, idesc, ((i % UCH) | ks) ? 1u : 0u);      // a chunk starts a fresh sum
+                tc05::mma_ss(tmem_d, ah, bl, idesc, 1u);
+                tc05::mma_ss(tmem_d, ah, bh, idesc, 1u);
             }
-            umma_commit(&empty_bar[s]);
-            if (chunk_end) umma_commit(&chunk_bar);
+            tc05::commit(&empty_bar[s]);
+            if (chunk_end) tc05::commit(&chunk_bar);
         }
         if (chunk_end) {
             // the chunk's MMAs are complete: warp w may read TMEM lanes 32 w .. 32 w + 31 = its output rows
-            mbar_wait(&chunk_bar, chunk_phase);
+            tc05::mbar_wait(&chunk_bar, chunk_phase);
             chunk_phase ^= 1u;
             __syncwarp();
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc05::fence_after();
             if (MULTI && i != nk - 1) {             // drain: acc += TMEM tile (rounded fp32 adds)
 #pragma unroll
                 for (int cc = 0; cc < NACC / 32; ++cc) {
                     const int c0 = (2 * cc + chalf) * 16;
                     if (c0 < bn) {
-                        float v[16];
-                        tmem_ld16(tmem_d + ((uint32_t)lanes0 << 16) + (uint32_t)c0, v);
+                        uint32_t v[16];
+                        tc05::ld16(tmem_d + ((uint32_t)lanes0 << 16) + (uint32_t)c0, v);
+                        tc05::wait_ld();
 #pragma unroll
-                        for (int j = 0; j < 16; ++j) acc[MULTI ? cc * 16 + j : 0] += v[j];
+                        for (int j = 0; j < 16; ++j) acc[MULTI ? cc * 16 + j : 0] += __uint_as_float(v[j]);
                     }
                 }
             }
@@ -339,8 +284,12 @@ __global__ void __launch_bounds__(UTHREADS) gemm_umma_kernel(GemmDev g, int bn, 
         for (int cc = 0; cc < (NACC >= 32 ? NACC / 32 : 1); ++cc) {
             const int c0 = (2 * cc + chalf) * 16;
             if (c0 < bn) {
+                uint32_t u[16];
+                tc05::ld16(tmem_d + ((uint32_t)lanes0 << 16) + (uint32_t)c0, u);
+                tc05::wait_ld();
                 float v[16];
-                tmem_ld16(tmem_d + ((uint32_t)lanes0 << 16) + (uint32_t)c0, v);
+#pragma unroll
+                for (int j = 0; j < 16; ++j) v[j] = __uint_as_float(u[j]);
                 if (MULTI) {
 #pragma unroll
                     for (int j = 0; j < 16; ++j) v[j] += acc[MULTI ? cc * 16 + j : 0];
@@ -351,9 +300,9 @@ __global__ void __launch_bounds__(UTHREADS) gemm_umma_kernel(GemmDev g, int bn, 
             }
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc05::fence_before();
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "r"(NACC) : "memory");
+    if (warp == 0) tc05::tmem_free(tmem_d, NACC);
 
     // step 2: tile -> global, one row per warp pass with the lanes along the columns (coalesced); bias / residual /
     // relu / mask are applied here

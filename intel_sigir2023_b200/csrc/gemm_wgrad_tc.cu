@@ -33,14 +33,6 @@ struct WgradArgs {
     const int32_t* nrows;
 };
 
-__device__ __forceinline__ void mbar_arrive_w(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc05::smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool elect_w() {
-    uint32_t p;
-    asm volatile("{\n.reg .pred P;\nelect.sync _|P, 0xffffffff;\nselp.u32 %0, 1, 0, P;\n}" : "=r"(p));
-    return p != 0;
-}
 // byte offset of 16-byte chunk `ch` (0..7) of row `r` (0..31) inside a sub-tile: 32-byte chunk index ^ (row & 3)
 __device__ __forceinline__ int sub_off(int r, int ch) { return r * 128 + ((((ch >> 1) ^ (r & 3)) << 1) | (ch & 1)) * 16; }
 }  // namespace
@@ -111,7 +103,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) gemm_wgrad_tc_kernel(WgradArgs 
                 for (int q = 0; q < 16; ++q) acc[q] += __uint_as_float(u[q]);
             }
             tc05::fence_before();
-            mbar_arrive_w(&acc_empty[buf]);
+            tc05::mbar_arrive(&acc_empty[buf]);
         };
         // unit u of a stage = (operand, sub-tile, row quad): a warp instruction moves 4 rows x 128 bytes of one sub-tile; warp w
         // takes row quad w of every sub-tile.  The loads of stage i + 1 are issued before stage i is converted, so the HBM
@@ -151,7 +143,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) gemm_wgrad_tc_kernel(WgradArgs 
                 }
             }
             tc05::fence_smem_to_mma();
-            mbar_arrive_w(&stage_full[st]);
+            tc05::mbar_arrive(&stage_full[st]);
 #pragma unroll
             for (int i = 0; i < 4; ++i) { va[i] = na[i]; vb[i] = nb[i]; }
             if ((it & 3) == 3 && it >= 7) fold((it >> 2) - 1);          // block (it / 4) is fed: fold the one before it
@@ -169,7 +161,7 @@ __global__ void __launch_bounds__(WG_THREADS, 1) gemm_wgrad_tc_kernel(WgradArgs 
         }
     } else {
         // ================= MMA issuer =================
-        if (elect_w()) {
+        if (tc05::elect_one()) {
             const uint32_t idesc = tc05::make_idesc(128, Np, 1, 1);
             uint32_t sc = 0;
             for (int64_t blk = 0; blk < nblk; ++blk) {
@@ -201,12 +193,9 @@ __global__ void __launch_bounds__(WG_THREADS, 1) gemm_wgrad_tc_kernel(WgradArgs 
     if (warp == 8) tc05::tmem_free(tm, 256);
 }
 
-static int g_wgrad_tc = 1;
-void gemm_debug_use_wgrad_tc(int on) { g_wgrad_tc = on ? 1 : 0; }
-
 // dW[M, N] += dY^T X (both stored [rows][cols]); false = shape not taken
-bool gemm_wgrad_tc_try(const Gemm& g, cudaStream_t s, const char* what, int* status) {
-    if (!g_wgrad_tc || !(g.a_t && g.b_t) || g.accumulate != 2 || g.relu_a || g.relu_b || g.relu_out || g.add || g.mask || g.bias) return false;
+bool gemm_wgrad_tc_try(const Gemm& g, cudaStream_t s, int* status) {
+    if (g.pass != GemmPass::WGRAD || g.accumulate != 2 || g.relu_a || g.relu_b || g.relu_out || g.add || g.mask || g.bias) return false;
     if (g.M < 128 || g.M % 128 || g.N < 32 || g.N > 128 || g.N % 4 || g.K < 16384) return false;
     if (g.lda % 4 || g.ldb % 4 || (((uintptr_t)g.A) | ((uintptr_t)g.B)) % 16) return false;
     const int nsub = (int)((g.N + 31) / 32);
@@ -224,19 +213,9 @@ bool gemm_wgrad_tc_try(const Gemm& g, cudaStream_t s, const char* what, int* sta
     const size_t smem = (size_t)WG_STAGES * WG_STAGE_BYTES + 1024;
     ensure_smem(gemm_wgrad_tc_kernel, smem);
     LAUNCH(gemm_wgrad_tc_kernel, dim3((unsigned)mslices, (unsigned)splits), dim3(WG_THREADS), smem, s, a);
-    if (prof_detail()) {
-        char name[96];
-        snprintf(name, sizeof(name), "%s[%lldx%lldx%lld,wgrad_tc]", what, (long long)g.M, (long long)g.N, (long long)g.K);
-        what = prof_intern(name);
-    }
-    *status = check_launch(what, 4.0 * ((double)g.M * g.K + (double)g.N * g.K + (double)g.M * g.N), 2.0 * g.M * g.N * g.K);
+    *status = gemm_check_launch(g, "wgrad_tc");
     return true;
 }
 
-}  // namespace intel
-#else
-namespace intel {
-void gemm_debug_use_wgrad_tc(int) {}
-bool gemm_wgrad_tc_try(const Gemm&, cudaStream_t, const char*, int*) { return false; }
 }  // namespace intel
 #endif

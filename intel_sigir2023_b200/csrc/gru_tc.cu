@@ -56,11 +56,6 @@ __device__ __forceinline__ float rcpa(float x) {
 // parity budget is 1e-5 of the tensor's largest entry)
 __device__ __forceinline__ float sigmoid_fast(float x) { return rcpa(1.0f + ex2a(-1.4426950408889634f * x)); }
 __device__ __forceinline__ float tanh_fast(float x) { return 1.0f - 2.0f * rcpa(1.0f + ex2a(2.885390081777927f * x)); }
-__device__ __forceinline__ bool elect_lane() {
-    uint32_t p;
-    asm volatile("{\n.reg .pred P;\nelect.sync _|P, 0xffffffff;\nselp.u32 %0, 1, 0, P;\n}" : "=r"(p));
-    return p != 0;
-}
 }  // namespace
 
 // Up to two encoders (the session-history and the item-history GRU of IntEL.predict_intent) share one launch: cluster q
@@ -163,7 +158,7 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(128, 1) gru_tc_fwd_k
         __syncthreads();
         if (warp == 0) {
             tc05::fence_after();
-            if (elect_lane()) {
+            if (tc05::elect_one()) {
 #pragma unroll 4
                 for (int ks = 0; ks < GT_H / 8; ++ks) {
                     const uint64_t bh = d_hi + (uint64_t)((ks * 2 * GT_W_LBO) >> 4), bl = d_lo + (uint64_t)((ks * 2 * GT_W_LBO) >> 4);

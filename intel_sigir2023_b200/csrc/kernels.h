@@ -6,18 +6,23 @@
 
 namespace intel {
 
-// ---- gemm.cu: fp32 FFMA tiled GEMM, C = epilogue(op(A) * op(B)) -------------------------------
+// ---- gemm.cu: fp32-parity (3xTF32) GEMM of the nn.Linear passes, C[M,N] = epilogue(A B^T) ----------------
+// The pass fixes the operand layouts: FWD   A [M][K], B [N][K]  (Y = X W^T, linear)
+//                                     DGRAD A [M][K], B [K][N]  (dX = dY W, linear_dx)
+//                                     WGRAD A [K][M], B [K][N]  (dW += dY^T X, linear_dw; accumulate == 2, the inner
+//                                                                dimension may be split over CTAs)
+enum class GemmPass { FWD, DGRAD, WGRAD };
 struct Gemm {
+    GemmPass pass = GemmPass::FWD;
     int64_t M = 0, N = 0, K = 0;
-    const float* A = nullptr; int64_t lda = 0; bool a_t = false;  // a_t: A stored [K][M]
-    const float* B = nullptr; int64_t ldb = 0; bool b_t = false;  // b_t: B stored [K][N]; else [N][K] (nn.Linear)
+    const float* A = nullptr; int64_t lda = 0;
+    const float* B = nullptr; int64_t ldb = 0;
     float* C = nullptr; int64_t ldc = 0;
     const float* bias = nullptr;                        // + bias[n]
     const float* add = nullptr; int64_t ldadd = 0;      // + add[m,n]
     const float* mask = nullptr; int64_t ldmask = 0;    // *= (mask[m,n] > 0)   (relu backward)
     bool relu_a = false, relu_b = false, relu_out = false;
-    int accumulate = 0;   // 0: C = r   1: C += r   2: atomicAdd(C, r) (required when splits > 1)
-    int splits = 1;       // split of the inner dimension (0 = pick automatically for accumulate == 2)
+    int accumulate = 0;   // 0: C = r   1: C += r   2: atomicAdd(C, r)
     // optional list of the rows that matter (device int32 [*nrows], *nrows on the device too): the rows of A and C for a
     // forward / input-gradient product, the contracted rows for a weight gradient.  Rows that are not listed are padding
     // (history slots behind a session's length): the persistent tcgen05 kernels walk the list and never touch them, the
@@ -26,12 +31,15 @@ struct Gemm {
     const int32_t* nrows = nullptr;
 };
 int gemm(const Gemm& g, cudaStream_t s);
+void gemm_debug_use_tcgen05(int on);     // off: every product on the mma.sync kernels
+void gemm_debug_use_rows_gemm(int on);   // off: not the two persistent kernels below (the generic tcgen05 kernel stays)
+// launch status of a product, recorded by the profiler as gemm_fwd / gemm_dgrad / gemm_wgrad, and per shape as
+// "<name>[MxNxK,<tag>]" under prof_detail(); tag_fmt is a printf format
+int gemm_check_launch(const Gemm& g, const char* tag_fmt, ...);
 // gemm_rows_tc.cu: persistent tcgen05 kernel for tall products with a resident weight operand; false = shape not taken
-bool gemm_rows_tc_try(const Gemm& g, cudaStream_t s, const char* what, int* status);
-void gemm_debug_use_rows_tc(int on);
+bool gemm_rows_tc_try(const Gemm& g, cudaStream_t s, int* status);
 // gemm_wgrad_tc.cu: dW += dY^T X over tens of thousands of rows, both operands MN-major natural tiles
-bool gemm_wgrad_tc_try(const Gemm& g, cudaStream_t s, const char* what, int* status);
-void gemm_debug_use_wgrad_tc(int on);
+bool gemm_wgrad_tc_try(const Gemm& g, cudaStream_t s, int* status);
 // C[M,N] = A[M,K] W[N,K]^T (+bias)
 int linear(int64_t M, int64_t N, int64_t K, const float* A, int64_t lda, const float* W, int64_t ldw,
            const float* bias, float* C, int64_t ldc, cudaStream_t s, bool relu_a = false, bool relu_out = false,
@@ -235,7 +243,6 @@ void trunk_debug_use_tcgen05(int on);
 void trunk_debug_sessions_per_cta(int n);
 void trunk_reserve_sms(int n);      // SMs the persistent backward kernel leaves to a concurrent collective ...
 void trunk_reserve_apply(bool on);  // ... in the launches made while this is on
-void gemm_debug_use_umma(int on);
 bool trunk_supported(int64_t L, int d, int heads, int layers);      // mma.sync kernels, forward and backward
 bool trunk_fwd_supported(int64_t L, int heads, int layers);         // any fused forward kernel (d = 32)
 // w.X[0] = stack input [B*L,32]; w.X[l+1] receives the output of layer l

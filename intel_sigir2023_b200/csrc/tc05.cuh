@@ -1,4 +1,4 @@
-// tcgen05 / tensor-memory primitives shared by the fused stack kernels (trunk_tc.cu).  Every form used here was
+// tcgen05 / tensor-memory primitives shared by the tcgen05 kernels (trunk_tc.cu, gru_tc.cu, the GEMMs).  Every form used here was
 // checked bit-exact on a B200 with tests/hw/umma_probe.cu (profiles/r02_probe.md):
 //   * kind::tf32 MMA with the A operand in shared memory (SS) or in tensor memory (TS), fp32 accumulator in TMEM;
 //   * the disable-output-lane mask (four 32-bit words, bit set = accumulator lane not written): two sessions that share
@@ -30,6 +30,15 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
         "}" ::"r"(smem_u32(bar)),
         "r"(parity)
         : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+// one lane of a converged warp (the MMA operands then stay in uniform registers instead of going through R2UR per MMA)
+__device__ __forceinline__ bool elect_one() {
+    uint32_t p;
+    asm volatile("{\n.reg .pred P;\nelect.sync _|P, 0xffffffff;\nselp.u32 %0, 1, 0, P;\n}" : "=r"(p));
+    return p != 0;
 }
 // one arrival on the mbarrier once every tcgen05.mma issued so far by this thread has completed
 __device__ __forceinline__ void commit(uint64_t* bar) {

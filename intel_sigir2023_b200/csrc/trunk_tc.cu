@@ -81,12 +81,6 @@ __device__ __forceinline__ void mma3_ts(uint32_t d, uint32_t a_hi, uint32_t a_lo
 
 }  // namespace
 
-// one lane of a converged warp (the MMA operands then stay in uniform registers instead of going through R2UR per MMA)
-__device__ __forceinline__ bool elect_one() {
-    uint32_t p;
-    asm volatile("{\n.reg .pred P;\nelect.sync _|P, 0xffffffff;\nselp.u32 %0, 1, 0, P;\n}" : "=r"(p));
-    return p != 0;
-}
 // descriptor of the same layout `bytes` further into shared memory
 __device__ __forceinline__ uint64_t desc_at(uint64_t base, uint32_t bytes) { return base + (uint64_t)(bytes >> 4); }
 
@@ -192,7 +186,7 @@ __global__ void __launch_bounds__(256, 1) trunk_tc_fwd_kernel(TrunkArgs a, int C
             TC_PUBLISH();
             if (warp == 0) {
                 tc05::fence_after();
-                if (elect_one()) {
+                if (tc05::elect_one()) {
 #pragma unroll
                     for (int ks = 0; ks < 4; ++ks)
                         mma3_ts(tm + cS, tm + cA + 8 * ks, tm + cA + 32 + 8 * ks, desc_at(d_wqkv_hi, ks * 2 * 1536),
@@ -236,7 +230,7 @@ __global__ void __launch_bounds__(256, 1) trunk_tc_fwd_kernel(TrunkArgs a, int C
                 TC_PUBLISH();
                 if (warp == 0) {
                     tc05::fence_after();
-                    if (elect_one()) {
+                    if (tc05::elect_one()) {
 #pragma unroll
                         for (int hd = 0; hd < HEADS; ++hd)
 #pragma unroll
@@ -320,7 +314,7 @@ __global__ void __launch_bounds__(256, 1) trunk_tc_fwd_kernel(TrunkArgs a, int C
                 TC_PUBLISH();
                 if (warp == 0) {
                     tc05::fence_after();
-                    if (elect_one()) {
+                    if (tc05::elect_one()) {
 #pragma unroll
                         for (int ss = 0; ss < NS; ++ss) {
                             const tc05::LaneMask m = tc05::mask_rows(ss * SR, SR);
@@ -351,7 +345,7 @@ __global__ void __launch_bounds__(256, 1) trunk_tc_fwd_kernel(TrunkArgs a, int C
                 TC_PUBLISH();
                 if (warp == 0) {
                     tc05::fence_after();
-                    if (elect_one()) {
+                    if (tc05::elect_one()) {
 #pragma unroll
                         for (int ks = 0; ks < 4; ++ks)
                             mma3_ts(tm + cS, tm + cA + 8 * ks, tm + cA + 32 + 8 * ks, desc_at(d_w1_hi, ks * 2 * 512), desc_at(d_w1_lo, ks * 2 * 512),
@@ -378,7 +372,7 @@ __global__ void __launch_bounds__(256, 1) trunk_tc_fwd_kernel(TrunkArgs a, int C
                 TC_PUBLISH();
                 if (warp == 0) {
                     tc05::fence_after();
-                    if (elect_one()) {
+                    if (tc05::elect_one()) {
 #pragma unroll
                         for (int ks = 0; ks < 4; ++ks)
                             mma3_ts(tm + cS + 32, tm + cA + 8 * ks, tm + cA + 32 + 8 * ks, desc_at(d_w2_hi, ks * 2 * 512),
@@ -528,7 +522,7 @@ __global__ void __launch_bounds__(256, 1) trunk_tc_long_fwd_kernel(TrunkArgs a, 
                 TL_PUBLISH();
                 if (warp == 0 && rows) {
                     tc05::fence_after();
-                    if (elect_one()) {
+                    if (tc05::elect_one()) {
 #pragma unroll
                         for (int ks = 0; ks < 4; ++ks)
                             mma3_ts(tm + cS, tm + cA + 8 * ks, tm + cA + 32 + 8 * ks, desc_at(d_wqkv_hi, ks * 2 * 1536),
@@ -600,7 +594,7 @@ __global__ void __launch_bounds__(256, 1) trunk_tc_long_fwd_kernel(TrunkArgs a, 
                     TL_PUBLISH();
                     if (warp == 0 && rows) {
                         tc05::fence_after();
-                        if (elect_one()) {
+                        if (tc05::elect_one()) {
 #pragma unroll
                             for (int ks = 0; ks < DK / 8; ++ks) {
                                 const uint32_t koff = (uint32_t)((hd * (DK / 4) + 2 * ks) * TL_K_LBO);
@@ -666,7 +660,7 @@ __global__ void __launch_bounds__(256, 1) trunk_tc_long_fwd_kernel(TrunkArgs a, 
                     inv[hd] = 1.0f / (pstat[t] + pstat[128 + t]);
                     if (warp == 0 && rows) {
                         tc05::fence_after();
-                        if (elect_one()) {
+                        if (tc05::elect_one()) {
 #pragma unroll 2
                             for (int ks = 0; ks < pv_steps; ++ks) {
                                 const uint32_t voff = (uint32_t)(hd * DK * 16 + ks * 2 * TC_VT_LBO);
@@ -696,7 +690,7 @@ __global__ void __launch_bounds__(256, 1) trunk_tc_long_fwd_kernel(TrunkArgs a, 
                     TL_PUBLISH();
                     if (warp == 0 && rows) {
                         tc05::fence_after();
-                        if (elect_one()) {
+                        if (tc05::elect_one()) {
 #pragma unroll
                             for (int ks = 0; ks < 4; ++ks)
                                 mma3_ts(tm + cS, tm + cA + 8 * ks, tm + cA + 32 + 8 * ks, desc_at(d_w1_hi, ks * 2 * 512), desc_at(d_w1_lo, ks * 2 * 512),
@@ -725,7 +719,7 @@ __global__ void __launch_bounds__(256, 1) trunk_tc_long_fwd_kernel(TrunkArgs a, 
                     TL_PUBLISH();
                     if (warp == 0 && rows) {
                         tc05::fence_after();
-                        if (elect_one()) {
+                        if (tc05::elect_one()) {
 #pragma unroll
                             for (int ks = 0; ks < 4; ++ks)
                                 mma3_ts(tm + cS + 32, tm + cA + 8 * ks, tm + cA + 32 + 8 * ks, desc_at(d_w2_hi, ks * 2 * 512),
