@@ -391,28 +391,59 @@ int gru_fwd_pair(const intel_dims_t* d, const History (&hs)[2], EncWs (&e)[2], f
     return INTEL_OK;
 }
 
-// w.dh holds d(last state) on entry (intel_intent_bwd_rows forms it for both encoders)
-int gru_bwd(const intel_dims_t* d, const intel_encoder_t& p, intel_encoder_t& g, EncWs& e, const int64_t* lens,
-            const float* dout, int64_t ld, cudaStream_t s) {
-    const int64_t B = d->B, T = e.T, R = B * T;
-    const int dd = e.d, h = d->gru_hidden;
-    GruWs& w = e.gru;
-    INTEL_TRY(linear_dw(B, dd, h, dout, ld, w.h_all + T * h, (T + 1) * h, g.w_out, h, nullptr, s));
-    // the recurrence kernel writes dgh_all[:, 0..T-1] of every session (zeros behind a session's end): only slot T, which
-    // pairs with the final state in the weight-gradient product below, needs clearing (6 MB instead of 132 MB)
-    cudaError_t ce = cudaMemset2DAsync(w.dgh_all + T * 3 * h, (size_t)(T + 1) * 3 * h * 4, 0, (size_t)3 * h * 4, (size_t)B, s);
-    INTEL_REQUIRE(ce == cudaSuccess, INTEL_ERR_CUDA, "cudaMemset2DAsync: %s", cudaGetErrorString(ce));
-    // with the length order, tiles of equally long sessions stop at their own last step; the order is the forward call's,
-    // its tile counter is reset here
-    if (w.order) INTEL_TRY(fill_zero(w.order + B, sizeof(int32_t), s));
-    // the kernel also sums the bias gradients (column sums of dgi / dgh) on its way
-    INTEL_TRY(gru_seq_bwd(B, T, lens, p.w_hh, w.h_all, w.gates, w.dh, w.dgi, w.dgh_all, g.b_ih, g.b_hh, s, w.order));
-    // gradient rows of padding slots are zero: the three products below contract / map the live rows only (the list was
-    // built by the forward call); d(seq) of the padding slots is cleared for the scatters that read every row
-    INTEL_TRY(linear_dw(B * (T + 1), 3 * h, h, w.dgh_all, 3 * h, w.h_all, h, g.w_hh, h, nullptr, s, false, w.rows_t1, w.nlive));
-    INTEL_TRY(linear_dw(R, 3 * h, dd, w.dgi, 3 * h, e.seq, dd, g.w_ih, dd, nullptr, s, false, w.rows_t, w.nlive));
-    if (w.rows_t) INTEL_TRY(fill_zero(e.dseq, (size_t)R * dd * 4, s));
-    return linear_dx(R, 3 * h, dd, w.dgi, 3 * h, p.w_ih, dd, e.dseq, dd, s, 0, nullptr, 0, w.rows_t, w.nlive);
+// Backward pass of both GRU encoders; w.dh holds d(last state) on entry (intel_intent_bwd_rows forms it for both).
+// The products of each encoder after the recurrence: dW_hh += dgh_all^T h_all over the [B, T+1] rows, dW_ih += dgi^T seq
+// and d(seq) = dgi W_ih over the [B, T] rows, each over the live rows alone when the encoder has the live-row lists.
+struct GruBwdProducts { Gemm whh, wih, dseq; };
+int gru_bwd_pair(const intel_dims_t* d, const History (&hs)[2], EncWs (&e)[2], const float* dfeat, int64_t ld, cudaStream_t s) {
+    const int64_t B = d->B;
+    const int h = d->gru_hidden;
+    GruBwdProducts pr[2];
+    GruBwdPair rec;
+    for (int i = 0; i < 2; ++i) {
+        const int64_t T = e[i].T, R = B * T;
+        const int dd = e[i].d;
+        GruWs& w = e[i].gru;
+        const intel_encoder_t &p = *hs[i].p, &g = *hs[i].g;
+        INTEL_TRY(linear_dw(B, dd, h, dfeat + hs[i].off, ld, w.h_all + T * h, (T + 1) * h, g.w_out, h, nullptr, s));
+        pr[i].whh = wgrad_gemm(B * (T + 1), 3 * h, h, w.dgh_all, 3 * h, w.h_all, h, g.w_hh, h, w.rows_t1, w.nlive);
+        pr[i].wih = wgrad_gemm(R, 3 * h, dd, w.dgi, 3 * h, e[i].seq, dd, g.w_ih, dd, w.rows_t, w.nlive);
+        pr[i].dseq = dgrad_gemm(R, 3 * h, dd, w.dgi, 3 * h, p.w_ih, dd, e[i].dseq, dd, w.rows_t, w.nlive);
+        // when all three products read the live rows alone, the recurrence writes nothing for the padding slots (about half
+        // of the [B, T] rows); otherwise it writes their gradient rows as zeros, and slot T of dgh_all, which pairs with the
+        // final state in the dW_hh product, is cleared here
+        const bool live_only = gemm_rows_only(pr[i].whh) && gemm_rows_only(pr[i].wih) && gemm_rows_only(pr[i].dseq);
+        if (!live_only) {
+            cudaError_t ce = cudaMemset2DAsync(w.dgh_all + T * 3 * h, (size_t)(T + 1) * 3 * h * 4, 0, (size_t)3 * h * 4, (size_t)B, s);
+            INTEL_REQUIRE(ce == cudaSuccess, INTEL_ERR_CUDA, "cudaMemset2DAsync: %s", cudaGetErrorString(ce));
+        }
+        // with the length order, tiles of equally long sessions stop at their own last step; the order is the forward call's,
+        // its tile counter (order[B]) is reset here
+        if (w.order) INTEL_TRY(fill_zero(w.order + B, sizeof(int32_t), s));
+        // the recurrence also sums the bias gradients (column sums of dgi / dgh) on its way
+        rec.e[i] = GruBwdOne{B, T, hs[i].lens, p.w_hh, w.h_all, w.gates, w.dh, w.dgi, w.dgh_all, g.b_ih, g.b_hh, w.order,
+                             w.order ? w.order + B : nullptr, live_only ? 1 : 0};
+    }
+    // one launch for both recurrences when both have the length order (their tiles are drawn from its counters), else one each
+    if (rec.e[0].counter && rec.e[1].counter) {
+        rec.n = 2;
+        INTEL_TRY(gru_seq_bwd_pair(rec, s));
+    } else {
+        for (int i = 0; i < 2; ++i) {
+            GruBwdPair one;
+            one.e[0] = rec.e[i];
+            one.n = 1;
+            INTEL_TRY(gru_seq_bwd_pair(one, s));
+        }
+    }
+    for (int i = 0; i < 2; ++i) {
+        INTEL_TRY(gemm(pr[i].whh, s));
+        INTEL_TRY(gemm(pr[i].wih, s));
+        // d(seq) of the padding slots is cleared for the scatters that read every row
+        if (e[i].gru.rows_t) INTEL_TRY(fill_zero(e[i].dseq, (size_t)B * e[i].T * e[i].d * 4, s));
+        INTEL_TRY(gemm(pr[i].dseq, s));
+    }
+    return INTEL_OK;
 }
 
 }  // namespace
@@ -785,8 +816,7 @@ int intel_intent_bwd_rows(const intel_dims_t* d, const intel_tensors_t* P, const
             for (int i = 0; i < 2; ++i)
                 INTEL_TRY(linear_dx(B, w.e[i].d, h, w.dfeat + hs[i].off, Dp, hs[i].p->w_out, h, w.e[i].gru.dh, h, s));
         }
-        for (int i = 0; i < 2; ++i)
-            INTEL_TRY(gru_bwd(d, *hs[i].p, *hs[i].g, w.e[i], hs[i].lens, w.dfeat + hs[i].off, Dp, s));
+        INTEL_TRY(gru_bwd_pair(d, hs, w.e, w.dfeat, Dp, s));
     }
     INTEL_TRY(fill_zero(w.dWt, (size_t)I * dint * 4, s));
     for (int i = 0; i < 2; ++i) {

@@ -667,25 +667,47 @@ int linear(int64_t M, int64_t N, int64_t K, const float* A, int64_t lda, const f
     return gemm(g, s);
 }
 
-int linear_dx(int64_t M, int64_t N, int64_t K, const float* dY, int64_t lddy, const float* W, int64_t ldw,
-              float* dX, int64_t lddx, cudaStream_t s, int accumulate, const float* mask, int64_t ldmask,
-              const int32_t* rows, const int32_t* nrows) {
+bool gemm_rows_only(const Gemm& g) {
+#ifndef INTEL_EMU
+    if (g.rows && g.nrows && g_tcgen05 && g_rows_gemm && !gemm_plan(g).prezero)
+        return gemm_rows_tc_try(g, nullptr, nullptr) || gemm_wgrad_tc_try(g, nullptr, nullptr);
+#endif
+    return false;
+}
+
+Gemm dgrad_gemm(int64_t M, int64_t N, int64_t K, const float* dY, int64_t lddy, const float* W, int64_t ldw, float* dX,
+                int64_t lddx, const int32_t* rows, const int32_t* nrows) {
     Gemm g;   // dX[M,K] = dY[M,N] * W[N,K]: inner dimension N, B operand stored [inner][out]
     g.pass = GemmPass::DGRAD;
     g.rows = rows; g.nrows = nrows;
     g.M = M; g.N = K; g.K = N; g.A = dY; g.lda = lddy; g.B = W; g.ldb = ldw;
-    g.C = dX; g.ldc = lddx; g.accumulate = accumulate; g.mask = mask; g.ldmask = ldmask;
+    g.C = dX; g.ldc = lddx;
+    return g;
+}
+
+Gemm wgrad_gemm(int64_t M, int64_t N, int64_t K, const float* dY, int64_t lddy, const float* X, int64_t ldx, float* dW,
+                int64_t lddw, const int32_t* rows, const int32_t* nrows) {
+    Gemm g;   // dW[N,K] += sum_m dY[m,n] X[m,k]: both operands stored [inner][out]
+    g.pass = GemmPass::WGRAD;
+    g.rows = rows; g.nrows = nrows;
+    g.M = N; g.N = K; g.K = M; g.A = dY; g.lda = lddy; g.B = X; g.ldb = ldx;
+    g.C = dW; g.ldc = lddw; g.accumulate = 2;
+    return g;
+}
+
+int linear_dx(int64_t M, int64_t N, int64_t K, const float* dY, int64_t lddy, const float* W, int64_t ldw,
+              float* dX, int64_t lddx, cudaStream_t s, int accumulate, const float* mask, int64_t ldmask,
+              const int32_t* rows, const int32_t* nrows) {
+    Gemm g = dgrad_gemm(M, N, K, dY, lddy, W, ldw, dX, lddx, rows, nrows);
+    g.accumulate = accumulate; g.mask = mask; g.ldmask = ldmask;
     return gemm(g, s);
 }
 
 int linear_dw(int64_t M, int64_t N, int64_t K, const float* dY, int64_t lddy, const float* X, int64_t ldx,
               float* dW, int64_t lddw, float* db, cudaStream_t s, bool relu_x, const int32_t* rows, const int32_t* nrows) {
     if (dW) {
-        Gemm g;   // dW[N,K] += sum_m dY[m,n] X[m,k]: both operands stored [inner][out]
-        g.pass = GemmPass::WGRAD;
-        g.rows = rows; g.nrows = nrows;
-        g.M = N; g.N = K; g.K = M; g.A = dY; g.lda = lddy; g.B = X; g.ldb = ldx;
-        g.C = dW; g.ldc = lddw; g.accumulate = 2; g.relu_b = relu_x;
+        Gemm g = wgrad_gemm(M, N, K, dY, lddy, X, ldx, dW, lddw, rows, nrows);
+        g.relu_b = relu_x;
         INTEL_TRY(gemm(g, s));
     }
     if (db) INTEL_TRY(colsum(M, N, dY, lddy, db, s));

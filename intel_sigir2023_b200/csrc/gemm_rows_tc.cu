@@ -316,6 +316,7 @@ bool gemm_rows_tc_try(const Gemm& g, cudaStream_t s, int* status) {
     const size_t plane = (size_t)Np * nkc * RT_KC * 4;
     const size_t smem = 2 * plane + 4 * 4096 + (size_t)((Np + 31) / 32 * 32) * 4 + 128;
     if (smem > 225 * 1024) return false;
+    if (!status) return true;
     RowsArgs a;
     a.M = g.M; a.N = (int)g.N; a.K = (int)g.K; a.A = g.A; a.lda = g.lda; a.W = g.B; a.ldw = g.ldb; a.w_t = g.pass == GemmPass::DGRAD;
     a.bias = g.bias; a.C = g.C; a.ldc = g.ldc; a.nkc = nkc; a.nnc = nnc;

@@ -200,6 +200,7 @@ bool gemm_wgrad_tc_try(const Gemm& g, cudaStream_t s, int* status) {
     if (g.lda % 4 || g.ldb % 4 || (((uintptr_t)g.A) | ((uintptr_t)g.B)) % 16) return false;
     const int nsub = (int)((g.N + 31) / 32);
     if (nsub == 3) return false;                                          // N padded to 96: the fold assumes 32 / 64 / 128 columns
+    if (!status) return true;
     WgradArgs a;
     a.R = g.K; a.M = (int)g.M; a.N = (int)g.N; a.dY = g.A; a.ldy = g.lda; a.X = g.B; a.ldx = g.ldb; a.dW = g.C; a.ldw = g.ldc;
     a.rows = (g.rows && g.nrows) ? g.rows : nullptr; a.nrows = g.nrows;

@@ -418,24 +418,74 @@ int gru_prep(int n, const GruPrepOne* e, cudaStream_t s) {
     return check_launch("gru_prep");
 }
 
-// Backward recurrence.  dh [B,128] holds d(loss)/d h_T on entry.  Writes dgi [B,T,384] and
-// dgh_all [B,T+1,384] (slot T untouched: the caller clears the buffer) for the weight-gradient GEMMs.
-__global__ void __launch_bounds__(256, 1) gru_seq_bwd_kernel(int64_t B, int64_t T, const int64_t* __restrict__ lens,
-                                                             const float* __restrict__ w_hh,
-                                                             const float* __restrict__ h_all,
-                                                             const float* __restrict__ gates,
-                                                             const float* __restrict__ dh_in, float* __restrict__ dgi,
-                                                             float* __restrict__ dgh_all, float* __restrict__ db_ih,
-                                                             float* __restrict__ db_hh, const int32_t* __restrict__ order,
-                                                             int32_t* __restrict__ counter) {
+// Backward recurrence of up to two encoders in one launch (GruBwdOne / GruBwdPair, kernels.h).  dh_in [B,128] holds
+// d(loss)/d h_T on entry.  Writes dgi [B,T,384] and dgh_all [B,T+1,384] (slot T untouched) for the weight-gradient GEMMs.
+// Each encoder has its own W_hh, and restaging it costs a CTA as much as a few steps: so every CTA draws the tiles of its
+// home encoder (blockIdx.x % n) from that encoder's counter, longest first, and only when they are gone the remaining
+// (shortest) tiles of the other one.  One launch then balances the SMs over the tiles of both encoders, and no CTA
+// stages W_hh more than twice.
+__global__ void __launch_bounds__(256, 1) gru_seq_bwd_kernel(GruBwdPair a) {
     DYN_SMEM(float, sm);
-    __shared__ int s_tile;
+    __shared__ int s_tile, s_enc;
+    __shared__ float s_bias[2][4][GH];       // per encoder: column sums of dgi (r, z, n) and of the n part of dgh
     float* Ws = sm;                          // [384][GW]   W_hh[k = gate column][n = hidden]
     float* ds = Ws + 3 * GH * GW;            // [GB_SB][GD] dgh of the current step
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int gq = lane >> 2, tq = lane & 3;
-    stage_whh(Ws, w_hh);                     // once per CTA: the CTA is persistent and walks tiles of GB_SB sessions
-    float sum_i[2][3][2], sum_h[2][2];        // bias-gradient partial sums: [ct][gate][e] of dgi, [ct][e] of the n-gate of dgh
+    for (int e = threadIdx.x; e < 2 * 4 * GH; e += blockDim.x) (&s_bias[0][0][0])[e] = 0.f;
+    const int home = (int)(blockIdx.x % a.n);
+    const int64_t ntiles0 = (a.e[0].B + GB_SB - 1) / GB_SB, ntiles1 = a.n > 1 ? (a.e[1].B + GB_SB - 1) / GB_SB : 0;
+    int staged = -1;                         // the encoder whose W_hh is in shared memory
+    for (int64_t it = 0;; ++it) {
+    // next tile: with the length-sorted orders the tiles are handed out longest first from the counters (the CTAs that
+    // drew short tiles come back for more), otherwise round robin (one encoder)
+    int64_t tile = (int64_t)blockIdx.x + it * gridDim.x;
+    int enc = 0;
+    if (a.e[0].counter) {
+        if (threadIdx.x == 0) {
+            int e = staged < 0 ? home : staged;
+            int t = atomicAdd(e ? a.e[1].counter : a.e[0].counter, 1);
+            if (t >= (e ? ntiles1 : ntiles0) && e == home && a.n > 1) {
+                e ^= 1;
+                t = atomicAdd(e ? a.e[1].counter : a.e[0].counter, 1);
+            }
+            s_tile = t;
+            s_enc = e;
+        }
+        __syncthreads();
+        tile = s_tile;
+        enc = s_enc;
+    }
+    if (tile >= (enc ? ntiles1 : ntiles0)) break;
+    const GruBwdOne E = enc ? a.e[1] : a.e[0];
+    const int64_t B = E.B, T = E.T;
+    const int64_t b0 = tile * GB_SB;
+    if (enc != staged) {
+        __syncthreads();                     // no warp still reads the other encoder's W_hh
+        stage_whh(Ws, E.w_hh);
+        staged = enc;
+    }
+    // the tile's sessions: consecutive entries of the length-sorted order (longest first), so the first one bounds the loop;
+    // session slots beyond B are marked with B (every access below is guarded by b < B)
+    auto sess = [&](int64_t i) -> int64_t { return i < B ? (E.order ? (int64_t)E.order[i] : i) : B; };
+    int64_t tmax = T;
+    if (E.order) {
+        const int64_t l0 = E.lens[sess(b0)];
+        tmax = l0 < 0 ? 0 : (l0 > T ? T : l0);
+    }
+    // without live_only, gradient rows behind the tile's last live step are zero (a product reads every row)
+    if (!E.live_only && tmax < T) {
+        const int64_t per = (T - tmax) * (3 * GH / 4);
+        for (int64_t e = threadIdx.x; e < (int64_t)GB_SB * per; e += blockDim.x) {
+            const int64_t b = sess(b0 + e / per), r = e % per;
+            if (b < B) {
+                const int64_t t = tmax + r / (3 * GH / 4), c4 = (r % (3 * GH / 4)) * 4;
+                *reinterpret_cast<float4*>(E.dgi + (b * T + t) * 3 * GH + c4) = make_float4(0.f, 0.f, 0.f, 0.f);
+                *reinterpret_cast<float4*>(E.dgh_all + (b * (T + 1) + t) * 3 * GH + c4) = make_float4(0.f, 0.f, 0.f, 0.f);
+            }
+        }
+    }
+    float sum_i[2][3][2], sum_h[2][2];        // the tile's bias-gradient partial sums: [ct][gate][e] of dgi, [ct][e] of dgh_n
 #pragma unroll
     for (int ct = 0; ct < 2; ++ct)
 #pragma unroll
@@ -444,50 +494,18 @@ __global__ void __launch_bounds__(256, 1) gru_seq_bwd_kernel(int64_t B, int64_t 
 #pragma unroll
             for (int q = 0; q < 3; ++q) sum_i[ct][q][e] = 0.f;
         }
-    const int64_t ntiles = (B + GB_SB - 1) / GB_SB;
-    for (int64_t it = 0;; ++it) {
-    // next tile: with the length-sorted order the tiles are handed out longest first from a device counter (the CTAs that
-    // drew short tiles come back for more), otherwise round robin
-    int64_t tile = (int64_t)blockIdx.x + it * gridDim.x;
-    if (counter) {
-        if (threadIdx.x == 0) s_tile = atomicAdd(counter, 1);
-        __syncthreads();
-        tile = s_tile;
-    }
-    if (tile >= ntiles) break;
-    const int64_t b0 = tile * GB_SB;
-    // the tile's sessions: consecutive entries of the length-sorted order (longest first), so the first one bounds the loop;
-    // session slots beyond B are marked with B (every access below is guarded by b < B)
-    auto sess = [&](int64_t i) -> int64_t { return i < B ? (order ? (int64_t)order[i] : i) : B; };
-    int64_t tmax = T;
-    if (order) {
-        const int64_t l0 = lens[sess(b0)];
-        tmax = l0 < 0 ? 0 : (l0 > T ? T : l0);
-    }
-    // gradient rows behind the tile's last live step are zero (the weight-gradient products read every row)
-    if (tmax < T) {
-        const int64_t per = (T - tmax) * (3 * GH / 4);
-        for (int64_t e = threadIdx.x; e < (int64_t)GB_SB * per; e += blockDim.x) {
-            const int64_t b = sess(b0 + e / per), r = e % per;
-            if (b < B) {
-                const int64_t t = tmax + r / (3 * GH / 4), c4 = (r % (3 * GH / 4)) * 4;
-                *reinterpret_cast<float4*>(dgi + (b * T + t) * 3 * GH + c4) = make_float4(0.f, 0.f, 0.f, 0.f);
-                *reinterpret_cast<float4*>(dgh_all + (b * (T + 1) + t) * 3 * GH + c4) = make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-        }
-    }
     int64_t len_r[2], b_r[2];
     float dh[2][2][2];                       // [half][ct][e]: rows gq / gq+8, cols 16*warp + 8*ct + 2*tq + e
 #pragma unroll
     for (int hh = 0; hh < 2; ++hh) {
         const int64_t b = sess(b0 + hh * 8 + gq);
         b_r[hh] = b;
-        len_r[hh] = (b < B) ? lens[b] : 0;
+        len_r[hh] = (b < B) ? E.lens[b] : 0;
 #pragma unroll
         for (int ct = 0; ct < 2; ++ct) {
             const int c = 16 * warp + 8 * ct + 2 * tq;
             float2 v = make_float2(0.f, 0.f);
-            if (b < B) v = *reinterpret_cast<const float2*>(dh_in + b * GH + c);
+            if (b < B) v = *reinterpret_cast<const float2*>(E.dh_in + b * GH + c);
             dh[hh][ct][0] = v.x;
             dh[hh][ct][1] = v.y;
         }
@@ -507,10 +525,10 @@ __global__ void __launch_bounds__(256, 1) gru_seq_bwd_kernel(int64_t B, int64_t 
 #pragma unroll
                 for (int q = 0; q < 5; ++q) v[hh][ct][q] = make_float2(0.f, 0.f);
                 if (live) {
-                    const float* gt = gates + (b * T + t) * 4 * GH;
+                    const float* gt = E.gates + (b * T + t) * 4 * GH;
 #pragma unroll
                     for (int q = 0; q < 4; ++q) v[hh][ct][q] = *reinterpret_cast<const float2*>(gt + q * GH + c);
-                    v[hh][ct][4] = *reinterpret_cast<const float2*>(h_all + (b * (T + 1) + t) * GH + c);
+                    v[hh][ct][4] = *reinterpret_cast<const float2*>(E.h_all + (b * (T + 1) + t) * GH + c);
                 }
             }
         }
@@ -541,9 +559,9 @@ __global__ void __launch_bounds__(256, 1) gru_seq_bwd_kernel(int64_t B, int64_t 
                     dh[hh][ct][0] = g0 * z.x;
                     dh[hh][ct][1] = g1 * z.y;
                 }
-                if (b < B) {
-                    float* di = dgi + (b * T + t) * 3 * GH;
-                    float* dg = dgh_all + (b * (T + 1) + t) * 3 * GH;
+                if (live || (!E.live_only && b < B)) {
+                    float* di = E.dgi + (b * T + t) * 3 * GH;
+                    float* dg = E.dgh_all + (b * (T + 1) + t) * 3 * GH;
                     *reinterpret_cast<float2*>(di + c) = dr;
                     *reinterpret_cast<float2*>(di + GH + c) = dz;
                     *reinterpret_cast<float2*>(di + 2 * GH + c) = dn;
@@ -564,77 +582,103 @@ __global__ void __launch_bounds__(256, 1) gru_seq_bwd_kernel(int64_t B, int64_t 
         float2 nx[2][2][5];
         fetch(t - 1, nx);
         // ---- dh_prev = dh * z + dgh W_hh : [16 x 384] x [384 x 128], this warp owns 16 output columns ----
-        float acc[2][4];
+        // hi*hi and the two small products go to separate accumulators, and so do even and odd k-slices: eight
+        // independent chains of at most 48 dependent MMAs per warp instead of two of 144
+        float hi[2][2][4], lo[2][2][4];      // [k-slice parity][ct][frag]
 #pragma unroll
-        for (int ct = 0; ct < 2; ++ct)
+        for (int p = 0; p < 2; ++p)
 #pragma unroll
-            for (int c = 0; c < 4; ++c) acc[ct][c] = 0.f;
-#pragma unroll 4
-        for (int ks = 0; ks < 3 * GH / 8; ++ks) {
-            const int k0 = ks * 8 + tq;
-            uint32_t ah[4], al[4];
-            split_tf32(ds[gq * GD + k0], ah[0], al[0]);
-            split_tf32(ds[(gq + 8) * GD + k0], ah[1], al[1]);
-            split_tf32(ds[gq * GD + k0 + 4], ah[2], al[2]);
-            split_tf32(ds[(gq + 8) * GD + k0 + 4], ah[3], al[3]);
-            uint32_t bh[2][2], bl[2][2];
+            for (int ct = 0; ct < 2; ++ct)
 #pragma unroll
-            for (int ct = 0; ct < 2; ++ct) {
-                const int n = 16 * warp + 8 * ct + gq;
-                split_tf32(Ws[k0 * GW + n], bh[ct][0], bl[ct][0]);
-                split_tf32(Ws[(k0 + 4) * GW + n], bh[ct][1], bl[ct][1]);
+                for (int c = 0; c < 4; ++c) hi[p][ct][c] = lo[p][ct][c] = 0.f;
+#pragma unroll 2
+        for (int ks = 0; ks < 3 * GH / 8; ks += 2) {
+#pragma unroll
+            for (int p = 0; p < 2; ++p) {
+                const int k0 = (ks + p) * 8 + tq;
+                uint32_t ah[4], al[4];
+                split_tf32(ds[gq * GD + k0], ah[0], al[0]);
+                split_tf32(ds[(gq + 8) * GD + k0], ah[1], al[1]);
+                split_tf32(ds[gq * GD + k0 + 4], ah[2], al[2]);
+                split_tf32(ds[(gq + 8) * GD + k0 + 4], ah[3], al[3]);
+                uint32_t bh[2][2], bl[2][2];
+#pragma unroll
+                for (int ct = 0; ct < 2; ++ct) {
+                    const int n = 16 * warp + 8 * ct + gq;
+                    split_tf32(Ws[k0 * GW + n], bh[ct][0], bl[ct][0]);
+                    split_tf32(Ws[(k0 + 4) * GW + n], bh[ct][1], bl[ct][1]);
+                }
+#pragma unroll
+                for (int ct = 0; ct < 2; ++ct) mma_tf32(lo[p][ct], al, bh[ct]);
+#pragma unroll
+                for (int ct = 0; ct < 2; ++ct) mma_tf32(lo[p][ct], ah, bl[ct]);
+#pragma unroll
+                for (int ct = 0; ct < 2; ++ct) mma_tf32(hi[p][ct], ah, bh[ct]);
             }
-#pragma unroll
-            for (int ct = 0; ct < 2; ++ct) mma_tf32(acc[ct], al, bh[ct]);
-#pragma unroll
-            for (int ct = 0; ct < 2; ++ct) mma_tf32(acc[ct], ah, bl[ct]);
-#pragma unroll
-            for (int ct = 0; ct < 2; ++ct) mma_tf32(acc[ct], ah, bh[ct]);
         }
 #pragma unroll
         for (int hh = 0; hh < 2; ++hh)
 #pragma unroll
             for (int ct = 0; ct < 2; ++ct) {
-                dh[hh][ct][0] += acc[ct][2 * hh];
-                dh[hh][ct][1] += acc[ct][2 * hh + 1];
+#pragma unroll
+                for (int e = 0; e < 2; ++e) {
+                    const int f = 2 * hh + e;
+                    dh[hh][ct][e] += (lo[0][ct][f] + lo[1][ct][f]) + (hi[0][ct][f] + hi[1][ct][f]);
+                }
 #pragma unroll
                 for (int q = 0; q < 5; ++q) sv[hh][ct][q] = nx[hh][ct][q];
             }
         __syncthreads();                    // the dgh tile is rewritten by the next step
     }
+    // ---- the tile's bias-gradient sums, added to the CTA's per-encoder sums (one owner lane per column) ----
+#pragma unroll
+    for (int ct = 0; ct < 2; ++ct)
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            float v[4] = {sum_i[ct][0][e], sum_i[ct][1][e], sum_i[ct][2][e], sum_h[ct][e]};
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                v[q] += __shfl_xor_sync(0xffffffffu, v[q], 4);
+                v[q] += __shfl_xor_sync(0xffffffffu, v[q], 8);
+                v[q] += __shfl_xor_sync(0xffffffffu, v[q], 16);
+            }
+            if (gq == 0) {
+                const int c = 16 * warp + 8 * ct + 2 * tq + e;
+#pragma unroll
+                for (int q = 0; q < 4; ++q) s_bias[enc][q][c] += v[q];
+            }
+        }
     }   // tile loop
     // ---- bias gradients: db_ih = column sums of dgi, db_hh = column sums of dgh (r and z parts are shared) ----
-    if (db_ih != nullptr || db_hh != nullptr) {
-#pragma unroll
-        for (int ct = 0; ct < 2; ++ct)
-#pragma unroll
-            for (int e = 0; e < 2; ++e) {
-                float v[4] = {sum_i[ct][0][e], sum_i[ct][1][e], sum_i[ct][2][e], sum_h[ct][e]};
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    v[q] += __shfl_xor_sync(0xffffffffu, v[q], 4);
-                    v[q] += __shfl_xor_sync(0xffffffffu, v[q], 8);
-                    v[q] += __shfl_xor_sync(0xffffffffu, v[q], 16);
-                }
-                if (gq == 0) {
-                    const int c = 16 * warp + 8 * ct + 2 * tq + e;
-                    if (db_ih) { atomicAdd(db_ih + c, v[0]); atomicAdd(db_ih + GH + c, v[1]); atomicAdd(db_ih + 2 * GH + c, v[2]); }
-                    if (db_hh) { atomicAdd(db_hh + c, v[0]); atomicAdd(db_hh + GH + c, v[1]); atomicAdd(db_hh + 2 * GH + c, v[3]); }
-                }
-            }
+    __syncthreads();
+    for (int i = 0; i < a.n; ++i) {
+        float *db_ih = a.e[i].db_ih, *db_hh = a.e[i].db_hh;
+        for (int c = threadIdx.x; c < GH; c += blockDim.x) {
+            const float r = s_bias[i][0][c], z = s_bias[i][1][c];
+            if (db_ih) { atomicAdd(db_ih + c, r); atomicAdd(db_ih + GH + c, z); atomicAdd(db_ih + 2 * GH + c, s_bias[i][2][c]); }
+            if (db_hh) { atomicAdd(db_hh + c, r); atomicAdd(db_hh + GH + c, z); atomicAdd(db_hh + 2 * GH + c, s_bias[i][3][c]); }
+        }
     }
 }
 
-int gru_seq_bwd(int64_t B, int64_t T, const int64_t* lens, const float* w_hh, const float* h_all, const float* gates,
-                const float* dh_in, float* dgi, float* dgh_all, float* db_ih, float* db_hh, cudaStream_t s, int32_t* order) {
-    if (B <= 0 || T <= 0) return INTEL_OK;
+int gru_seq_bwd_pair(const GruBwdPair& p, cudaStream_t s) {
+    int64_t tiles = 0;
+    double bytes = 0.0, flops = 0.0;
+    INTEL_REQUIRE(p.n == 1 || (p.n == 2 && p.e[0].counter && p.e[1].counter), INTEL_ERR_ARG,
+                  "gru_seq_bwd: two encoders need a tile counter each");
+    for (int i = 0; i < p.n; ++i) {
+        const GruBwdOne& o = p.e[i];
+        INTEL_REQUIRE(o.B >= 0 && o.T >= 0, INTEL_ERR_ARG, "gru_seq_bwd: bad shape");
+        tiles += ceil_div(o.B, GB_SB);
+        bytes += (double)o.B * o.T * (4 + 1 + 3 + 3) * GH * 4.0;
+        flops += 2.0 * o.B * o.T * 3 * GH * GH;
+    }
+    if (tiles <= 0) return INTEL_OK;
     const size_t smem = (size_t)(3 * GH * GW + GB_SB * GD) * 4;
     ensure_smem(gru_seq_bwd_kernel, smem);
-    // persistent: one CTA per SM (W_hh fills its shared memory), tiles drawn from the counter behind `order` (order[B])
-    const unsigned grid = stream_grid(ceil_div(B, GB_SB), 1);
-    LAUNCH(gru_seq_bwd_kernel, dim3(grid), dim3(256), smem, s, B, T, lens, w_hh, h_all, gates,
-           dh_in, dgi, dgh_all, db_ih, db_hh, (const int32_t*)order, order ? order + B : (int32_t*)nullptr);
-    return check_launch("gru_seq_bwd", (double)B * T * (4 + 1 + 3 + 3) * GH * 4.0, 2.0 * B * T * 3 * GH * GH);
+    // persistent: one CTA per SM (W_hh fills its shared memory)
+    LAUNCH(gru_seq_bwd_kernel, dim3(stream_grid(tiles, 1)), dim3(256), smem, s, p);
+    return check_launch("gru_seq_bwd", bytes, flops);
 }
 
 }  // namespace intel

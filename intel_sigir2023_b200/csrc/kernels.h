@@ -26,7 +26,8 @@ struct Gemm {
     // optional list of the rows that matter (device int32 [*nrows], *nrows on the device too): the rows of A and C for a
     // forward / input-gradient product, the contracted rows for a weight gradient.  Rows that are not listed are padding
     // (history slots behind a session's length): the persistent tcgen05 kernels walk the list and never touch them, the
-    // generic kernels ignore the list and compute them as well - the listed rows come out the same either way.
+    // generic kernels ignore the list and compute them as well - the listed rows come out the same either way.  A weight
+    // gradient on a generic kernel contracts the unlisted rows too: they must hold zeros unless gemm_rows_only(g).
     const int32_t* rows = nullptr;
     const int32_t* nrows = nullptr;
 };
@@ -36,10 +37,19 @@ void gemm_debug_use_rows_gemm(int on);   // off: not the two persistent kernels 
 // launch status of a product, recorded by the profiler as gemm_fwd / gemm_dgrad / gemm_wgrad, and per shape as
 // "<name>[MxNxK,<tag>]" under prof_detail(); tag_fmt is a printf format
 int gemm_check_launch(const Gemm& g, const char* tag_fmt, ...);
-// gemm_rows_tc.cu: persistent tcgen05 kernel for tall products with a resident weight operand; false = shape not taken
+// true when gemm(g) reads and writes the rows listed in g.rows alone (a persistent kernel below takes the product); rows
+// outside the list then need not hold zeros
+bool gemm_rows_only(const Gemm& g);
+// gemm_rows_tc.cu: persistent tcgen05 kernel for tall products with a resident weight operand; false = shape not taken;
+// status null: nothing is launched
 bool gemm_rows_tc_try(const Gemm& g, cudaStream_t s, int* status);
-// gemm_wgrad_tc.cu: dW += dY^T X over tens of thousands of rows, both operands MN-major natural tiles
+// gemm_wgrad_tc.cu: dW += dY^T X over tens of thousands of rows, both operands MN-major natural tiles; same convention
 bool gemm_wgrad_tc_try(const Gemm& g, cudaStream_t s, int* status);
+// the products of linear_dx / linear_dw (below) as descriptors, for callers that ask gemm_rows_only first
+Gemm dgrad_gemm(int64_t M, int64_t N, int64_t K, const float* dY, int64_t lddy, const float* W, int64_t ldw, float* dX,
+                int64_t lddx, const int32_t* rows, const int32_t* nrows);
+Gemm wgrad_gemm(int64_t M, int64_t N, int64_t K, const float* dY, int64_t lddy, const float* X, int64_t ldx, float* dW,
+                int64_t lddw, const int32_t* rows, const int32_t* nrows);
 // C[M,N] = A[M,K] W[N,K]^T (+bias)
 int linear(int64_t M, int64_t N, int64_t K, const float* A, int64_t lda, const float* W, int64_t ldw,
            const float* bias, float* C, int64_t ldc, cudaStream_t s, bool relu_a = false, bool relu_out = false,
@@ -171,8 +181,21 @@ struct GruTcPair { GruTcOne e[2]; int n, save_gates; };    // save_gates = 0: fo
 bool gru_tc_supported();
 int gru_tc_fwd_pair(const GruTcPair& p, cudaStream_t s);
 void gru_debug_use_tcgen05(int on);
-int gru_seq_bwd(int64_t B, int64_t T, const int64_t* lens, const float* w_hh, const float* h_all, const float* gates,
-                const float* dh_in, float* dgi, float* dgh_all, float* db_ih, float* db_hh, cudaStream_t s, int32_t* order);
+// backward recurrence of up to two encoders in one launch.  order (nullable): sessions by decreasing length (gru_prep);
+// counter (nullable; needed for two encoders): the encoder's tile counter, zero on entry (tiles round robin without it).
+// live_only: dgi / dgh_all rows of padding slots (t >= len) are left unwritten, for products that read the live rows
+// alone; otherwise they are written as zeros, except slot T of dgh_all, which the caller clears
+struct GruBwdOne {
+    int64_t B, T;
+    const int64_t* lens;
+    const float *w_hh, *h_all, *gates, *dh_in;
+    float *dgi, *dgh_all, *db_ih, *db_hh;
+    const int32_t* order;
+    int32_t* counter;
+    int live_only;
+};
+struct GruBwdPair { GruBwdOne e[2]; int n; };
+int gru_seq_bwd_pair(const GruBwdPair& p, cudaStream_t s);
 // output projections (Linear(128 -> d <= 64), no bias) of both encoders in one launch, and their input gradients
 bool gru_outproj_pair_ok(int n0, int n1);
 int gru_outproj_pair_fwd(int64_t B, const int* n, const float* const* W, const float* const* h_last, const int64_t* ldh,
